@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--envs B] [--nodes 100] [--chargers 3] [--actions controller|uniform]
     python bench.py --impl reference ...        # the CPU restatement of the reference on the host cores, same law
+    python bench.py ... --dump-outputs DIR      # also write the outputs of the last timed step as DIR/<name>.npy
 
 One *step* = one pass of the hot path over the batch: the controller's action for every environment that holds a request,
 ``WRSN.step`` (advance to the next charger decision — at most ``--budget`` work units per launch, a longer step continues
@@ -34,7 +35,7 @@ UNIT = "decisions/s"
 def parse(argv=None):
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=60)
+    p.add_argument("--steps", type=int, default=None, help="timed steps (default 60); --workload ippo: timed training iterations")
     p.add_argument("--warmup", type=int, default=5)
     p.add_argument("--envs", type=int, default=4096, help="environments per GPU")
     p.add_argument("--nodes", type=int, default=100)
@@ -56,14 +57,26 @@ def parse(argv=None):
                    help="rollout: the simulator's hot path under the configured controller (the headline); ippo: BASELINE.json "
                         "configs[2], the IPPO training loop (alg_args/ippo.yaml) on the batched simulator — roll_out + clipped-PPO "
                         "update with the gradient all-reduce, U-Net actors / CNN critics per charger (SURVEY 8 f2)")
-    p.add_argument("--iterations", type=int, default=3, help="--workload ippo: timed training iterations")
+    p.add_argument("--iterations", type=int, default=3, help="--workload ippo: timed training iterations when --steps is not given")
     p.add_argument("--window", type=int, default=4, help="--workload ippo: rollout steps per collection window")
     p.add_argument("--impl", default="b200", choices=["b200", "reference"])
     p.add_argument("--cpu-seconds", type=float, default=15.0, help="budget of the cpu_baseline sample")
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-extras", action="store_true", help="skip the side figures (uniform actions, standalone kernels)")
     p.add_argument("--engine-switch", type=int, default=0, help="diagnostic: hdr[OPT_NOBATCH] of every environment (see include/wrsn_b200.h)")
-    return p.parse_args(argv)
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the last timed step handed its caller to DIR/<name>.npy (rank 0's environments; see dump_outputs)")
+    a = p.parse_args(argv)
+    if a.workload == "ippo":                         # one timed step of the IPPO workload is one training iteration
+        a.iterations = a.iterations if a.steps is None else a.steps
+        a.steps = a.iterations
+    elif a.steps is None:
+        a.steps = 60
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.workload != "rollout"):
+        p.error("--dump-outputs covers the rollout workload of --impl b200")
+    return a
 
 
 DEFAULT_BUDGET = 100
@@ -204,6 +217,36 @@ def config_common(a, **extra):
 
 
 # ----------------------------------------------------------------------------------------------- GPU side
+DUMP_OBS_ROWS = 64                                   # observation rows kept by --dump-outputs (160 KB each at S = 100)
+DUMP_MAX_ENVS = 1 << 18                              # environments kept by --dump-outputs: 136 B each, 36 MB at most
+
+
+def dump_outputs(out_dir, groups, act, obs):
+    """``--dump-outputs``: what the last timed step handed its caller, one ``<name>.npy`` per array, so that two builds run with
+    the same arguments (hence the same scenarios, seeds and step count) can be compared output for output.  The request record
+    (``request_*``, float64; ``request_stats`` holds the running totals of the whole run, ``request_flags`` the engine's error
+    bits) and the actions the step applied (``action``) of every environment, or of a fixed, seeded sample of ``DUMP_MAX_ENVS``
+    of them (their indices in ``env_rows``); the float32 observations of a fixed, seeded sample of ``DUMP_OBS_ROWS`` environments
+    (``observation``, their indices in ``observation_rows``): all of them would be 655 MB at 4096 environments.  A row without a
+    request (``request_agent_id < 0``) has no reward, detail or action (the reference's None, NaN in the record): written as 0."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    B, Bg = sum(env.B for env in groups), obs[0].shape[0]
+    env_rows = np.arange(B) if B <= DUMP_MAX_ENVS else np.sort(np.random.default_rng(1).choice(B, size=DUMP_MAX_ENVS, replace=False))
+    rows = np.sort(np.random.default_rng(0).choice(B, size=min(B, DUMP_OBS_ROWS), replace=False))
+    out = {"request_" + name: torch.cat([getattr(env.req, name) for env in groups]).to(torch.float64).cpu().numpy()[env_rows]
+           for name in ("agent_id", "terminal", "reward", "now", "action", "detail", "flags", "stats")}
+    none = out["request_agent_id"] < 0
+    for name in ("reward", "detail", "action"):
+        out["request_" + name][none] = 0.0
+    out["action"] = torch.cat(act).cpu().numpy()[env_rows]
+    out["env_rows"] = env_rows.astype(np.float64)
+    out["observation"] = np.stack([obs[r // Bg][r % Bg].cpu().numpy() for r in rows])
+    out["observation_rows"] = rows.astype(np.float64)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 class ClockSampler:
     Q = ("clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown,"
          "clocks_event_reasons.sw_thermal_slowdown,clocks_event_reasons.sw_power_cap")
@@ -333,6 +376,8 @@ def run_b200(a):
         time.sleep(0.3)
     elapsed_ms, (decisions, ticks, episodes), t_wall0, t_wall1 = timed(a.actions, a.steps)
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
+    if a.dump_outputs and rank == 0:                 # before the legs below advance the same environments
+        dump_outputs(a.dump_outputs, groups, act, obs)
     # per group and step: [k_decode_map, k_decode_locate,] [k_step_order (launches of >= 2048 rows),] k_env<STEP>, k_env<RESTORE_RESET>, k_observe
     launches_per_step = ((6 if a.actions == "controller" else 4) - (0 if 2048 <= Bg <= 16384 else 1)) * G
     n_launch = launches_per_step * a.steps

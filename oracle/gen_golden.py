@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Generate the committed golden fixtures under ``tests/golden/`` by running the
-UNMODIFIED reference (``/root/reference``) under the oracle shims.
+UNMODIFIED reference (a checkout: set ``WRSN_REFERENCE_ROOT``) under the oracle shims.
 
 TEST INFRASTRUCTURE (oracle side).  Run from the repo root in the build container:
 
@@ -121,7 +121,7 @@ def pure_network(R, scn, snap_times=(0.25, 0.75, 1.25, 10.75, 11.25, 100.0 - 0.2
 
 
 def _scenario_arrays(io_or_path):
-    """The scenario as plain arrays, so tests need neither /root/reference nor its YAML files."""
+    """The scenario as plain arrays, so tests need neither a checkout of the reference nor its YAML files."""
     import yaml
     with open(io_or_path) as f:
         d = yaml.safe_load(f)

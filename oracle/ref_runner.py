@@ -1,4 +1,4 @@
-"""Run the UNMODIFIED reference (`/root/reference`) under the oracle shims.
+"""Run the UNMODIFIED reference (a checkout of the original project) under the oracle shims.
 
 TEST INFRASTRUCTURE.  Used only (a) here, in the build container, to generate the
 golden fixtures under ``tests/golden/`` (see ``oracle/gen_golden.py``) and to
@@ -13,7 +13,7 @@ Nothing in the product package imports this file.
 fixtures under it; no such wheel exists in this image, so that test is skipped here).
 
 The reference root is looked up in this order: ``$WRSN_REFERENCE_ROOT``,
-``/root/reference``, ``<repo>/baseline/_ref``.
+``<repo>/baseline/_ref``.
 """
 import os
 import sys
@@ -23,8 +23,7 @@ _REPO = os.path.dirname(_HERE)
 
 
 def reference_root():
-    for cand in (os.environ.get("WRSN_REFERENCE_ROOT"), "/root/reference",
-                 os.path.join(_REPO, "baseline", "_ref")):
+    for cand in (os.environ.get("WRSN_REFERENCE_ROOT"), os.path.join(_REPO, "baseline", "_ref")):
         if cand and os.path.isfile(os.path.join(cand, "rl_env", "WRSN.py")):
             return cand
     return None

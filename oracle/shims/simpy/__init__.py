@@ -1,6 +1,6 @@
 """SimPy-4.0.1-semantics shim (TEST INFRASTRUCTURE, oracle side only).
 
-The reference (`/root/reference`) pins ``simpy==4.0.1`` (requirements.txt:52) but
+The reference pins ``simpy==4.0.1`` (requirements.txt:52) but
 SimPy is not installed in this image and there is no network.  This module
 restates the part of SimPy's published scheduling contract that the reference
 uses (call sites: NetworkIO.py:33; WRSN.py:43,53,62,127,302,307-311;

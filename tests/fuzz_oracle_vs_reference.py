@@ -1,4 +1,4 @@
-"""TEST INFRASTRUCTURE (not collected by pytest; build container only — needs /root/reference): the C restatement of the
+"""TEST INFRASTRUCTURE (not collected by pytest; needs a checkout of the reference: set WRSN_REFERENCE_ROOT): the C restatement of the
 reference (oracle/wrsn_oracle.c) against the UNMODIFIED Python reference run under the oracle shims, on RANDOM synthetic
 scenarios and action streams — beyond the 16 committed fixtures.  Decision by decision: agent id, terminal flag, env.now and
 every node's status identical; reward, node energies, charger energies at 1e-9 relative.

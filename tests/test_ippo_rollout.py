@@ -12,6 +12,7 @@ import torch
 
 from multi_agent_rl_wrsn_b200 import _lib, synthetic
 from multi_agent_rl_wrsn_b200.controllers import select_batch
+from oracle.ref_runner import reference_root
 from tests import parity_cases as pc
 from tests.helpers import REPO
 
@@ -134,11 +135,10 @@ def test_per_agent_policy_matches_ippo_evaluate():
         PerAgentPolicy(actors[:2])(agent, obs)
 
 
-REFERENCE = "/root/reference"
+REFERENCE = reference_root()
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REFERENCE, "controller", "ppo", "actor", "UnetActor.py")),
-                    reason="needs a checkout of the reference (build container only)")
+@pytest.mark.skipif(REFERENCE is None, reason="needs a checkout of the reference (set WRSN_REFERENCE_ROOT)")
 def test_reference_networks_fit_the_batched_interfaces():
     """The reference's own UNet actor and CNNCritic (imported unmodified, CPU) behind PerAgentPolicy and ppo_update: shapes,
     the squeezed batch of one, and log-probabilities that IPPO.evaluate reproduces."""

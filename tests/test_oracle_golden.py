@@ -9,6 +9,7 @@ import os
 import numpy as np
 import pytest
 
+from oracle.ref_runner import reference_root
 from oracle.wrsn_oracle import OracleWRSN
 from tests.helpers import golden, golden_names, mc_dict_of, scenario_of
 
@@ -105,7 +106,7 @@ def test_episode(name):
     _close(o.consts()["avg_nodes_agent"], float(g["avg_nodes_agent"]), rtol=1e-15)
 
 
-@pytest.mark.skipif(not os.path.isfile("/root/reference/rl_env/WRSN.py"), reason="needs the reference checkout (build container only)")
+@pytest.mark.skipif(reference_root() is None, reason="needs a checkout of the reference (set WRSN_REFERENCE_ROOT)")
 def test_oracle_vs_live_reference_on_random_scenarios():
     """Beyond the frozen fixtures: the C restatement against the unmodified reference run here under the shims, two random
     synthetic scenarios with random actions (tests/fuzz_oracle_vs_reference.py is the long form: 44 configurations clean)."""

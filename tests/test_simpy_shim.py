@@ -14,6 +14,7 @@ import sys
 
 import pytest
 
+from oracle.ref_runner import reference_root
 from tests.helpers import REPO
 
 
@@ -173,7 +174,7 @@ def _genuine_simpy():
 
 
 @pytest.mark.skipif(not _genuine_simpy(), reason="no genuine simpy distribution in this image (requirements.txt:52 pins simpy==4.0.1)")
-@pytest.mark.skipif(not os.path.isfile("/root/reference/rl_env/WRSN.py"), reason="reference sources absent")
+@pytest.mark.skipif(reference_root() is None, reason="needs a checkout of the reference (set WRSN_REFERENCE_ROOT)")
 def test_goldens_under_genuine_simpy(tmp_path):
     """Pins the one layer the fixtures inherit from the shim: regenerate one pure-network trace and one episode with the
     UNMODIFIED reference under the GENUINE simpy package and demand the committed fixtures byte for byte.  Skipped where no

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Time the UNMODIFIED Python reference (`/root/reference`, run under the oracle shims: oracle/ref_runner.py) on the host cores,
+"""Time the UNMODIFIED Python reference (a checkout found through $WRSN_REFERENCE_ROOT, run under the oracle shims: oracle/ref_runner.py) on the host cores,
 as BASELINE.md §4 plans it: one `WRSN` per process on all cores, the reference's own loop (runner/checkRL.py:33-36) —
 `RandomController.make_action` -> `WRSN.step` with `density_map=True` (default), or uniform 3-vector actions with
 `--actions uniform` — for a fixed wall budget after `reset()`.  Prints one JSON line (`kind: "python-reference"`).
@@ -59,7 +59,7 @@ if __name__ == "__main__":
                           per_core=per / a.cores, decisions=n, seconds_per_worker=a.seconds,
                           reset_seconds=sum(r[2] for r in res) / len(res), simulated_seconds=sum(r[3] for r in res),
                           sim_seconds_per_decision=sum(r[3] for r in res) / max(n, 1),
-                          sample="unmodified /root/reference under oracle/shims (SimPy-4.0.1-semantics shim), %s.yaml, 3 chargers, "
+                          sample="unmodified reference under oracle/shims (SimPy-4.0.1-semantics shim), %s.yaml, 3 chargers, "
                                  "map 100, %s, one WRSN per process x %d processes, %.0f s each after reset()" % (
                                      a.scenario, "RandomController density maps (density_map=True)" if a.actions == "controller"
                                      else "uniform 3-vector actions (density_map=False)", a.cores, a.seconds),
