@@ -68,13 +68,6 @@
 #define WRSN_LEAD(c) ((c).tid == 0)
 #endif
 
-#undef WRSN_NPT_MAX                                 /* node slots per thread the register-resident loops are built for */
-#if WRSN_GFIX == 32
-#define WRSN_NPT_MAX 4                              /* one warp: N <= 128 */
-#else
-#define WRSN_NPT_MAX 9                              /* 256 threads: N <= 2304 (shared memory ends before that) */
-#endif
-
 #undef WRSN_LDG                                     /* read-only scenario data (CSR graph, flags): the non-coherent L1 path */
 #if defined(WRSN_HOST_EMU)
 #define WRSN_LDG(p) (*(p))
@@ -216,6 +209,21 @@ WRSN_D void ctx_bind(Ctx &c, const wrsn_dims &d, const WrsnLayout &L, const char
     c.direct = (const uint8_t *)(scen_row + L.soff[WRSN_S_DIRECT]);
 }
 
+/* 32-bit shared-memory addressing for the hot loop: on the device an address is the byte offset inside the CTA's shared
+ * window (ld.shared / st.shared with a register address: no generic pointers, nothing to re-derive inside the loop); in
+ * the host emulation it is the offset from the environment's image. */
+#if !defined(WRSN_HOST_EMU)
+typedef uint32_t saddr_t;
+WRSN_DI saddr_t saddr_of(const void *p) { return (saddr_t)__cvta_generic_to_shared(p); }
+WRSN_DI double lds64(saddr_t a) { double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
+WRSN_DI void sts64(saddr_t a, double v) { asm volatile("st.shared.f64 [%0], %1;" :: "r"(a), "d"(v) : "memory"); }
+#else
+typedef size_t saddr_t;
+WRSN_DI saddr_t saddr_of(const void *p) { return (saddr_t)((const char *)p - WRSN_SMEM_BASE); }
+WRSN_DI double lds64(saddr_t a) { return *(const double *)(WRSN_SMEM_BASE + a); }
+WRSN_DI void sts64(saddr_t a, double v) { *(double *)(WRSN_SMEM_BASE + a) = v; }
+#endif
+
 /* ------------------------------------------------------------------ group primitives */
 WRSN_D void gsync(const Ctx &c) {
 #if defined(WRSN_HOST_EMU)
@@ -273,42 +281,47 @@ WRSN_D double red_min(const Ctx &c, double v) {
 /* sums of TWO values over the environment's threads with ONE barrier: the per-warp partial sums are exchanged through
  * alternating halves of c.red (`buf` flips at every call), so the writes of call r+1 cannot meet the reads of call r; the
  * reads of call r-1 are over because every thread has passed call r's barrier since.  The caller puts one barrier before
- * the first call of a sequence (other users of c.red) and keeps `buf` in a register. */
-WRSN_DI void red_sum2(const Ctx &c, double &a, double &b, int &buf) {
+ * the first call of a sequence (other users of c.red) and keeps `buf` in a register.  `red` is saddr_of(c.red): the hot
+ * loop calls these with registers only.
+ * ptxas gives every shuffle a divergent-warp fallback (BRA.DIV to a WARPSYNC / ENDCOLLECTIVE copy at the end of the
+ * function) because it cannot prove that the warp arrives converged at the entry of a __noinline__ function; a
+ * __syncwarp() in front does not change that.  The fallback is never taken (every lane of every warp calls these) and sits
+ * outside the loop's instruction stream. */
+WRSN_DI void red_sum2(saddr_t red, int tid, int G, double &a, double &b, int &buf) {
 #if defined(WRSN_HOST_EMU)
-    (void)c; (void)a; (void)b; (void)buf;
+    (void)red; (void)tid; (void)G; (void)a; (void)b; (void)buf;
 #else
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) { a += __shfl_xor_sync(0xffffffffu, a, o); b += __shfl_xor_sync(0xffffffffu, b, o); }
 #if WRSN_GFIX != 32
-    double *x = c.red + 16 * buf;
+    const saddr_t x = red + 128u * (uint32_t)buf;
     buf ^= 1;
-    const int nw = c.G >> 5;
-    if ((c.tid & 31) == 0) { x[2 * (c.tid >> 5)] = a; x[2 * (c.tid >> 5) + 1] = b; }
+    const int nw = G >> 5;
+    if ((tid & 31) == 0) { sts64(x + 16u * (uint32_t)(tid >> 5), a); sts64(x + 16u * (uint32_t)(tid >> 5) + 8u, b); }
     __syncthreads();
-    a = x[0]; b = x[1];
-    for (int k = 1; k < nw; k++) { a += x[2 * k]; b += x[2 * k + 1]; }
+    a = lds64(x); b = lds64(x + 8u);
+    for (int k = 1; k < nw; k++) { a += lds64(x + 16u * (uint32_t)k); b += lds64(x + 16u * (uint32_t)k + 8u); }
 #else
-    (void)c; (void)buf;
+    (void)red; (void)tid; (void)G; (void)buf;
 #endif
 #endif
 }
-WRSN_DI void red_sum1(const Ctx &c, double &a, int &buf) {
+WRSN_DI void red_sum1(saddr_t red, int tid, int G, double &a, int &buf) {
 #if defined(WRSN_HOST_EMU)
-    (void)c; (void)a; (void)buf;
+    (void)red; (void)tid; (void)G; (void)a; (void)buf;
 #else
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
 #if WRSN_GFIX != 32
-    double *x = c.red + 16 * buf;
+    const saddr_t x = red + 128u * (uint32_t)buf;
     buf ^= 1;
-    const int nw = c.G >> 5;
-    if ((c.tid & 31) == 0) x[c.tid >> 5] = a;
+    const int nw = G >> 5;
+    if ((tid & 31) == 0) sts64(x + 8u * (uint32_t)(tid >> 5), a);
     __syncthreads();
-    a = x[0];
-    for (int k = 1; k < nw; k++) a += x[k];
+    a = lds64(x);
+    for (int k = 1; k < nw; k++) a += lds64(x + 8u * (uint32_t)k);
 #else
-    (void)c; (void)buf;
+    (void)red; (void)tid; (void)G; (void)buf;
 #endif
 #endif
 }
@@ -403,7 +416,7 @@ WRSN_D double wrsn_rsqrt(double v) {                /* 1 / sqrt(v), v > 0 normal
 /* exp(z) for |z| < 700, relative error <= 1e-13: z = (64 n + j) ln2/64 + r, |r| <= ln2/128;
  * exp(z) = 2^n * 2^(j/64) * (1 + r + r^2/2 + r^3/6 + r^4/24) — table of 64 doubles in shared memory (c.exptab, copied from
  * wrsn_exp2_tab at kernel start), four FMAs.  The caller's z is a z-score of N values: |z| <= sqrt(N - 1). */
-WRSN_DI double wrsn_exp_tab(const double *tab, double z) {
+WRSN_DI double wrsn_exp_tab(saddr_t tab, double z) {
     const double t = __fma_rn(z, 92.33248261689366, 6755399441055744.0);          /* 64 / ln2; 1.5 * 2^52: the integer lands in the low word */
     const int k = __double2loint(t);
     const double r = __fma_rn(t - 6755399441055744.0, -0.010830424696249145, z); /* ln2 / 64 */
@@ -411,7 +424,7 @@ WRSN_DI double wrsn_exp_tab(const double *tab, double z) {
     p = __fma_rn(p, r, 0.5);
     p = __fma_rn(p, r, 1.0);
     p = __fma_rn(p, r, 1.0);
-    const double y = p * tab[k & 63];
+    const double y = p * lds64(tab + 8u * (uint32_t)(k & 63));
     return __hiloint2double(__double2hiint(y) + ((k >> 6) << 20), __double2loint(y));
 }
 #else
@@ -419,11 +432,11 @@ WRSN_D double wrsn_fma(double a, double b, double c) { return a * b + c; }
 WRSN_D double wrsn_rcp(double d) { return 1.0 / d; }
 WRSN_D double wrsn_rsqrt(double v) { return 1.0 / sqrt(v); }
 #endif
-WRSN_DI double wrsn_exp_b(const Ctx &c, double z) {
+WRSN_DI double wrsn_exp_b(saddr_t tab, double z) {  /* tab = saddr_of(c.exptab) */
 #if defined(WRSN_HOST_EMU)
-    (void)c; return exp(z);
+    (void)tab; return exp(z);
 #else
-    return wrsn_exp_tab(c.exptab.ptr(), z);
+    return wrsn_exp_tab(tab, z);
 #endif
 }
 
@@ -1038,7 +1051,7 @@ WRSN_D double charge_rate_to(Ctx &c, const double *m, int node) {   /* alpha / (
 
 /* the softmax priority + incentive sums; only reached when some incentive sum is non-empty */
 WRSN_NOINLINE double drain_node(double e, double rr, double es, double er, int nb, int ow, int na, double cap);
-WRSN_D void catch_up_for_reward(Ctx &c, double t_reward);
+WRSN_NOINLINE void catch_up_for_reward(Ctx &c, double t_reward);
 
 WRSN_D bool reward_pairs(Ctx &c) {                 /* is there any (charging charger, connected alive node) pair? */
     bool any = false;
@@ -1053,21 +1066,12 @@ WRSN_D bool reward_pairs(Ctx &c) {                 /* is there any (charging cha
     return any;
 }
 
-/* per-thread node slots of the register-resident loops (reward_loop below): compile-time arrays on the device, the
- * whole node range in the single-lane host build */
+/* per-slot flags of a thread (slot s = node tid + s * G, reward_loop below): one bit mask per flag on the device
+ * (registers; the launcher keeps N <= 9 * threads), byte arrays in the host emulation (one "thread" owns all N nodes there) */
 #undef WRSN_EMU_MAXN
-#undef WRSN_SLOT_ARR
-#undef WRSN_FOR_SLOTS
 #if defined(WRSN_HOST_EMU)
 #define WRSN_EMU_MAXN 32768
-#define WRSN_SLOT_ARR(T, name) static thread_local T name[WRSN_EMU_MAXN]
-#define WRSN_FOR_SLOTS(s) for (int s = 0; s < NPT; s++)
-#else
-#define WRSN_SLOT_ARR(T, name) T name[NPT_T > 0 ? NPT_T : WRSN_NPT_MAX]
-#define WRSN_FOR_SLOTS(s) _Pragma("unroll") for (int s = 0; s < (NPT_T > 0 ? NPT_T : NPT); s++)
 #endif
-/* per-slot flags of a thread: one bit mask per flag on the device (registers), byte arrays in the host emulation (one
- * "thread" owns all N nodes there) */
 #undef WRSN_FLAGS_DECL
 #undef WRSN_FL_GET
 #undef WRSN_FL_SET
@@ -1236,23 +1240,8 @@ WRSN_NOINLINE void pairs_phase(Ctx &c, double tot, int n_pairs) {
     }
 }
 
-/* 32-bit shared-memory addressing for the hot loop: on the device an address is the byte offset inside the CTA's shared
- * window (ld.shared / st.shared with a register address: no generic pointers, nothing to re-derive inside the loop); in
- * the host emulation it is the offset from the environment's image. */
-#if !defined(WRSN_HOST_EMU)
-typedef uint32_t saddr_t;
-WRSN_DI saddr_t saddr_of(const void *p) { return (saddr_t)__cvta_generic_to_shared(p); }
-WRSN_DI double lds64(saddr_t a) { double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
-WRSN_DI void sts64(saddr_t a, double v) { asm volatile("st.shared.f64 [%0], %1;" :: "r"(a), "d"(v) : "memory"); }
-#else
-typedef size_t saddr_t;
-WRSN_DI saddr_t saddr_of(const void *p) { return (saddr_t)((const char *)p - WRSN_SMEM_BASE); }
-WRSN_DI double lds64(saddr_t a) { return *(const double *)(WRSN_SMEM_BASE + a); }
-WRSN_DI void sts64(saddr_t a, double v) { *(double *)(WRSN_SMEM_BASE + a) = v; }
-#endif
-
 /* ------------------------------------------------------------------ the hot loop: update_reward second by second
- * `n_cycles` consecutive update_reward ticks (WRSN.py:100-127) with the node rows of this thread IN REGISTERS.
+ * `n_cycles` consecutive update_reward ticks (WRSN.py:100-127) on the node rows in shared memory.
  * batch == 0 (event path): one tick on the node rows as they are.
  * batch != 0 (whole-cycle batches, nodes_batch): the grid events around every tick are applied on the way — the k+1.0
  *   bookkeeping of the PREVIOUS second (second top-up; energyCS towards its fixed point), then this second's k+0.5
@@ -1264,47 +1253,29 @@ WRSN_DI void sts64(saddr_t a, double v) { *(double *)(WRSN_SMEM_BASE + a) = v; }
  *   fixed whole number of ulps (sub_chain's argument; D1, D2, H of the table), so the second is four exact additions
  *   and two minima while the energy stays between the table's guards, and the literal tick (spec_second) otherwise.
  *   The incentive sums work the same way: thread p < n_pairs owns the p-th (charging charger, connected alive node)
- *   pair.  Nothing in the steady-state path goes through the context record: 32-bit shared-memory addresses, computed
- *   before the loop.
+ *   pair.
+ * Thread tid owns the nodes i = tid, tid + G, ... (slot s = node tid + s * G) and walks them in a ROLLED loop: energy in
+ * c.energy, energyCS in c.cs, the per-second decrement in c.scr1, x_n in c.scr0 (overwritten in place by the softmax
+ * numerator of the nodes the incentive sums read; nobody else touches a slot's scr0 before the barrier of the tot sum).
+ * Rolled, not unrolled into registers: the unrolled slots (one instantiation per slot count) were 31 KB of code that the
+ * instruction caches could not hold next to the event code of the other environments on the SM; the rolled loop is one
+ * function of about 15 KB for every group size and pays a few shared-memory loads and stores per slot and second (DESIGN
+ * §4.1 has the measurement).  Per-slot flags stay in registers.  Nothing in the per-node passes goes through the context
+ * record (it sits in the kernel's stack frame): 32-bit shared-memory addresses and registers, computed before the loop.
  * Arithmetic of the tick itself: x_n = energyCS / (energy - threshold + eps) by reciprocal (wrsn_rcp), mean and variance
  * from one pass (sum and sum of squares; two passes when the variance is small against mean^2), 1 / std by wrsn_rsqrt,
- * the softmax numerators by wrsn_exp_b — see the note at those helpers.  The event path and the batches run this very
- * code, so they produce the same bits (tests: batches == event path).
- * NPT = node slots per thread (compile time on the device: everything below unrolls into registers). */
-template <int NPT_T>
-WRSN_NOINLINE void reward_loop(Ctx &c, int batch, int n_cycles, double t_reward, int watched, int n_spec) {
-    const int N = c.N, G = WRSN_GSZ(c), tid = c.tid, M = c.M;
-#if defined(WRSN_HOST_EMU)
-    const int NPT = N;
-#else
-    const int NPT = NPT_T > 0 ? NPT_T : (N + G - 1) / G;   /* NPT_T == 0: any N, the slot arrays in local memory (rolled loops) */
-#endif
-    const double thr = c.par[WRSN_P_THR], eps = c.par[WRSN_P_EPSENV], inv_n = c.par[WRSN_P_INVN], cap = c.par[WRSN_P_CAP];
-    const double ab2 = c.par[WRSN_P_MC_AB2], inv_ab2 = wrsn_rcp(ab2);
-    const double *dec = c.scr1.ptr();
-    const saddr_t a_energy = saddr_of(c.energy.ptr()) + 8 * tid, a_q = saddr_of(c.scr0.ptr()) + 8 * tid;
-    WRSN_SLOT_ARR(double, e); WRSN_SLOT_ARR(double, cs); WRSN_SLOT_ARR(double, d); WRSN_SLOT_ARR(double, x);
-    WRSN_FLAGS_DECL(f_in); WRSN_FLAGS_DECL(f_inc); WRSN_FLAGS_DECL(f_special); WRSN_FLAGS_DECL(f_unfixed);
-    int any_inc = 0, any_unfixed = 0, buf = 0;
-    gsync(c);
-    WRSN_FOR_SLOTS(s) {
-        const int i = tid + s * G;
-        const bool ok = i < N && c.status[i] != 0;
-        e[s] = ok ? c.energy[i] : cap; cs[s] = ok ? c.cs[i] : 0.0; d[s] = (ok && batch) ? dec[i] : 0.0;
-        if (i < N) WRSN_FL_SET(f_in, s);
-        if (ok) {
-            if (node_in_incentive(c, i)) { WRSN_FL_SET(f_inc, s); any_inc = 1; }
-            if (batch) { WRSN_FL_SET(f_unfixed, s); any_unfixed = 1; }
-            if (d[s] != d[s]) WRSN_FL_SET(f_special, s);
-        }
-    }
-    any_inc = red_or(c, any_inc);                    /* (uniform over the environment: it decides about barriers) */
-    /* the (charging charger, connected alive node) pairs of the incentive sums, charger by charger in node order */
+ * the softmax numerators by wrsn_exp_b — see the note at those helpers.  A dead node enters the sums with x_n = 0 and
+ * its softmax numerator enters tot.  The event path and the batches run this very code, so they produce the same bits
+ * (tests: batches == event path). */
+
+/* the (charging charger, connected alive node) pairs of the incentive sums, charger by charger in node order (thread 0
+ * builds the list; every thread gets the count) */
+WRSN_NOINLINE int reward_pair_list(Ctx &c) {
     double *pair_term = c.pairs.ptr();
     int *pair_ids = (int *)(pair_term + WRSN_PAIR_MAX), *pair_seg = pair_ids + 2 * WRSN_PAIR_MAX;
-    if (tid == 0) {
+    if (c.tid == 0) {
         int np = 0;
-        for (int a = 0; a < M; a++) {
+        for (int a = 0; a < c.M; a++) {
             const double *m = c.mc + a * WRSN_MC_LEN;
             pair_seg[2 * a] = np;
             if (m[WRSN_MC_STATUS] != 0.0 && m[WRSN_MC_TYPE] != 0.0) {
@@ -1322,29 +1293,74 @@ WRSN_NOINLINE void reward_loop(Ctx &c, int batch, int n_cycles, double t_reward,
         c.bcast[8] = np;
     }
     gsync(c);
-    const int n_pairs = c.bcast[8];
+    return c.bcast[8];
+}
+
+/* the textbook two-pass variance sum (np.std) over x_n in scr0, for a tick whose one-pass variance cancels (cold).  Flips
+ * the reduction buffer once: the caller does the same with its copy of `buf`. */
+WRSN_NOINLINE double reward_two_pass(const Ctx &c, double mean, int buf) {
+    const int G = WRSN_GSZ(c);
+    const saddr_t a_x = saddr_of(c.scr0.ptr() + c.tid);
+    double q = 0.0;
+    for (int i = c.tid, o = 0; i < c.N; i += G, o += 8 * G) { const double u = lds64(a_x + o) - mean; q = wrsn_fma(u, u, q); }
+    red_sum1(saddr_of(c.red.ptr()), c.tid, G, q, buf);
+    return q;
+}
+
+WRSN_NOINLINE void reward_loop(Ctx &c, int batch, int n_cycles, double t_reward, int watched, int n_spec) {
+    const int N = c.N, G = WRSN_GSZ(c), tid = c.tid, M = c.M;
+#if defined(WRSN_HOST_EMU)
+    const int NPT = N;                               /* (WRSN_FLAGS_DECL) */
+#endif
+    const double thr = c.par[WRSN_P_THR], eps = c.par[WRSN_P_EPSENV], inv_n = c.par[WRSN_P_INVN], cap = c.par[WRSN_P_CAP];
+    const double ab2 = c.par[WRSN_P_MC_AB2], inv_ab2 = wrsn_rcp(ab2);
+    /* this thread's first node in each row; slot s is 8 * s * G bytes further */
+    const saddr_t a_e = saddr_of(c.energy.ptr() + tid), a_cs = saddr_of(c.cs.ptr() + tid), a_x = saddr_of(c.scr0.ptr() + tid);
+    const saddr_t a_dec = saddr_of(c.scr1.ptr() + tid), a_logc = saddr_of(c.logc.ptr() + tid);
+    const saddr_t a_tab = saddr_of(c.exptab.ptr()), a_red = saddr_of(c.red.ptr());
+    const int step = 8 * G;
+    WRSN_FLAGS_DECL(f_ok); WRSN_FLAGS_DECL(f_inc); WRSN_FLAGS_DECL(f_special); WRSN_FLAGS_DECL(f_unfixed);
+    int any_inc = 0, any_unfixed = 0, buf = 0;
+    gsync(c);
+    _Pragma("unroll 1")
+    for (int i = tid, s = 0; i < N; i += G, s++) {
+        if (c.status[i] == 0) continue;
+        WRSN_FL_SET(f_ok, s);
+        if (node_in_incentive(c, i)) { WRSN_FL_SET(f_inc, s); any_inc = 1; }
+        if (batch) {
+            WRSN_FL_SET(f_unfixed, s); any_unfixed = 1;
+            if (c.scr1[i] != c.scr1[i]) WRSN_FL_SET(f_special, s);
+        }
+    }
+    any_inc = red_or(c, any_inc);                    /* (uniform over the environment: it decides about barriers) */
+    const int n_pairs = reward_pair_list(c);
     const bool listed = n_pairs <= WRSN_PAIR_MAX && n_pairs <= G && M <= G;   /* one thread per pair, one per charger */
     const bool own_pair = listed && tid < n_pairs;
     saddr_t a_pe = 0, a_pc = 0, a_pq = 0, a_pt = 0, a_excl = 0, a_seg = 0;
-    int p_node = 0, p_chg = 0, seg_n = 0;
-    if (own_pair) {
-        p_chg = pair_ids[2 * tid]; p_node = pair_ids[2 * tid + 1];
-        a_pe = saddr_of(c.energy.ptr() + p_node); a_pc = saddr_of(c.cs.ptr() + p_node); a_pq = saddr_of(c.scr0.ptr() + p_node);
-        a_pt = saddr_of(pair_term + tid);
-    }
-    if (listed && tid < M) {
-        seg_n = pair_seg[2 * tid + 1] - pair_seg[2 * tid];
-        a_seg = saddr_of(pair_term + pair_seg[2 * tid]);
-        a_excl = saddr_of(c.mc.ptr() + tid * WRSN_MC_LEN + WRSN_MC_EXCL);
+    int p_node = 0, seg_n = 0;
+    const double *p_mc = nullptr;
+    {
+        double *pair_term = c.pairs.ptr();
+        const int *pair_ids = (const int *)(pair_term + WRSN_PAIR_MAX), *pair_seg = pair_ids + 2 * WRSN_PAIR_MAX;
+        if (own_pair) {
+            p_mc = c.mc + pair_ids[2 * tid] * WRSN_MC_LEN; p_node = pair_ids[2 * tid + 1];
+            a_pe = saddr_of(c.energy.ptr() + p_node); a_pc = saddr_of(c.cs.ptr() + p_node); a_pq = saddr_of(c.scr0.ptr() + p_node);
+            a_pt = saddr_of(pair_term + tid);
+        }
+        if (listed && tid < M) {
+            seg_n = pair_seg[2 * tid + 1] - pair_seg[2 * tid];
+            a_seg = saddr_of(pair_term + pair_seg[2 * tid]);
+            a_excl = saddr_of(c.mc.ptr() + tid * WRSN_MC_LEN + WRSN_MC_EXCL);
+        }
     }
     /* this thread's table entry (t = tid; more entries than threads: the rest through spec_second) */
     const bool own_spec = tid < n_spec, more_spec = n_spec > G;
     double sD1 = 0.0, sD2 = 0.0, sH = 0.0, sLo = INFINITY, sHi = -INFINITY;
     saddr_t a_spec_e = 0;
+    const saddr_t a_sp = saddr_of(c.spec.ptr() + tid * WRSN_SPEC_LEN);
     if (own_spec) {
-        const double *sp = c.spec + tid * WRSN_SPEC_LEN;
-        sD1 = sp[0]; sD2 = sp[1]; sH = sp[2]; sLo = sp[3]; sHi = sp[4];
-        a_spec_e = saddr_of(c.energy.ptr() + (int)sp[5]);
+        sD1 = lds64(a_sp); sD2 = lds64(a_sp + 8); sH = lds64(a_sp + 16); sLo = lds64(a_sp + 24); sHi = lds64(a_sp + 32);
+        a_spec_e = saddr_of(c.energy.ptr() + (int)lds64(a_sp + 40));
     }
     _Pragma("unroll 1")
     for (int j = 0; j < n_cycles; j++) {
@@ -1358,52 +1374,52 @@ WRSN_NOINLINE void reward_loop(Ctx &c, int batch, int n_cycles, double t_reward,
                     sts64(a_spec_e, (en < cap ? en : cap) - sD2);
                 } else {
                     spec_second(c, tid, j > 0, 1);   /* literal second; the entry may have been rebuilt */
-                    const double *sp = c.spec + tid * WRSN_SPEC_LEN;
-                    sD1 = sp[0]; sD2 = sp[1]; sH = sp[2]; sLo = sp[3]; sHi = sp[4];
+                    sD1 = lds64(a_sp); sD2 = lds64(a_sp + 8); sH = lds64(a_sp + 16); sLo = lds64(a_sp + 24); sHi = lds64(a_sp + 32);
                 }
             }
-            if (more_spec) { for (int t = tid + G; t < n_spec; t += G) spec_second(c, t, j > 0, 1); }
+            if (more_spec) { _Pragma("unroll 1") for (int t = tid + G; t < n_spec; t += G) spec_second(c, t, j > 0, 1); }
             gsync(c);
         }
         if (j > 0 && red_or_warp(any_unfixed)) {     /* energyCS towards its fixed point (bookkeeping of the previous second;
                                                         cold: a node gets there after one or two applications) */
             any_unfixed = 0;
-            WRSN_FOR_SLOTS(s) {
+            _Pragma("unroll 1")
+            for (int i = tid, s = 0, o = 0; i < N; i += G, s++, o += step) {
                 if (WRSN_FL_GET(f_unfixed, s)) {
-                    const int i = tid + s * G;
-                    const double nx = cs_step(cs[s], c.logc[i]);
-                    if (nx == cs[s]) WRSN_FL_CLR(f_unfixed, s);
-                    else { cs[s] = nx; any_unfixed = 1; if (WRSN_FL_GET(f_inc, s)) c.cs[i] = nx; }
+                    const double cs = lds64(a_cs + o), nx = cs_step(cs, lds64(a_logc + o));
+                    if (nx == cs) WRSN_FL_CLR(f_unfixed, s);
+                    else { sts64(a_cs + o, nx); any_unfixed = 1; }
                 }
             }
         }
         double s1 = 0.0, s2 = 0.0;
-        WRSN_FOR_SLOTS(s) {
-            const double e_next = e[s] - d[s];       /* (event path: d == 0) */
-            e[s] = WRSN_FL_GET(f_special, s) ? lds64(a_energy + 8 * s * G) : e_next;
-            x[s] = cs[s] * wrsn_rcp(e[s] - thr + eps);
-            s1 += x[s]; s2 = wrsn_fma(x[s], x[s], s2);
+        _Pragma("unroll 1")
+        for (int i = tid, s = 0, o = 0; i < N; i += G, s++, o += step) {
+            double x = 0.0;                          /* dead node: energy = capacity, energyCS = 0 */
+            if (WRSN_FL_GET(f_ok, s)) {
+                double e = lds64(a_e + o);
+                if (batch && !WRSN_FL_GET(f_special, s)) { e = e - lds64(a_dec + o); sts64(a_e + o, e); }
+                x = lds64(a_cs + o) * wrsn_rcp(e - thr + eps);
+            }
+            sts64(a_x + o, x);
+            s1 += x; s2 = wrsn_fma(x, x, s2);
         }
-        red_sum2(c, s1, s2, buf);
+        red_sum2(a_red, tid, G, s1, s2, buf);
         const double mean = s1 * inv_n;
         double var = wrsn_fma(s2, inv_n, -(mean * mean));
         if (!(var > 1e-3 * (mean * mean))) {         /* cancellation: the textbook two passes (np.std) */
-            double q = 0.0;
-            WRSN_FOR_SLOTS(s) { const double u = WRSN_FL_GET(f_in, s) ? x[s] - mean : 0.0; q = wrsn_fma(u, u, q); }
-            red_sum1(c, q, buf);
-            var = q * inv_n;
+            var = reward_two_pass(c, mean, buf) * inv_n;
+            buf ^= 1;
         }
         const double a = var > 0.0 ? wrsn_rsqrt(var) : 1.0 / eps;       /* std == 0 -> std = epsilon (:104-105) */
         double tot = 0.0;
-        WRSN_FOR_SLOTS(s) {
-            const double q = wrsn_exp_b(c, (x[s] - mean) * a);
-            tot += WRSN_FL_GET(f_in, s) ? q : 0.0;
-            if (WRSN_FL_GET(f_inc, s)) {             /* what the incentive sums read */
-                sts64(a_q + 8 * s * G, q);
-                if (batch && !WRSN_FL_GET(f_special, s)) sts64(a_energy + 8 * s * G, e[s]);
-            }
+        _Pragma("unroll 1")
+        for (int i = tid, s = 0, o = 0; i < N; i += G, s++, o += step) {
+            const double q = wrsn_exp_b(a_tab, (lds64(a_x + o) - mean) * a);
+            tot += q;
+            if (WRSN_FL_GET(f_inc, s)) sts64(a_x + o, q);   /* what the incentive sums read */
         }
-        red_sum1(c, tot, buf);                       /* (its barrier also publishes the stores above) */
+        red_sum1(a_red, tid, G, tot, buf);           /* (its barrier also publishes the stores above) */
         if (WRSN_GFIX == 32) gsync(c);
         if (tot == 0.0) tot = eps;
         if (n_pairs > 0) {
@@ -1411,12 +1427,13 @@ WRSN_NOINLINE void reward_loop(Ctx &c, int batch, int n_cycles, double t_reward,
                 if (own_pair) {
                     const double ec = lds64(a_pe) - lds64(a_pc);
                     double e_with = cap;             /* max(ec + rate, capacity) with rate <= alpha / beta^2 */
-                    if (ec + ab2 > cap) e_with = fmax(ec + charge_rate_fast(c, c.mc + p_chg * WRSN_MC_LEN, p_node), cap);
+                    if (ec + ab2 > cap) e_with = fmax(ec + charge_rate_fast(c, p_mc, p_node), cap);
                     sts64(a_pt, (lds64(a_pq) * wrsn_rcp(tot)) * (e_with - (ec < thr ? ec : thr)) * inv_ab2);
                 }
                 gsync(c);
                 if (seg_n > 0) {
                     double incentive = 0.0;
+                    _Pragma("unroll 1")
                     for (int p = 0; p < seg_n; p++) incentive += lds64(a_seg + 8 * p);
                     sts64(a_excl, lds64(a_excl) + incentive);
                 }
@@ -1424,34 +1441,17 @@ WRSN_NOINLINE void reward_loop(Ctx &c, int batch, int n_cycles, double t_reward,
         }
         if (any_inc || n_spec > 0 || watched || WRSN_GFIX != 32) gsync(c);
     }
-    if (batch) {                                     /* bookkeeping of the last second; rows back to shared memory */
+    if (batch) {                                     /* bookkeeping of the last second */
         if (n_spec > 0) spec_phase(c, n_spec, 1, 0);
-        WRSN_FOR_SLOTS(s) {
-            const int i = tid + s * G;
-            if (!(i < N && c.status[i] != 0)) continue;
-            if (WRSN_FL_GET(f_unfixed, s)) cs[s] = cs_step(cs[s], c.logc[i]);
-            c.cs[i] = cs[s];
-            if (!WRSN_FL_GET(f_special, s)) c.energy[i] = e[s];
-        }
+        _Pragma("unroll 1")
+        for (int i = tid, s = 0, o = 0; i < N; i += G, s++, o += step)
+            if (WRSN_FL_GET(f_unfixed, s)) sts64(a_cs + o, cs_step(lds64(a_cs + o), lds64(a_logc + o)));
         gsync(c);
     }
 }
 
-WRSN_NOINLINE void reward_cycles_any(Ctx &c, int batch, int n_cycles, double t_reward, int watched, int n_spec) {
-#if defined(WRSN_HOST_EMU)
-    reward_loop<0>(c, batch, batch ? n_cycles : 1, t_reward, batch ? watched : 0, batch ? n_spec : 0);
-#else
-    const int npt = (c.N + WRSN_GSZ(c) - 1) / WRSN_GSZ(c);
-    if (!batch) { n_cycles = 1; watched = 0; n_spec = 0; }
-    if (npt <= 1) reward_loop<1>(c, batch, n_cycles, t_reward, watched, n_spec);
-    else if (npt <= 2) reward_loop<2>(c, batch, n_cycles, t_reward, watched, n_spec);
-    else if (npt <= 4) reward_loop<4>(c, batch, n_cycles, t_reward, watched, n_spec);
-    else reward_loop<0>(c, batch, n_cycles, t_reward, watched, n_spec);
-#endif
-}
-
 WRSN_D void ev_update_reward(Ctx &c) {
-    if (reward_pairs(c)) reward_cycles_any(c, 0, 1, 0.0, 0, 0);   /* otherwise every incentive sum is empty: excl += 0 */
+    if (reward_pairs(c)) reward_loop(c, 0, 1, 0.0, 0, 0);   /* otherwise every incentive sum is empty: excl += 0 */
 }
 
 /* ------------------------------------------------------------------ WRSN.get_network_fitness (WRSN.py:188-220) -> min */
@@ -1810,7 +1810,7 @@ WRSN_D void catch_up_many(Ctx &c, double limit, int kind) {
     gsync(c);
 }
 /* update_reward is about to read the chargers' positions */
-WRSN_D void catch_up_for_reward(Ctx &c, double t_reward) { catch_up_many(c, t_reward, 2); }
+WRSN_NOINLINE void catch_up_for_reward(Ctx &c, double t_reward) { catch_up_many(c, t_reward, 2); }
 
 /* a death: every lazy run ends (the alive set of a charge, hence its rate, changes from the next connection on) */
 WRSN_DI void wake_lazy_all(Ctx &c, Clk &k) {
@@ -2198,7 +2198,7 @@ WRSN_NOINLINE int nodes_batch(Ctx &c, int n_max, int ur_on, double t_reward, int
            drain, the tick and the previous second's bookkeeping in one pass over the nodes per second (reward_loop) */
         int watched = 0;                             /* is there a lazy move whose position update_reward reads (Q2)? */
         for (int q = 0; q < c.n_slot; q++) watched |= slot_i(slot_of(c, q))[WRSN_PRI_LAZY] == 2 ? 1 : 0;
-        reward_cycles_any(c, 1, n_safe, t_reward, watched, n_spec);
+        reward_loop(c, 1, n_safe, t_reward, watched, n_spec);
         WRSN_PROFC_END(c, WRSN_H_PROF3, pc2);
     }
     if (c.tid == 0) {
