@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define WRSN_ABI_VERSION 18
+#define WRSN_ABI_VERSION 19
 #define WRSN_MAX_MC 16          /* chargers per environment */
 #define WRSN_RING 10            /* Node.operate keeps the last 10 per-second consumptions (Node.py:70-77) */
 
@@ -45,6 +45,7 @@ enum {
     WRSN_P_CAPMTHR,                                    /* capacity - threshold */
     WRSN_P_ESMAX,                                      /* largest per-hop cost in the scenario (slack of the no-death test) */
     WRSN_P_INVN,                                       /* 1 / number of nodes (mean and variance of update_reward's priorities) */
+    WRSN_P_NNODES, WRSN_P_NTARGETS,                    /* this scenario's own node and target counts (at most wrsn_dims.N / T) */
     WRSN_P_LEN = 32
 };
 
@@ -142,7 +143,10 @@ enum {
 
 typedef struct wrsn_dims {
     int32_t B;        /* environments in this shard */
-    int32_t N, T, M;  /* nodes, targets, chargers (same for every scenario of the batch) */
+    int32_t N, T, M;  /* nodes and targets: the largest over the batch's scenarios (each scenario's own counts are its par
+                         row's WRSN_P_NNODES / WRSN_P_NTARGETS; its node slots [own N, Npad) are dead padding); chargers
+                         (the same for every scenario).  Npad, W, Tw, the layouts, the shared-memory size and `threads`
+                         derive from these maxima, so every environment of a batch runs on the same thread count */
     int32_t S;        /* map_size */
     int32_t Emax;     /* neighbour CSR capacity per scenario */
     int32_t TEmax;    /* node->target CSR capacity per scenario */
@@ -268,7 +272,8 @@ int wrsn_decode_linear_controller(const wrsn_dims *d, const void *scen, const in
 int wrsn_record_transitions(const wrsn_dims *d, const wrsn_request *req, int64_t t, const int64_t *agent_prev,
                             int64_t *last, double *resets_seen, int64_t *agent_next, int64_t *link_next,
                             uint8_t *new_episode_next, double *reward_next, double *now_next, void *stream);
-/* WRSN.get_network_fitness (:188-220): per-target values fitness[B][T] (may be NULL) and their minimum fit_min[B]. */
+/* WRSN.get_network_fitness (:188-220): per-target values fitness[B][T] (may be NULL) and their minimum fit_min[B] over the row's own
+ * targets; the columns beyond a row's own target count are not written. */
 int wrsn_fitness(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state,
                  double *fitness, double *fit_min, void *stream);
 
@@ -286,7 +291,8 @@ int wrsn_k_reward(const wrsn_dims *d, const void *scen, const int32_t *scen_id, 
  * ORDER (bit-exact with the reference's sequential +=).  The fused step kernel applies the same model incrementally (connect /
  * disconnect events); this entry point is the standalone form for unit parity and profiling.  Does not modify the state. */
 int wrsn_k_charge(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state, const uint8_t *charging,
-                  double *node_rate /* [B][N] */, double *mc_rate /* [B][M] */, void *stream);
+                  double *node_rate /* [B][N]: columns beyond a row's own node count are not written */, double *mc_rate /* [B][M] */,
+                  void *stream);
 
 #ifdef __cplusplus
 }

@@ -50,8 +50,13 @@ class Requests:
 class BatchedWRSN:
     def __init__(self, scenarios, num_agent=3, mc_type=None, num_envs=None, scenario_index=None, map_size=100,
                  warm_up_time=100, device=None, threads=0, step_budget=0, step_rounds=0):
-        """``scenarios``: one or several ``Scenario`` / YAML paths (all with the same N and T);
-        ``scenario_index[b]`` picks the scenario of environment b (default: round robin).
+        """``scenarios``: one or several ``Scenario`` / YAML paths, possibly of different sizes;
+        ``scenario_index[b]`` picks the scenario of environment b (default: round robin).  Every environment simulates
+        exactly its own scenario.  ``self.N`` / ``self.T`` are the largest node and target counts of the batch and
+        ``self.num_nodes`` / ``self.num_targets`` (int32 [B] on the device) each row's own.  Per-node and per-target views
+        keep the shape [B, N] / [B, T]: the columns beyond a row's own count are padding (status 0, energy 0,
+        ``targets_active`` 0, fitness 0, never written by the kernels).  All rows run on the thread count of the largest
+        scenario.  ``num_agent``, ``mc_type``, ``map_size`` and ``warm_up_time`` are the same for the whole batch.
         ``step_budget`` (``wrsn_dims.step_budget``, may be changed later through ``self.dims``): 0 = every ``step`` returns
         the environment's next request, as the reference does; > 0 = work units per launch and environment — a step that
         needs more comes back with ``agent_id == -4`` and continues at the next call, so one launch over thousands of
@@ -70,9 +75,7 @@ class BatchedWRSN:
         self.warm_up_time = float(warm_up_time)
         statics = [build_static(s, self.mc_type, self.warm_up_time) for s in self.scenarios]
         self.statics = statics
-        N, T = statics[0]["N"], statics[0]["T"]
-        if any(st["N"] != N or st["T"] != T for st in statics):
-            raise ValueError("all scenarios of a batch must have the same number of nodes and targets")
+        N, T = max(st["N"] for st in statics), max(st["T"] for st in statics)
         n_scen = len(statics)
         B = int(num_envs) if num_envs is not None else (len(scenario_index) if scenario_index is not None else n_scen)
         self.B, self.N, self.T, self.M, self.S = B, N, T, self.num_agent, self.map_size
@@ -98,6 +101,9 @@ class BatchedWRSN:
         if scenario_index is None:
             scenario_index = np.arange(B) % n_scen
         self.scen_id = torch.as_tensor(np.asarray(scenario_index, np.int32), device=self.device)
+        sid = np.asarray(scenario_index, np.int64)
+        self.num_nodes = torch.as_tensor(np.array([statics[k]["N"] for k in sid], np.int32), device=self.device)
+        self.num_targets = torch.as_tensor(np.array([statics[k]["T"] for k in sid], np.int32), device=self.device)
         self.state = torch.zeros((B, d.state_bytes), dtype=torch.uint8, device=self.device)
         self.req = Requests(B, self.device)
         self._all = None
@@ -281,7 +287,8 @@ class BatchedWRSN:
         return out
 
     def get_network_fitness(self):
-        """``WRSN.get_network_fitness`` (:188-220): per-target values [B, T] and their minimum [B]."""
+        """``WRSN.get_network_fitness`` (:188-220): per-target values [B, T] and their minimum [B] over each row's own
+        targets (columns beyond a row's own target count stay 0)."""
         fit = torch.zeros((self.B, max(self.T, 1)), dtype=torch.float64, device=self.device)
         mn = torch.zeros((self.B,), dtype=torch.float64, device=self.device)
         self._call(self.L.wrsn_fitness, C.byref(self.dims), self.scen.data_ptr(), self.scen_id.data_ptr(),
@@ -313,7 +320,8 @@ class BatchedWRSN:
         """The node x charger charging model, dense (``wrsn_k_charge``; ``Node.charger_connection`` ``Node.py:134-139`` over
         the ``connected_nodes`` of ``MobileCharger.charge`` ``MobileCharger.py:56-59``): the ``energyRR`` every alive node
         would receive [B, N] and the ``chargingRate`` every charger would draw [B, M] if the chargers selected by
-        ``charging`` (uint8 [B, M]; default all) charged at their present positions.  Does not touch the state."""
+        ``charging`` (uint8 [B, M]; default all) charged at their present positions.  Does not touch the state.  The columns
+        of [B, N] beyond a row's own node count are not written."""
         if out is not None:                              # (node [B, N], mc [B, max(M, 1)]) of an earlier call, reused
             node, mc = out[0], out[1] if out[1].shape[1] == max(self.M, 1) else None
         else:

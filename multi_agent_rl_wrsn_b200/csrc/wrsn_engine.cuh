@@ -177,7 +177,12 @@ enum {   /* program counter of a charger process slot */
 WRSN_D void ctx_bind(Ctx &c, const wrsn_dims &d, const WrsnLayout &L, const char *scen_row, char *state_row,
                      int tid, int G, uint32_t sbase = 0u) {
     c.tid = tid; c.G = G; c.work0 = 0;
-    c.N = d.N; c.T = d.T; c.M = d.M; c.W = d.W; c.Tw = d.Tw; c.Npad = d.Npad; c.n_slot = d.n_slot;
+    {   /* the scenario's own counts (d.N / d.T are the batch's largest), read from the GLOBAL row: the shared copy below is only
+           visible after the caller's first barrier */
+        const double *gpar = (const double *)(scen_row + L.soff[WRSN_S_PAR]);
+        c.N = (int)gpar[WRSN_P_NNODES]; c.T = (int)gpar[WRSN_P_NTARGETS];
+    }
+    c.M = d.M; c.W = d.W; c.Tw = d.Tw; c.Npad = d.Npad; c.n_slot = d.n_slot;
     c.scr_len = L.scr_len;
     c.hdr.off = sbase + (uint32_t)L.off[WRSN_F_HDR]; c.mc.off = sbase + (uint32_t)L.off[WRSN_F_MC]; c.proc.off = sbase + (uint32_t)L.off[WRSN_F_PROC];
     c.energy.off = sbase + (uint32_t)L.off[WRSN_F_ENERGY]; c.rr.off = sbase + (uint32_t)L.off[WRSN_F_RR]; c.cs.off = sbase + (uint32_t)L.off[WRSN_F_CS];
@@ -207,6 +212,13 @@ WRSN_D void ctx_bind(Ctx &c, const wrsn_dims &d, const WrsnLayout &L, const char
     c.nbr_idx = (const int32_t *)(scen_row + L.soff[WRSN_S_NBR_IDX]);
     c.tgt_idx = (const int32_t *)(scen_row + L.soff[WRSN_S_TGT_IDX]);
     c.direct = (const uint8_t *)(scen_row + L.soff[WRSN_S_DIRECT]);
+}
+
+/* the targets of word w of a target bitmask: Tw comes from the batch's largest scenario, so the trailing words of a smaller
+ * scenario hold no target (empty mask: neither active nor dead) */
+WRSN_DI uint32_t tact_word_mask(const Ctx &c, int w) {
+    const int bits = c.T - 32 * w;
+    return bits >= 32 ? 0xffffffffu : (bits <= 0 ? 0u : ((1u << bits) - 1u));
 }
 
 /* 32-bit shared-memory addressing for the hot loop: on the device an address is the byte offset inside the CTA's shared
@@ -686,9 +698,7 @@ WRSN_NOINLINE void do_bfs(Ctx &c) {
     /* alive = min(targets_active) */
     int dead_t = 0;
     for (int w = c.tid; w < c.Tw; w += WRSN_GSZ(c)) {
-        int bits = c.T - 32 * w; if (bits > 32) bits = 32;
-        uint32_t full = bits == 32 ? 0xffffffffu : ((1u << bits) - 1u);
-        if ((c.tact[w] & full) != full) dead_t = 1;
+        if ((c.tact[w] & tact_word_mask(c, w)) != tact_word_mask(c, w)) dead_t = 1;
     }
     dead_t = red_or(c, dead_t);
     build_tree(c);
@@ -2399,10 +2409,7 @@ WRSN_D void entry_init_network(Ctx &c, int with_reward) {
         c.logtick[i] = 0.0;
         for (int k = 0; k < WRSN_RING; k++) c.ring[(size_t)k * c.Npad + i] = 0.0;
     }
-    for (int w = c.tid; w < c.Tw; w += WRSN_GSZ(c)) {
-        int bits = c.T - 32 * w; if (bits > 32) bits = 32;
-        c.tact[w] = bits == 32 ? 0xffffffffu : ((1u << bits) - 1u);
-    }
+    for (int w = c.tid; w < c.Tw; w += WRSN_GSZ(c)) c.tact[w] = tact_word_mask(c, w);
     for (int w = c.tid; w < (c.M > 0 ? c.M : 1) * c.W; w += WRSN_GSZ(c)) c.conn[w] = 0u;
     for (int k = c.tid; k < WRSN_H_LEN; k += WRSN_GSZ(c)) c.hdr[k] = 0.0;
     for (int k = c.tid; k < (c.M > 0 ? c.M : 1) * WRSN_MC_LEN; k += WRSN_GSZ(c)) c.mc[k] = 0.0;

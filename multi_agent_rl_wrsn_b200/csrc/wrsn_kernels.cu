@@ -130,7 +130,7 @@ __global__ void k_obs_tables(const wrsn_dims d, const WrsnLayout L, char *scen) 
     const double x0 = (nx[n] - f0) / Wd, y0 = (ny[n] - f2) / Hd, hx = R / Wd, hy = R / Hd;
     for (int i = threadIdx.x; i < TP; i += blockDim.x) {
         const double cc = start + (double)i * delta, ux = cc - x0, uy = cc - y0;
-        const bool in = i < S && n < d.N;
+        const bool in = i < S && n < (int)par[WRSN_P_NNODES];
         gx[(size_t)n * TP + i] = in ? (float)exp(ux * ux / (-2.0 * (hx * hx))) : 0.f;
         gy[(size_t)n * TP + i] = in ? (float)exp(uy * uy / (-2.0 * (hy * hy))) : 0.f;
     }
@@ -142,7 +142,7 @@ template <typename AccT, int TJ, int THREADS>
 __global__ void __launch_bounds__(THREADS, sizeof(AccT) == 4 ? OBS_MINB32 : 1) k_observe(const KParams P, const int32_t *agent_id, AccT *obs) {
     constexpr int CH = sizeof(AccT) == 4 ? OBS_CH32 : 16;      /* sources staged per pass */
     extern __shared__ uint4 smem_u4[];
-    const int S = P.d.S, N = P.d.N, M = P.d.M, TP = P.d.obs_pitch;
+    const int S = P.d.S, M = P.d.M, TP = P.d.obs_pitch;
     const int tiles_i = (S + OBS_TI - 1) / OBS_TI, tiles_j = (S + TJ - 1) / TJ;
     AccT *gx = reinterpret_cast<AccT *>(smem_u4);                             /* [CH][TP] */
     AccT *gy = gx + CH * TP;                                                  /* [CH][TP] */
@@ -153,6 +153,7 @@ __global__ void __launch_bounds__(THREADS, sizeof(AccT) == 4 ? OBS_MINB32 : 1) k
     const char *row = P.state + (size_t)b * P.L.total;
     const char *scen_row = P.scen + (size_t)P.scen_id[b] * P.L.scen_total;
     const double *par = (const double *)(scen_row + P.L.soff[WRSN_S_PAR]);
+    const int N = (int)par[WRSN_P_NNODES];                                    /* this scenario's nodes (P.d.N: the batch's largest) */
     const double *nx = (const double *)(scen_row + P.L.soff[WRSN_S_NX]);
     const double *ny = (const double *)(scen_row + P.L.soff[WRSN_S_NY]);
     const double *energy = (const double *)(row + P.L.off[WRSN_F_ENERGY]);
@@ -347,18 +348,19 @@ struct WinSrc { int sx, sy; };       /* first row / column of the window; sx < -
 template <int OBW>                   /* window in cells (multiple of 4): >= 12.2 sigma + 6, chosen by the launcher */
 __global__ void __launch_bounds__(OBW_THREADS, OBW <= 40 ? 4 : (OBW <= 56 ? 3 : 2)) k_observe_win(const KParams P, const int32_t *agent_id, float *obs) {
     extern __shared__ uint4 smem_u4[];
-    const int S = P.d.S, N = P.d.N, M = P.d.M, TP = P.d.obs_pitch;
-    const int NS = N + 2 * M;                                   /* nodes | chargers as channel-3 sources | as channel-4 sources */
-    float *gxw = reinterpret_cast<float *>(smem_u4);            /* [NS][OBW] */
-    float *gyw = gxw + (size_t)NS * OBW;                        /* [NS][OBM + OBW + OBM] */
-    float *own = gyw + (size_t)NS * (OBW + 2 * OBM);            /* [2][TP]: the observer's own position, full width */
-    WinSrc *win = reinterpret_cast<WinSrc *>(own + 2 * TP);     /* [NS] */
+    const int S = P.d.S, M = P.d.M, TP = P.d.obs_pitch;
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
     const int ag = agent_id[b];
     if (ag < 0) return;
     const char *row = P.state + (size_t)b * P.L.total;
     const char *scen_row = P.scen + (size_t)P.scen_id[b] * P.L.scen_total;
     const double *par = (const double *)(scen_row + P.L.soff[WRSN_S_PAR]);
+    const int N = (int)par[WRSN_P_NNODES];                      /* this scenario's nodes (P.d.N, the batch's largest, sizes smem) */
+    const int NS = N + 2 * M;                                   /* nodes | chargers as channel-3 sources | as channel-4 sources */
+    float *gxw = reinterpret_cast<float *>(smem_u4);            /* [NS][OBW] */
+    float *gyw = gxw + (size_t)NS * OBW;                        /* [NS][OBM + OBW + OBM] */
+    float *own = gyw + (size_t)NS * (OBW + 2 * OBM);            /* [2][TP]: the observer's own position, full width */
+    WinSrc *win = reinterpret_cast<WinSrc *>(own + 2 * TP);     /* [NS] */
     const double *nx = (const double *)(scen_row + P.L.soff[WRSN_S_NX]);
     const double *ny = (const double *)(scen_row + P.L.soff[WRSN_S_NY]);
     const double *energy = (const double *)(row + P.L.off[WRSN_F_ENERGY]);
@@ -666,13 +668,14 @@ __global__ void __launch_bounds__(32 * LOC_WARPS) k_decode_locate(const KParams 
     const int b = blockIdx.x * LOC_WARPS + wrp;
     if (b >= P.d.B || agent_id[b] < 0) return;           /* whole warps leave together; only __syncwarp below */
     double *cn_x = s_cn[wrp][0], *cn_y = s_cn[wrp][1], *cn_w = s_cn[wrp][2];
-    const int S = P.d.S, N = P.d.N;
+    const int S = P.d.S;
     const int flat0 = (int)action[3 * (size_t)b];
     double out_x, out_y;
     {
         const char *row = P.state + (size_t)b * P.L.total;
         const char *scen_row = P.scen + (size_t)P.scen_id[b] * P.L.scen_total;
         const double *par = (const double *)(scen_row + P.L.soff[WRSN_S_PAR]);
+        const int N = (int)par[WRSN_P_NNODES];               /* this scenario's nodes */
         const double *nx = (const double *)(scen_row + P.L.soff[WRSN_S_NX]), *ny = (const double *)(scen_row + P.L.soff[WRSN_S_NY]);
         const double *energy = (const double *)(row + P.L.off[WRSN_F_ENERGY]), *cs = (const double *)(row + P.L.off[WRSN_F_CS]);
         const uint8_t *status = (const uint8_t *)(row + P.L.off[WRSN_F_STATUS]);
@@ -1024,10 +1027,11 @@ __global__ void __launch_bounds__(32 * CHG_WARPS) k_charge(const KParams P, cons
     const int wrp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int b = blockIdx.x * CHG_WARPS + wrp;
     if (b >= P.d.B) return;                                   /* whole warps leave together; only __syncwarp below */
-    const int N = P.d.N, M = P.d.M;
+    const int NP = P.d.N, M = P.d.M;                          /* node_rate's row pitch: the batch's largest node count */
     const char *row = P.state + (size_t)b * P.L.total;
     const char *scen_row = P.scen + (size_t)P.scen_id[b] * P.L.scen_total;
     const double *par = (const double *)(scen_row + P.L.soff[WRSN_S_PAR]);
+    const int N = (int)par[WRSN_P_NNODES];                    /* this scenario's nodes; node_rate[b][N..NP) is left untouched */
     const double *nx = (const double *)(scen_row + P.L.soff[WRSN_S_NX]), *ny = (const double *)(scen_row + P.L.soff[WRSN_S_NY]);
     const uint8_t *status = (const uint8_t *)(row + P.L.off[WRSN_F_STATUS]);
     const double *mc = (const double *)(row + P.L.off[WRSN_F_MC]);
@@ -1066,7 +1070,7 @@ __global__ void __launch_bounds__(32 * CHG_WARPS) k_charge(const KParams P, cons
                 __syncwarp();
             }
         }
-        if (n < N) node_rate[(size_t)b * N + n] = acc;
+        if (n < N) node_rate[(size_t)b * NP + n] = acc;
     }
     __syncwarp();
     for (int m = lane; m < M; m += 32) mc_rate[(size_t)b * M + m] = s_sum[wrp][m];

@@ -147,7 +147,7 @@ def build_static(sc, mc, warm_up_time=100.0):
                MC_AB2=mc["alpha"] / (mc["beta"] ** 2), MC_CAP200=mc["capacity"] / 200.0, MC_PMV=mc["pm"] * mc["velocity"],
                EPSENV=1e-9, CAPMTHR=cap - thr,
                ESMAX=max([float(spe["er"] * spe["package_size"])] + list(nbr_esend) + list(bs_esend)),
-               INVN=1.0 / float(N))
+               INVN=1.0 / float(N), NNODES=N, NTARGETS=T)
     return dict(N=N, T=T, x=x, y=y, nbr_ptr=nbr_ptr, nbr_idx=nbr_idx, nbr_dist=nbr_dist, nbr_esend=nbr_esend,
                 tgt_ptr=tgt_ptr, tgt_idx=tgt_idx, direct=direct, bs_esend=bs_esend,
                 par={k: float(v) for k, v in par.items()}, frame=np.array([f0, f1, f2, f3]), nodes_density=density)

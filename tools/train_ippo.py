@@ -6,6 +6,7 @@ YAML files (and, with ``--reference-networks``, its own network classes) are use
 
     python tools/train_ippo.py --envs 2048 --iterations 10
     python tools/train_ippo.py --reference-root /path/to/multi_agent_rl_wrsn --envs 2048 --iterations 1000
+    python tools/train_ippo.py --reference-root /path/to/multi_agent_rl_wrsn --scenario physical_env/network/network_scenarios/hanoi1000n{50,100,150,200}.yaml
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/train_ippo.py --envs 16384
 
 Under torchrun the ``--envs`` environments are split into contiguous blocks, one per rank / GPU (``sharding.shard_range``); the
@@ -30,7 +31,8 @@ def main():
     p.add_argument("--reference-root", default=None, help="checkout of the reference (its YAML files; its networks with --reference-networks)")
     p.add_argument("--reference-networks", action="store_true")
     p.add_argument("--step-budget", type=int, default=100)
-    p.add_argument("--scenario", default="physical_env/network/network_scenarios/hanoi1000n50.yaml")   # runner/IPPO.py:19
+    p.add_argument("--scenario", nargs="+", default=["physical_env/network/network_scenarios/hanoi1000n50.yaml"],   # runner/IPPO.py:19
+                   help="with --reference-root: one or several scenario files, of any sizes, assigned to the environments round robin")
     p.add_argument("--agent-type", default="physical_env/mc/mc_types/default.yaml")
     p.add_argument("--alg-args", default="alg_args/ippo.yaml")
     p.add_argument("--num-agent", type=int, default=3)
@@ -57,7 +59,7 @@ def main():
         ref = lambda rel: rel if os.path.isabs(rel) else os.path.join(a.reference_root, rel)
         with open(ref(a.alg_args)) as f:
             args = yaml.safe_load(f)["alg_args"]
-        scenarios, mc = [ref(a.scenario)], ref(a.agent_type)
+        scenarios, mc = [ref(s) for s in a.scenario], ref(a.agent_type)
         if a.reference_networks:
             sys.path.insert(0, a.reference_root)
             from controller.ppo.actor.UnetActor import UNet                # the reference's networks, unmodified
