@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define WRSN_ABI_VERSION 19
+#define WRSN_ABI_VERSION 20
 #define WRSN_MAX_MC 16          /* chargers per environment */
 #define WRSN_RING 10            /* Node.operate keeps the last 10 per-second consumptions (Node.py:70-77) */
 
@@ -173,12 +173,7 @@ typedef struct wrsn_dims {
                              events, fitness, deaths, cheap batches: everything but ...) and the batch kernel (... the
                              second-by-second loop of the seconds in which update_reward is active, at most step_budget of them
                              per launch).  Same results; the hot loop runs in launches of its own, where nothing else
-                             competes for the instruction caches.
-                             R < 0 (one warp per environment only; needs wrsn_request.queue; a measured experiment, slower than R = 0):
-                             ONE persistent launch, one CTA of sixteen warps per SM, every warp one environment at a time from a
-                             queue; the warps of an SM do the same KIND of work at the same time (event phase / batch phase, flipping
-                             when enough warps wait for the other one).  step_budget (0 = none) bounds the work per environment and
-                             launch as above.  Same results. */
+                             competes for the instruction caches.  R < 0 is rejected. */
 } wrsn_dims;
 
 /* request record written by reset / step, device pointers, one row per environment */
@@ -198,8 +193,6 @@ typedef struct wrsn_request {
     int32_t *order;                     /* [B]  scratch of wrsn_step / wrsn_rollout_step (may be NULL): the order in which the step kernel's CTAs take the
                                            rows — longest predicted step first (time to the earliest charger's next decision, read from the
                                            process slots and the new actions), so that the launch does not end on a late, long environment */
-    int32_t *queue;                     /* [2]  work queue of the persistent step kernel (wrsn_dims.step_rounds < 0): zeroed once by the caller,
-                                           left zeroed by every launch; may be NULL otherwise.  One per request record (= per stream). */
 } wrsn_request;
 
 const char *wrsn_last_error(void);

@@ -25,7 +25,7 @@ class Dims(C.Structure):
 
 class Request(C.Structure):
     _fields_ = [("agent_id", C.c_void_p), ("terminal", C.c_void_p), ("reward", C.c_void_p), ("now", C.c_void_p),
-                ("action", C.c_void_p), ("detail", C.c_void_p), ("flags", C.c_void_p), ("stats", C.c_void_p), ("sticky", C.c_void_p), ("order", C.c_void_p), ("queue", C.c_void_p)]
+                ("action", C.c_void_p), ("detail", C.c_void_p), ("flags", C.c_void_p), ("stats", C.c_void_p), ("sticky", C.c_void_p), ("order", C.c_void_p)]
 
 
 def enums():

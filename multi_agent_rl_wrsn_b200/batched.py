@@ -41,10 +41,9 @@ class Requests:
         self.stats = torch.zeros((B, 3), dtype=torch.float64, device=device)   # running totals: decisions, simulated seconds, resets
         self.sticky = torch.zeros((B,), dtype=torch.int32, device=device)      # OR of every `flags` value written so far (see raise_on_error)
         self.order = torch.zeros((B,), dtype=torch.int32, device=device)       # scratch: launch order of the step kernel's CTAs (longest step first)
-        self.queue = torch.zeros((2,), dtype=torch.int32, device=device)       # work queue of the persistent step kernel (step_rounds < 0)
         self.c = _lib.Request(self.agent_id.data_ptr(), self.terminal.data_ptr(), self.reward.data_ptr(),
                               self.now.data_ptr(), self.action.data_ptr(), self.detail.data_ptr(), self.flags.data_ptr(),
-                              self.stats.data_ptr(), self.sticky.data_ptr(), self.order.data_ptr(), self.queue.data_ptr())
+                              self.stats.data_ptr(), self.sticky.data_ptr(), self.order.data_ptr())
 
 
 class BatchedWRSN:
@@ -63,7 +62,7 @@ class BatchedWRSN:
         environments lasts as long as the budget instead of as long as its slowest environment.
         ``step_rounds`` (``wrsn_dims.step_rounds``, with a budget): R > 0 cuts a step by kind of work as well — R rounds of
         two launches per call, the events kernel and the batch kernel that holds nothing but the hot second-by-second
-        loop (same results, better instruction-cache behaviour; see include/wrsn_b200.h)."""
+        loop (same results, better instruction-cache behaviour; see include/wrsn_b200.h).  R < 0 is rejected."""
         self.L = _lib.lib()
         self.device = self._require_device(device)
         if isinstance(scenarios, (str, Scenario)):

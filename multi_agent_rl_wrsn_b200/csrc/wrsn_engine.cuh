@@ -139,8 +139,9 @@ struct SArr {
 
 struct Ctx {
     int tid, G;
-    int work0;                                       /* work units this environment has spent in the current launch before the running
-                                                        call (k_env_sync calls run_loop / run_batches several times per launch) */
+    SArr<double> spec;                               /* [WRSN_SPEC_MAX][WRSN_SPEC_LEN] irregular nodes of the current batch.  First: every
+                                                        other field then sits at the offset at which ptxas allocates the cold entry
+                                                        points (fitness, BFS) without extra registers (-Xptxas -v) */
     int N, T, M, W, Tw, Npad, n_slot, scr_len;
     /* shared-memory image */
     SArr<double> hdr, mc, proc;
@@ -155,7 +156,6 @@ struct Ctx {
     SArr<double> par;                                /* scenario constants, copied next to the state */
     SArr<double> pairs;                              /* see wrsn_layout.h: s_pairs */
     SArr<double> exptab;                             /* 2^(j/64), j = 0..63 (wrsn_exp_b) */
-    SArr<double> spec;                               /* [WRSN_SPEC_MAX][WRSN_SPEC_LEN] irregular nodes of the current batch */
     /* global, per environment */
     double *logtick, *ring;
     char *gscratch;
@@ -173,10 +173,8 @@ enum {   /* program counter of a charger process slot */
     PC_CH_DONE, PC_OP_DONE
 };
 
-/* `sbase`: byte offset of this environment's image inside the CTA's dynamic shared memory (k_env_sync keeps one image per warp) */
-WRSN_D void ctx_bind(Ctx &c, const wrsn_dims &d, const WrsnLayout &L, const char *scen_row, char *state_row,
-                     int tid, int G, uint32_t sbase = 0u) {
-    c.tid = tid; c.G = G; c.work0 = 0;
+WRSN_D void ctx_bind(Ctx &c, const wrsn_dims &d, const WrsnLayout &L, const char *scen_row, char *state_row, int tid, int G) {
+    c.tid = tid; c.G = G;
     {   /* the scenario's own counts (d.N / d.T are the batch's largest), read from the GLOBAL row: the shared copy below is only
            visible after the caller's first barrier */
         const double *gpar = (const double *)(scen_row + L.soff[WRSN_S_PAR]);
@@ -184,14 +182,14 @@ WRSN_D void ctx_bind(Ctx &c, const wrsn_dims &d, const WrsnLayout &L, const char
     }
     c.M = d.M; c.W = d.W; c.Tw = d.Tw; c.Npad = d.Npad; c.n_slot = d.n_slot;
     c.scr_len = L.scr_len;
-    c.hdr.off = sbase + (uint32_t)L.off[WRSN_F_HDR]; c.mc.off = sbase + (uint32_t)L.off[WRSN_F_MC]; c.proc.off = sbase + (uint32_t)L.off[WRSN_F_PROC];
-    c.energy.off = sbase + (uint32_t)L.off[WRSN_F_ENERGY]; c.rr.off = sbase + (uint32_t)L.off[WRSN_F_RR]; c.cs.off = sbase + (uint32_t)L.off[WRSN_F_CS];
-    c.esend.off = sbase + (uint32_t)L.off[WRSN_F_ESEND]; c.logc.off = sbase + (uint32_t)L.off[WRSN_F_LOGC];
-    c.nbef.off = sbase + (uint32_t)L.off[WRSN_F_NBEF]; c.naft.off = sbase + (uint32_t)L.off[WRSN_F_NAFT];
-    c.level.off = sbase + (uint32_t)L.off[WRSN_F_LEVEL]; c.parent.off = sbase + (uint32_t)L.off[WRSN_F_PARENT];
-    c.status.off = sbase + (uint32_t)L.off[WRSN_F_STATUS]; c.tact.off = sbase + (uint32_t)L.off[WRSN_F_TACT]; c.conn.off = sbase + (uint32_t)L.off[WRSN_F_CONN];
-    c.own.off = sbase + (uint32_t)L.s_own; c.scr0.off = sbase + (uint32_t)L.s_scr0; c.scr1.off = sbase + (uint32_t)L.s_scr1;
-    c.bcast.off = sbase + (uint32_t)L.s_bcast; c.red.off = sbase + (uint32_t)L.s_red; c.par.off = sbase + (uint32_t)L.s_par; c.spec.off = sbase + (uint32_t)L.s_spec; c.exptab.off = sbase + (uint32_t)L.s_exptab; c.pairs.off = sbase + (uint32_t)L.s_pairs;
+    c.hdr.off = (uint32_t)L.off[WRSN_F_HDR]; c.mc.off = (uint32_t)L.off[WRSN_F_MC]; c.proc.off = (uint32_t)L.off[WRSN_F_PROC];
+    c.energy.off = (uint32_t)L.off[WRSN_F_ENERGY]; c.rr.off = (uint32_t)L.off[WRSN_F_RR]; c.cs.off = (uint32_t)L.off[WRSN_F_CS];
+    c.esend.off = (uint32_t)L.off[WRSN_F_ESEND]; c.logc.off = (uint32_t)L.off[WRSN_F_LOGC];
+    c.nbef.off = (uint32_t)L.off[WRSN_F_NBEF]; c.naft.off = (uint32_t)L.off[WRSN_F_NAFT];
+    c.level.off = (uint32_t)L.off[WRSN_F_LEVEL]; c.parent.off = (uint32_t)L.off[WRSN_F_PARENT];
+    c.status.off = (uint32_t)L.off[WRSN_F_STATUS]; c.tact.off = (uint32_t)L.off[WRSN_F_TACT]; c.conn.off = (uint32_t)L.off[WRSN_F_CONN];
+    c.own.off = (uint32_t)L.s_own; c.scr0.off = (uint32_t)L.s_scr0; c.scr1.off = (uint32_t)L.s_scr1;
+    c.bcast.off = (uint32_t)L.s_bcast; c.red.off = (uint32_t)L.s_red; c.par.off = (uint32_t)L.s_par; c.spec.off = (uint32_t)L.s_spec; c.exptab.off = (uint32_t)L.s_exptab; c.pairs.off = (uint32_t)L.s_pairs;
     c.logtick = (double *)(state_row + L.off[WRSN_F_LOGTICK]);
     c.ring = (double *)(state_row + L.off[WRSN_F_RING]);
     c.gscratch = state_row + L.off[WRSN_F_SCRATCH];
@@ -2274,7 +2272,7 @@ WRSN_D bool any_watched(Ctx &c) {                   /* a lazy move whose positio
 WRSN_DI int run_loop(Ctx &c, int budget, int split) {
     Clk k;
     clk_load(c, k);
-    k.work = c.work0;
+    k.work = 0;
     const double maxtime = c.par[WRSN_P_MAXTIME];
     bool rescan = true;
     int interrupted = 0;
@@ -2358,7 +2356,6 @@ WRSN_DI int run_loop(Ctx &c, int budget, int split) {
     catch_up_many(c, k.now, 1);
     WRSN_PROFB_END(c, WRSN_H_PROF2); }
     clk_store(c, k);
-    c.work0 = k.work;
     return interrupted;
 }
 
@@ -2369,7 +2366,7 @@ WRSN_DI int run_loop(Ctx &c, int budget, int split) {
 WRSN_DI int run_batches(Ctx &c, int budget) {
     Clk k;
     clk_load(c, k);
-    k.work = c.work0;
+    k.work = 0;
     mc_scan(c, k);                                   /* (nothing in here moves a charger event) */
     const double maxtime = c.par[WRSN_P_MAXTIME];
     int ret = 1;
@@ -2392,7 +2389,6 @@ WRSN_DI int run_batches(Ctx &c, int budget) {
         batch_commit(k, gt, batched);
     }
     clk_store(c, k);
-    c.work0 = k.work;
     return ret;
 }
 

@@ -1,5 +1,6 @@
-/* wrsn_env_kernel.cuh — the one-CTA-per-environment kernel; included once per group-size specialisation (see
- * wrsn_engine.cuh), inside the same namespace. */
+/* wrsn_env_kernel.cuh — one environment for one launch (env_run) and the one-CTA-per-environment kernel around it; included
+ * once per group-size specialisation (see wrsn_engine.cuh), inside the same namespace, and once by the host emulation, whose
+ * launcher calls env_run row by row on one lane. */
 #ifndef WRSN_GANY_MINB
 #define WRSN_GANY_MINB 2                            /* CTAs per SM the multi-warp build is compiled for: 128 registers (a few hundred bytes of spills)
                                                        instead of 238 — 1000 nodes / 10 chargers 0.046 -> 0.074 M decisions/s, 500 / 5 0.269 -> 0.340 M */
@@ -8,10 +9,48 @@
 #define WRSN_G32_MINB 16                            /* CTAs per SM the one-warp build is compiled for (128 registers; measured: 18 CTAs at 96 registers
                                                        and 0.7 KB of spills is 3 % slower, shared memory allows no more than 18) */
 #endif
+
+/* bytes: a multiple of 16 */
+WRSN_DI void copy16(char *dst, const char *src, int64_t bytes, int tid, int G) {
+#if defined(WRSN_HOST_EMU)
+    (void)tid; (void)G;
+    memcpy(dst, src, (size_t)bytes);
+#else
+    const uint4 *s = reinterpret_cast<const uint4 *>(src);
+    uint4 *d = reinterpret_cast<uint4 *>(dst);
+    const int n = (int)(bytes >> 4);
+    for (int i = tid; i < n; i += G) d[i] = s[i];
+#endif
+}
+
+WRSN_DI void zero16(char *dst, int64_t bytes, int tid, int G) {
+#if defined(WRSN_HOST_EMU)
+    (void)tid; (void)G;
+    memset(dst, 0, (size_t)bytes);
+#else
+    uint4 *z = reinterpret_cast<uint4 *>(dst);
+    for (int i = tid; i < (int)(bytes >> 4); i += G) z[i] = make_uint4(0u, 0u, 0u, 0u);
+#endif
+}
+
+WRSN_DI void write_request(const wrsn_request &q, int b, const ReqOut &r) {
+    if (q.agent_id) q.agent_id[b] = r.agent;
+    if (q.terminal) q.terminal[b] = (uint8_t)r.terminal;
+    if (q.reward) q.reward[b] = r.reward;
+    if (q.now) q.now[b] = r.now;
+    if (q.action) for (int k = 0; k < 3; k++) q.action[3 * b + k] = r.act[k];
+    if (q.detail) { q.detail[2 * b] = r.detail[0]; q.detail[2 * b + 1] = r.detail[1]; }
+    if (q.flags) q.flags[b] = r.flags;
+    if (q.sticky && r.flags) q.sticky[b] |= r.flags;
+}
+
+/* Row `blk` of the launch (the CTA index; MODE_STEP maps it through P.order) on threads tid = 0 .. G-1: select the row, load its
+ * image into shared memory, run the mode's entry point, write the image back and, for the modes that hand out a request, the
+ * request record and the running totals. */
 template <int MODE>
-__global__ void __launch_bounds__(WRSN_GFIX ? WRSN_GFIX : 256, WRSN_GFIX ? WRSN_G32_MINB : WRSN_GANY_MINB) k_env(const KParams P) {
-    char *smem = reinterpret_cast<char *>(wrsn_smem_u4);
-    const int b = (MODE == MODE_STEP && P.order) ? P.order[blockIdx.x] : (int)blockIdx.x, tid = threadIdx.x, G = blockDim.x;
+WRSN_DI void env_run(const KParams &P, int blk, int tid, int G) {
+    char *smem = WRSN_SMEM_BASE;
+    const int b = (MODE == MODE_STEP && P.order) ? P.order[blk] : blk;
     if (P.mask && !P.mask[b]) return;
     if (P.mask_mode == 1 && P.req.agent_id[b] < 0 && P.req.agent_id[b] != -4) return;     /* (-4: a step in flight continues) */
     if (P.mask_mode == 2 && (P.req.agent_id[b] >= 0 || P.req.agent_id[b] == -4)) return;
@@ -32,14 +71,13 @@ __global__ void __launch_bounds__(WRSN_GFIX ? WRSN_GFIX : 256, WRSN_GFIX ? WRSN_
     } else if (MODE != MODE_INIT) {
         copy16(smem, row, P.L.resident, tid, G);
     } else {                                         /* alignment gaps between the fields: defined bytes in the record */
-        uint4 *z = reinterpret_cast<uint4 *>(smem);
-        for (int i = tid; i < (int)(P.L.resident >> 4); i += G) z[i] = make_uint4(0u, 0u, 0u, 0u);
+        zero16(smem, P.L.resident, tid, G);
     }
     for (int i = tid; i < c.Npad; i += G) c.own[i] = i < c.N ? (uint16_t)(c.tgt_ptr[i + 1] - c.tgt_ptr[i]) : (uint16_t)0;
     gsync(c);
 
     const double now_before = c.hdr[WRSN_H_NOW];
-#if defined(WRSN_PROF)
+#if defined(WRSN_PROF) && !defined(WRSN_HOST_EMU)
     const long long prof_start = clock64();
     if (MODE == MODE_STEP) { gsync(c); if (tid == 0) for (int q = WRSN_H_PROF0; q <= WRSN_H_PROF4; q++) c.hdr[q] = 0.0; gsync(c); }
 #endif
@@ -64,7 +102,7 @@ __global__ void __launch_bounds__(WRSN_GFIX ? WRSN_GFIX : 256, WRSN_GFIX ? WRSN_
     case MODE_K_REWARD: ev_update_reward(c); break;
     }
     gsync(c);
-#if defined(WRSN_PROF)
+#if defined(WRSN_PROF) && !defined(WRSN_HOST_EMU)
     if (MODE == MODE_STEP) { if (tid == 0) c.hdr[WRSN_H_PROF0] = (double)(clock64() - prof_start); gsync(c); }
 #endif
     if (MODE != MODE_FITNESS) copy16(row, smem, P.L.resident, tid, G);
@@ -78,108 +116,9 @@ __global__ void __launch_bounds__(WRSN_GFIX ? WRSN_GFIX : 256, WRSN_GFIX ? WRSN_
     }
 }
 
-
-#if WRSN_GFIX == 32
-/* k_env_sync — WRSN.step for the whole batch in ONE persistent launch whose SMs work phase by phase (wrsn_dims.step_rounds < 0).
- * A MEASURED EXPERIMENT, kept as an option (profiles/r02_icache.md): it proves what bounds the step kernel, and it is slower.
- *
- * A step is two kinds of work — the event machinery (charger state machines, closed-form batches, BFS, death ticks, fitness,
- * request: > 100 KB of code, little of it reused) and the second-by-second loop of the seconds in which update_reward is active
- * (16 KB, half of the executed instructions).  With one independent CTA per environment an SM holds sixteen environments in
- * sixteen different places of that code: its instruction caches hit 56 % and `no_instruction` is half of all stall cycles.
- * Here one CTA of WRSN_SYNC_WARPS warps stays on its SM, each warp owns one environment at a time (its own slice of shared
- * memory) and takes the next one from a queue when it is done; and the CTA is in ONE phase at a time: phase E, every warp whose
- * environment needs event work runs it (entry_step with split = 1 stops in front of a batch of the active kind); phase B, every
- * warp whose environment stands in front of such a batch runs it (entry_batches), a quantum of simulated seconds at a time.  A
- * warp whose environment needs the other phase parks at the CTA barrier; the phase flips when `th` warps are parked (or nobody
- * wants the current one).  Measured on 4096 environments: instruction-cache hits 56 % -> 82 %, `no_instruction` 11.3 -> 1.6 stall
- * cycles per issued instruction, every other stall reason unchanged — and 24.9 cycles per issue parked at the barrier, because
- * the lengths of the pieces vary too much for sixteen warps to stay in step: 2.6 ms against 1.7 ms per launch.
- * Same results as the other shapes of the step (tests/test_gpu_parity.py::test_phase_synchronous_step_kernel). */
-#define WRSN_SYNC_WARPS 16
-__global__ void __launch_bounds__(32 * WRSN_SYNC_WARPS, 1) k_env_sync(const KParams P) {
-    __shared__ int s_phase, s_nother, s_th, s_alldone, s_want[WRSN_SYNC_WARPS];
-    const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
-    const uint32_t sbase = (uint32_t)wrp * (uint32_t)P.sync_slice;
-    char *smem = reinterpret_cast<char *>(wrsn_smem_u4) + sbase;
-    if (threadIdx.x == 0) { s_phase = 0; s_nother = 0; s_th = (WRSN_SYNC_WARPS * P.sync_th + 15) / 16; s_alldone = 0; }
-    __syncthreads();
-    const int budget = P.d.step_budget > 0 ? P.d.step_budget : (1 << 30);
-    Ctx c;
-    ReqOut r;
-    int b = -1, want = 2;                           /* want: 0 event work, 1 batch work, 2 no environment */
-    bool exhausted = false;
-    double now_before = 0.0;
-    char *row = nullptr;
-    for (;;) {
-        while (want == 2 && !exhausted) {           /* take the next environment of the launch */
-            int nb = 0;
-            if (lane == 0) nb = atomicAdd(P.req.queue, 1);
-            nb = __shfl_sync(0xffffffffu, nb, 0);
-            if (nb >= P.d.B) { exhausted = true; break; }
-            if (P.mask && !P.mask[nb]) continue;
-            const int aid = P.req.agent_id ? P.req.agent_id[nb] : 0;
-            if (P.mask_mode == 1 && aid < 0 && aid != -4) continue;
-            b = nb;
-            row = P.state + (size_t)b * P.L.total;
-            ctx_bind(c, P.d, P.L, P.scen + (size_t)P.scen_id[b] * P.L.scen_total, row, lane, 32, sbase);
-            copy16(smem, row, P.L.resident, lane, 32);
-            for (int i = lane; i < c.Npad; i += 32) c.own[i] = i < c.N ? (uint16_t)(c.tgt_ptr[i + 1] - c.tgt_ptr[i]) : (uint16_t)0;
-            __syncwarp();
-            now_before = c.hdr[WRSN_H_NOW];
-            want = (aid == -4 && c.hdr[WRSN_H_INFLIGHT] == 2.0) ? 1 : 0;
-        }
-        const int phase = *(volatile int *)&s_phase;
-        if (want == phase) {
-            r.agent = -3; r.terminal = 0; r.reward = 0; r.now = 0; r.flags = 0;
-            r.act[0] = r.act[1] = r.act[2] = 0; r.detail[0] = r.detail[1] = 0;
-            if (want == 0) entry_step(c, P.agent_in ? P.agent_in[b] : -1, P.action_in ? P.action_in + 3 * (size_t)b : nullptr, &r, budget, 1);
-            else { const int q = c.work0 + P.sync_quantum; entry_batches(c, &r, q < budget ? q : budget); }
-            __syncwarp();
-            bool finished = true;
-            if (__shfl_sync(0xffffffffu, r.agent, 0) == -4) {   /* (the entry points fill the request record in lane 0 only) */
-                /* interrupted: in front of a batch (2), by the budget (1), or — batches — at an event (1) */
-                const int code = (int)c.hdr[WRSN_H_INFLIGHT];
-                if (c.work0 < budget) { finished = false; want = code == 2 ? 1 : 0; }
-            }
-            if (finished) {
-                copy16(row, smem, P.L.resident, lane, 32);
-                if (lane == 0) {
-                    write_request(P.req, b, r);
-                    if (P.req.stats) {
-                        if (r.agent >= 0) P.req.stats[3 * b] += 1.0;
-                        P.req.stats[3 * b + 1] += r.now - now_before;
-                    }
-                }
-                __syncwarp();
-                want = 2;
-                continue;                            /* next environment (taken in whatever phase the CTA is in) */
-            }
-            if (want == phase && *(volatile int *)&s_nother < *(volatile int *)&s_th) continue;
-        }
-        /* park: this warp needs the other phase, has nothing left, or enough others are waiting for the other phase */
-        if (lane == 0) {
-            s_want[wrp] = want;
-            if (want != 2 && want != phase) atomicAdd(&s_nother, 1);
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            int n0 = 0, n1 = 0;
-            for (int w = 0; w < WRSN_SYNC_WARPS; w++) { n0 += s_want[w] == 0; n1 += s_want[w] == 1; }
-            const int active = n0 + n1, cur = s_phase;
-            const int n_other = cur ? n0 : n1, n_cur = active - n_other;
-            int th = (active * P.sync_th + 15) / 16; if (th < 1) th = 1;
-            if (active == 0) s_alldone = 1;
-            else if (n_cur == 0 || n_other >= th) s_phase = cur ^ 1;
-            s_th = th; s_nother = 0;
-        }
-        __syncthreads();
-        if (s_alldone) break;
-    }
-    /* the queue is ready for the next launch once every CTA has left it */
-    if (threadIdx.x == 0) {
-        __threadfence();
-        if (atomicAdd(P.req.queue + 1, 1) == (int)gridDim.x - 1) { P.req.queue[0] = 0; P.req.queue[1] = 0; __threadfence(); }
-    }
+#if !defined(WRSN_HOST_EMU)
+template <int MODE>
+__global__ void __launch_bounds__(WRSN_GFIX ? WRSN_GFIX : 256, WRSN_GFIX ? WRSN_G32_MINB : WRSN_GANY_MINB) k_env(const KParams P) {
+    env_run<MODE>(P, (int)blockIdx.x, threadIdx.x, blockDim.x);
 }
 #endif

@@ -9,53 +9,10 @@
 #include <stdio.h>
 #include <stdlib.h>
 
-#include "wrsn_layout.h"
+#include "wrsn_launch.h"
 
-static thread_local char g_err[512] = "";
 #define WRSN_MAX_DEVICES 64
-#define WRSN_FAIL(...) do { snprintf(g_err, sizeof(g_err), __VA_ARGS__); return -1; } while (0)
 #define WRSN_CUDA(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) WRSN_FAIL("%s: %s", #x, cudaGetErrorString(e_)); } while (0)
-
-enum { MODE_INIT = 0, MODE_RUN_UNTIL, MODE_RESET_FINISH, MODE_RESTORE_RESET, MODE_STEP, MODE_FITNESS, MODE_K_BFS,
-       MODE_K_DRAIN, MODE_K_BOOK, MODE_K_REWARD, MODE_STEP_BATCH };
-
-struct KParams {
-    wrsn_dims d;
-    WrsnLayout L;
-    const char *scen;
-    const int32_t *scen_id;
-    char *state;
-    const char *snap;
-    const uint8_t *mask;
-    int mask_mode;                                   /* 0: mask[] (or all); 1: rows with req.agent_id >= 0; 2: rows with req.agent_id < 0 */
-    const double *t_until;
-    const int32_t *agent_in;
-    const double *action_in;
-    wrsn_request req;
-    double *fitness, *fit_min;
-    int with_reward;
-    int resume_only;                                 /* later rounds of a split step: only rows whose step is in flight (agent_id == -4) */
-    const int32_t *order;                            /* MODE_STEP: row taken by CTA k (k_step_order), or NULL = k */
-    int sync_slice, sync_th, sync_quantum;           /* k_env_sync: bytes of shared memory per warp, parked sixteenths that flip the phase, seconds per batch quantum */
-};
-
-__device__ __forceinline__ void copy16(char *dst, const char *src, int64_t bytes, int tid, int G) {
-    const uint4 *s = reinterpret_cast<const uint4 *>(src);
-    uint4 *d = reinterpret_cast<uint4 *>(dst);
-    const int n = (int)(bytes >> 4);
-    for (int i = tid; i < n; i += G) d[i] = s[i];
-}
-
-__device__ __forceinline__ void write_request(const wrsn_request &q, int b, const ReqOut &r) {
-    if (q.agent_id) q.agent_id[b] = r.agent;
-    if (q.terminal) q.terminal[b] = (uint8_t)r.terminal;
-    if (q.reward) q.reward[b] = r.reward;
-    if (q.now) q.now[b] = r.now;
-    if (q.action) for (int k = 0; k < 3; k++) q.action[3 * b + k] = r.act[k];
-    if (q.detail) { q.detail[2 * b] = r.detail[0]; q.detail[2 * b + 1] = r.detail[1]; }
-    if (q.flags) q.flags[b] = r.flags;
-    if (q.sticky && r.flags) q.sticky[b] |= r.flags;
-}
 
 /* 2^(j/64), j = 0..63, correctly rounded: the table of wrsn_exp_b (wrsn_engine.cuh; reward path only) */
 __device__ const double wrsn_exp2_tab[64] = {
@@ -100,12 +57,9 @@ namespace gany {                                     /* 64 ... 256 threads per e
  * IN SOURCE ORDER.  AccT = double: multiply and add rounded separately, exactly the reference's `map += w*gx*gy`
  * (parity path, float64 out).  AccT = float: the vectors are rounded to fp32 once and accumulated with FFMA (the
  * observation the policy networks consume is float32; error ~1e-6 of the channel maximum). */
-#define OBS_TI 4
-#define OBS_TJ64 10                 /* fp64 parity raster: 4 x 10 tiles, 256 threads */
-#define OBS_THREADS64 256
-#ifndef OBS_TJ32
-#define OBS_TJ32 20                 /* fp32 raster: 4 x 20 tiles, 128 threads */
-#define OBS_THREADS32 128
+#define OBS_THREADS64 256           /* fp64 parity raster: 4 x 10 tiles (OBS_TI x OBS_TJ64, wrsn_layout.h) */
+#ifndef OBS_THREADS32
+#define OBS_THREADS32 128           /* fp32 raster: 4 x 20 tiles (OBS_TI x OBS_TJ32) */
 #endif
 #ifndef OBS_CH32
 #define OBS_CH32 32                 /* sources staged per pass (fp32 raster) */
@@ -766,123 +720,6 @@ __global__ void __launch_bounds__(32 * LOC_WARPS) k_decode_locate(const KParams 
     if (lane == 0) { action[3 * (size_t)b] = out_x; action[3 * (size_t)b + 1] = out_y; }
 }
 
-/* ------------------------------------------------------------------ host side of the C ABI */
-static int check_dims(const wrsn_dims *d) {
-    if (!d) WRSN_FAIL("dims is NULL");
-    if (d->N <= 0 || d->N > 32000 || d->T < 0 || d->T > 65000 || d->M < 0 || d->M > WRSN_MAX_MC || d->B <= 0 || d->S <= 0)
-        WRSN_FAIL("bad dims N=%d T=%d M=%d B=%d S=%d", d->N, d->T, d->M, d->B, d->S);
-    if (d->Npad < d->N || (d->Npad & 15) || d->state_bytes <= 0) WRSN_FAIL("dims not finalized (call wrsn_dims_finalize)");
-    /* the register-resident per-node loops hold at most 4 (one warp) / 9 (several warps) nodes per thread */
-    if (d->threads < 32 || d->threads % 32 || d->threads > 256 || (int64_t)d->N > (int64_t)d->threads * (d->threads == 32 ? 4 : 9))
-        WRSN_FAIL("threads = %d cannot hold N = %d nodes (at most %d per thread)", d->threads, d->N, d->threads == 32 ? 4 : 9);
-    return 0;
-}
-
-extern "C" {
-
-const char *wrsn_last_error(void) { return g_err; }
-int wrsn_abi_version(void) { return WRSN_ABI_VERSION; }
-int wrsn_field_count(int which) {
-    switch (which) {
-    case 0: return WRSN_P_LEN; case 1: return WRSN_H_LEN; case 2: return WRSN_MC_LEN; case 3: return WRSN_PR_LEN;
-    case 4: return WRSN_F_COUNT; case 5: return WRSN_S_COUNT; default: return -1;
-    }
-}
-
-int wrsn_dims_finalize(wrsn_dims *d) {
-    if (!d) WRSN_FAIL("dims is NULL");
-    d->Npad = (d->N + 15) & ~15;
-    d->W = (d->N + 31) / 32;
-    d->Tw = (d->T + 31) / 32; if (d->Tw < 1) d->Tw = 1;
-    d->n_slot = d->M + 3;
-    if (d->Emax < 1) d->Emax = 1;
-    if (d->TEmax < 1) d->TEmax = 1;
-    if (d->threads <= 0) {
-        int per = (d->N + 3) / 4;                    /* about four nodes per thread: 100 nodes run on ONE warp (measured on the
-                                                        RandomController workload: 1.08 M decisions/s against 0.88 M on two
-                                                        warps — no block-wide barriers, no shared-memory reductions, and the
-                                                        per-second loops keep four independent chains per lane in flight) */
-        int t = 32; while (t < per && t < 128) t *= 2;    /* above 128 nodes: at most four warps, then up to nine nodes per thread
-                                                        (measured, RandomController law, 2 CTAs per SM: 1000 nodes 0.079 M decisions/s on
-                                                        128 threads against 0.074 M on 256; 500 nodes 0.340 M on 128 against 0.287 M on 64) */
-        if (d->N > 9 * t) t = 256;
-        d->threads = t;
-    }
-    if (d->threads % 32 || d->threads > 256) WRSN_FAIL("threads must be a multiple of 32, at most 256");
-    if ((int64_t)d->N > (int64_t)d->threads * (d->threads == 32 ? 4 : 9))
-        WRSN_FAIL("threads = %d cannot hold N = %d nodes (at most %d per thread)", d->threads, d->N, d->threads == 32 ? 4 : 9);
-    {
-        const int ti = (d->S + OBS_TI - 1) / OBS_TI;
-        const int tj = (d->S + OBS_TJ64 - 1) / OBS_TJ64, tk = (d->S + OBS_TJ32 - 1) / OBS_TJ32;
-        const int pk = (tk * OBS_TJ32 + 3) & ~3;
-        int pi = ti * OBS_TI, pj = (tj * OBS_TJ64 + 3) & ~3;
-        if (pk > pj) pj = pk;
-        d->obs_pitch = pi > pj ? pi : pj;
-    }
-    WrsnLayout L;
-    wrsn_make_layout(d, &L);
-    d->state_bytes = (int32_t)L.total; d->state_resident_bytes = (int32_t)L.resident;
-    d->scen_bytes = (int32_t)L.scen_total; d->smem_bytes = (int32_t)L.smem_total;
-    if (L.smem_total > 227 * 1024) WRSN_FAIL("environment does not fit shared memory (%lld bytes)", (long long)L.smem_total);
-    return 0;
-}
-
-int wrsn_state_layout(const wrsn_dims *d, int64_t *offsets) {
-    if (check_dims(d)) return -1;
-    WrsnLayout L; wrsn_make_layout(d, &L);
-    for (int k = 0; k < WRSN_F_COUNT; k++) offsets[k] = L.off[k];
-    return 0;
-}
-int wrsn_scen_layout(const wrsn_dims *d, int64_t *offsets) {
-    if (check_dims(d)) return -1;
-    WrsnLayout L; wrsn_make_layout(d, &L);
-    for (int k = 0; k < WRSN_S_COUNT; k++) offsets[k] = L.soff[k];
-    return 0;
-}
-
-int wrsn_device_ok(void) {
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) { cudaGetLastError(); snprintf(g_err, sizeof(g_err), "no CUDA device"); return 0; }
-    int dev = 0; cudaGetDevice(&dev);
-    cudaDeviceProp p;
-    if (cudaGetDeviceProperties(&p, dev) != cudaSuccess) return 0;
-    if (p.major != 10) { snprintf(g_err, sizeof(g_err), "device is sm_%d%d, this library is built for sm_100a only", p.major, p.minor); return 0; }
-    return 1;
-}
-
-}  /* extern "C" */
-
-template <int MODE>
-static int launch_env(KParams &P, void *stream) {
-    if (check_dims(&P.d)) return -1;
-    wrsn_make_layout(&P.d, &P.L);
-    if (!P.scen || !P.scen_id || !P.state) WRSN_FAIL("scen / scen_id / state must not be NULL");
-    /* the opt-in dynamic shared-memory limit is a per-DEVICE attribute of the function: cache it per template instance, group
-       build and device (a second GPU in the same process needs its own opt-in) */
-    static int64_t attr_cache[2][WRSN_MAX_DEVICES];
-    static bool attr_init = false;
-    if (!attr_init) { for (int w_ = 0; w_ < 2; w_++) for (int q = 0; q < WRSN_MAX_DEVICES; q++) attr_cache[w_][q] = 48 * 1024; attr_init = true; }
-    int dev = 0;
-    WRSN_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= WRSN_MAX_DEVICES) WRSN_FAIL("device ordinal %d not supported", dev);
-    static int64_t pad = -1;                         /* TUNING KNOB (WRSN_SMEM_PAD bytes): fewer resident environments per SM */
-    if (pad < 0) { const char *e = getenv("WRSN_SMEM_PAD"); pad = e ? atoll(e) : 0; if (pad < 0 || pad > 200 * 1024) pad = 0; }
-    const int w = P.d.threads == 32 ? 0 : 1;
-    const int64_t smem = P.L.smem_total + pad;
-    if (smem > attr_cache[w][dev]) {
-        if (w == 0) WRSN_CUDA(cudaFuncSetAttribute(g32::k_env<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        else WRSN_CUDA(cudaFuncSetAttribute(gany::k_env<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_cache[w][dev] = smem;
-    }
-    if (w == 0) g32::k_env<MODE><<<P.d.B, 32, (size_t)smem, (cudaStream_t)stream>>>(P);
-    else gany::k_env<MODE><<<P.d.B, P.d.threads, (size_t)smem, (cudaStream_t)stream>>>(P);
-    WRSN_CUDA(cudaGetLastError());
-    return 0;
-}
-
-/* WRSN.step: one launch of the whole engine, or — wrsn_dims.step_rounds > 0 with a step budget — rounds of two launches, the
- * events kernel and the batch kernel (see include/wrsn_b200.h).  In the later launches a row is selected by its own state
- * (request record -4 + hdr[INFLIGHT]); rows that finished their step stay out. */
 /* Launch order of the step kernel: the hardware hands CTAs to the SMs in index order, and a launch whose last CTAs are long
  * environments ends on a tail of idle SMs (measured: 11 of 16 resident warps active on average).  One CTA sorts the rows by the
  * work their step is expected to take — the time to the earliest next decision among the alive chargers, read from the process
@@ -950,74 +787,6 @@ __global__ void __launch_bounds__(ORD_THREADS) k_step_order(const KParams P, int
         if (bins[q] >= 0) order[atomicAdd(&s_off[bins[q]], 1)] = threadIdx.x + q * ORD_THREADS;
 }
 
-static int launch_step_sync(KParams &P, void *stream);
-static int launch_step(KParams &P, void *stream) {
-    if (P.d.step_rounds < 0 && P.d.threads == 32) return launch_step_sync(P, stream);
-    /* Measured (4096 environments, RandomController law): one launch of 4096 rows 1.03 -> 1.13 M decisions/s with the order; four
-       groups of 1024 rows on four streams 1.20 -> 1.23 M (the other groups' kernels already fill the tail, and the ordering kernel
-       costs 23 us per launch).  So: rows are ordered when one launch holds at least 2048 of them.  TUNING KNOB WRSN_STEP_ORDER:
-       0 never, 1 always (B > 32). */
-    static int use_order = -1;
-    if (use_order < 0) { const char *e = getenv("WRSN_STEP_ORDER"); use_order = e ? atoi(e) : 2; }
-    if (use_order && P.req.order && P.d.B > (use_order == 2 ? 2047 : 32) && P.d.B <= ORD_THREADS * ORD_MAX_ROWS && P.scen && P.scen_id && P.state) {
-        if (check_dims(&P.d)) return -1;
-        wrsn_make_layout(&P.d, &P.L);
-        k_step_order<<<1, ORD_THREADS, 0, (cudaStream_t)stream>>>(P, P.req.order);
-        WRSN_CUDA(cudaGetLastError());
-        P.order = P.req.order;
-    }
-    if (!(P.d.step_budget > 0 && P.d.step_rounds > 0)) return launch_env<MODE_STEP>(P, stream);
-    if (!P.req.agent_id) WRSN_FAIL("split steps need req->agent_id");
-    for (int r = 0; r < P.d.step_rounds; r++) {
-        if (launch_env<MODE_STEP>(P, stream)) return -1;
-        KParams Q = P;
-        Q.agent_in = nullptr; Q.action_in = nullptr;
-        if (launch_env<MODE_STEP_BATCH>(Q, stream)) return -1;
-        P.resume_only = 1;                           /* later rounds: only rows still in flight (the others hold a fresh request) */
-    }
-    return 0;
-}
-
-/* wrsn_dims.step_rounds < 0: the persistent, phase-synchronous step kernel (wrsn_env_kernel.cuh: k_env_sync), one CTA of sixteen
- * warps per SM, environments handed out through req->queue. */
-static int launch_step_sync(KParams &P, void *stream) {
-    if (check_dims(&P.d)) return -1;
-    wrsn_make_layout(&P.d, &P.L);
-    if (!P.scen || !P.scen_id || !P.state) WRSN_FAIL("scen / scen_id / state must not be NULL");
-    if (!P.req.queue) WRSN_FAIL("step_rounds < 0 needs req->queue (two zeroed int32 on the device)");
-    int dev = 0;
-    WRSN_CUDA(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= WRSN_MAX_DEVICES) WRSN_FAIL("device ordinal %d not supported", dev);
-    static int sms[WRSN_MAX_DEVICES];
-    static int64_t attr_cache[WRSN_MAX_DEVICES];
-    static int th = -1, quantum = -1;
-    if (th < 0) {                                    /* TUNING KNOBS (measured flat: 0.80 - 0.87 M decisions/s over th 4..16, quantum 16..64) */
-        const char *e = getenv("WRSN_SYNC_TH"); th = e ? atoi(e) : 8; if (th < 1 || th > 16) th = 8;
-        e = getenv("WRSN_SYNC_Q"); quantum = e ? atoi(e) : 32; if (quantum < 1) quantum = 32;
-    }
-    if (!sms[dev]) WRSN_CUDA(cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev));
-    P.sync_slice = (int)wrsn_a16(P.L.smem_total); P.sync_th = th; P.sync_quantum = quantum;
-    const int64_t smem = (int64_t)P.sync_slice * WRSN_SYNC_WARPS;
-    if (smem > 227 * 1024 - 256) WRSN_FAIL("step_rounds < 0: %d environments of %lld bytes do not fit one SM's shared memory", WRSN_SYNC_WARPS, (long long)P.L.smem_total);
-    if (smem > attr_cache[dev]) {
-        WRSN_CUDA(cudaFuncSetAttribute(g32::k_env_sync, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_cache[dev] = smem;
-    }
-    int grid = (P.d.B + WRSN_SYNC_WARPS - 1) / WRSN_SYNC_WARPS;
-    if (grid > sms[dev]) grid = sms[dev];
-    g32::k_env_sync<<<grid, 32 * WRSN_SYNC_WARPS, (size_t)smem, (cudaStream_t)stream>>>(P);
-    WRSN_CUDA(cudaGetLastError());
-    return 0;
-}
-
-static KParams base_params(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, const uint8_t *mask) {
-    KParams P;
-    memset(&P, 0, sizeof(P));
-    if (d) P.d = *d;
-    P.scen = (const char *)scen; P.scen_id = scen_id; P.state = (char *)state; P.mask = mask;
-    return P;
-}
-
 /* the charging model, dense: one warp per environment (see include/wrsn_b200.h: wrsn_k_charge) */
 #define CHG_WARPS 4
 __global__ void __launch_bounds__(32 * CHG_WARPS) k_charge(const KParams P, const uint8_t *__restrict__ charging,
@@ -1077,32 +846,72 @@ __global__ void __launch_bounds__(32 * CHG_WARPS) k_charge(const KParams P, cons
 }
 
 /* roll_out bookkeeping (IPPO.py:138-155): one thread per environment, see include/wrsn_b200.h */
-__global__ void k_record_transitions(int B, int M, wrsn_request req, long long t, const long long *__restrict__ agent_prev,
-                                     long long *__restrict__ last, double *__restrict__ resets_seen,
-                                     long long *__restrict__ agent_next, long long *__restrict__ link_next,
+__global__ void k_record_transitions(int B, int M, wrsn_request req, int64_t t, const int64_t *__restrict__ agent_prev,
+                                     int64_t *__restrict__ last, double *__restrict__ resets_seen,
+                                     int64_t *__restrict__ agent_next, int64_t *__restrict__ link_next,
                                      uint8_t *__restrict__ new_episode_next, double *__restrict__ reward_next,
                                      double *__restrict__ now_next) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
-    long long *row = last + (size_t)b * M;
-    const long long ap = agent_prev[b];
-    if (ap >= 0 && ap < M) row[ap] = t;
-    const double resets = req.stats[(size_t)b * 3 + 2];
-    const bool ended = resets != resets_seen[b];
-    resets_seen[b] = resets;
-    if (ended)
-        for (int a = 0; a < M; a++) row[a] = -1;
-    int an = req.agent_id[b];                        /* < 0: no request for this row (-4: its step is still in flight) */
-    if (an >= M) an = M - 1;
-    agent_next[b] = an < 0 ? -1 : an;
-    link_next[b] = an < 0 ? -1 : row[an];
-    new_episode_next[b] = ended ? 1 : 0;
-    const double r = req.reward[b];
-    reward_next[b] = (r == r) ? r : 0.0;
-    now_next[b] = req.now[b];
+    record_transition(b, M, req, t, agent_prev, last, resets_seen, agent_next, link_next, new_episode_next, reward_next, now_next);
+}
+
+#include "wrsn_abi_host.h"
+
+template <int MODE>
+static int launch_env(KParams &P, void *stream) {
+    if (prepare_launch(P)) return -1;
+    /* the opt-in dynamic shared-memory limit is a per-DEVICE attribute of the function: cache it per template instance, group
+       build and device (a second GPU in the same process needs its own opt-in) */
+    static int64_t attr_cache[2][WRSN_MAX_DEVICES];
+    static bool attr_init = false;
+    if (!attr_init) { for (int w_ = 0; w_ < 2; w_++) for (int q = 0; q < WRSN_MAX_DEVICES; q++) attr_cache[w_][q] = 48 * 1024; attr_init = true; }
+    int dev = 0;
+    WRSN_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= WRSN_MAX_DEVICES) WRSN_FAIL("device ordinal %d not supported", dev);
+    static int64_t pad = -1;                         /* TUNING KNOB (WRSN_SMEM_PAD bytes): fewer resident environments per SM */
+    if (pad < 0) { const char *e = getenv("WRSN_SMEM_PAD"); pad = e ? atoll(e) : 0; if (pad < 0 || pad > 200 * 1024) pad = 0; }
+    const int w = P.d.threads == 32 ? 0 : 1;
+    const int64_t smem = P.L.smem_total + pad;
+    if (smem > attr_cache[w][dev]) {
+        if (w == 0) WRSN_CUDA(cudaFuncSetAttribute(g32::k_env<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        else WRSN_CUDA(cudaFuncSetAttribute(gany::k_env<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        attr_cache[w][dev] = smem;
+    }
+    if (w == 0) g32::k_env<MODE><<<P.d.B, 32, (size_t)smem, (cudaStream_t)stream>>>(P);
+    else gany::k_env<MODE><<<P.d.B, P.d.threads, (size_t)smem, (cudaStream_t)stream>>>(P);
+    WRSN_CUDA(cudaGetLastError());
+    return 0;
+}
+
+/* Measured (4096 environments, RandomController law): one launch of 4096 rows 1.03 -> 1.13 M decisions/s with the order; four
+   groups of 1024 rows on four streams 1.20 -> 1.23 M (the other groups' kernels already fill the tail, and the ordering kernel
+   costs 23 us per launch).  So: rows are ordered when one launch holds at least 2048 of them.  TUNING KNOB WRSN_STEP_ORDER:
+   0 never, 1 always (B > 32). */
+static int order_rows(KParams &P, void *stream) {
+    static int use_order = -1;
+    if (use_order < 0) { const char *e = getenv("WRSN_STEP_ORDER"); use_order = e ? atoi(e) : 2; }
+    if (use_order && P.req.order && P.d.B > (use_order == 2 ? 2047 : 32) && P.d.B <= ORD_THREADS * ORD_MAX_ROWS && P.scen && P.scen_id && P.state) {
+        if (check_dims(&P.d)) return -1;
+        wrsn_make_layout(&P.d, &P.L);
+        k_step_order<<<1, ORD_THREADS, 0, (cudaStream_t)stream>>>(P, P.req.order);
+        WRSN_CUDA(cudaGetLastError());
+        P.order = P.req.order;
+    }
+    return 0;
 }
 
 extern "C" {
+
+int wrsn_device_ok(void) {
+    int n = 0;
+    if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) { cudaGetLastError(); snprintf(g_err, sizeof(g_err), "no CUDA device"); return 0; }
+    int dev = 0; cudaGetDevice(&dev);
+    cudaDeviceProp p;
+    if (cudaGetDeviceProperties(&p, dev) != cudaSuccess) return 0;
+    if (p.major != 10) { snprintf(g_err, sizeof(g_err), "device is sm_%d%d, this library is built for sm_100a only", p.major, p.minor); return 0; }
+    return 1;
+}
 
 int wrsn_build_obs_tables(const wrsn_dims *d, void *scen, void *stream) {
     if (check_dims(d)) return -1;
@@ -1111,81 +920,6 @@ int wrsn_build_obs_tables(const wrsn_dims *d, void *scen, void *stream) {
     k_obs_tables<<<dim3(d->n_scen, d->Npad), 128, 0, (cudaStream_t)stream>>>(*d, L, (char *)scen);
     WRSN_CUDA(cudaGetLastError());
     return 0;
-}
-
-int wrsn_init_network(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state,
-                      const uint8_t *env_mask, int with_reward_process, void *stream) {
-    KParams P = base_params(d, scen, scen_id, state, env_mask);
-    P.with_reward = with_reward_process;
-    return launch_env<MODE_INIT>(P, stream);
-}
-
-int wrsn_run_until(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state,
-                   const uint8_t *env_mask, const double *t_until, void *stream) {
-    if (!t_until) WRSN_FAIL("t_until is NULL");
-    KParams P = base_params(d, scen, scen_id, state, env_mask);
-    P.t_until = t_until;
-    return launch_env<MODE_RUN_UNTIL>(P, stream);
-}
-
-int wrsn_reset_finish(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state,
-                      const uint8_t *env_mask, wrsn_request *req, void *stream) {
-    if (!req) WRSN_FAIL("req is NULL");
-    KParams P = base_params(d, scen, scen_id, state, env_mask);
-    P.req = *req;
-    return launch_env<MODE_RESET_FINISH>(P, stream);
-}
-
-int wrsn_reset_from_snapshot(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state,
-                             const void *snap, const uint8_t *env_mask, wrsn_request *req, void *stream) {
-    if (!req || !snap) WRSN_FAIL("req / snap is NULL");
-    KParams P = base_params(d, scen, scen_id, state, env_mask);
-    P.req = *req; P.snap = (const char *)snap;
-    return launch_env<MODE_RESTORE_RESET>(P, stream);
-}
-
-int wrsn_step(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state,
-              const uint8_t *env_mask, const int32_t *agent_id_in, const double *action_in,
-              wrsn_request *req, void *stream) {
-    if (!req) WRSN_FAIL("req is NULL");
-    if (agent_id_in && !action_in) WRSN_FAIL("action_in is NULL");
-    KParams P = base_params(d, scen, scen_id, state, env_mask);
-    P.agent_in = agent_id_in; P.action_in = action_in; P.req = *req;
-    return launch_step(P, stream);
-}
-
-int wrsn_rollout_step(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, const void *snap,
-                      const double *action_in, wrsn_request *req, void *obs, int obs_f64, void *stream) {
-    if (!req || !req->agent_id || !snap || !action_in) WRSN_FAIL("req / req->agent_id / snap / action_in is NULL");
-    KParams P = base_params(d, scen, scen_id, state, nullptr);
-    P.req = *req; P.agent_in = req->agent_id; P.action_in = action_in; P.mask_mode = 1;
-    if (launch_step(P, stream)) return -1;
-    KParams R = base_params(d, scen, scen_id, state, nullptr);
-    R.req = *req; R.snap = (const char *)snap; R.mask_mode = 2;
-    if (launch_env<MODE_RESTORE_RESET>(R, stream)) return -1;
-    if (obs) return wrsn_observe(d, scen, scen_id, state, req->agent_id, obs, obs_f64, stream);
-    return 0;
-}
-
-int wrsn_record_transitions(const wrsn_dims *d, const wrsn_request *req, int64_t t, const int64_t *agent_prev,
-                            int64_t *last, double *resets_seen, int64_t *agent_next, int64_t *link_next,
-                            uint8_t *new_episode_next, double *reward_next, double *now_next, void *stream) {
-    if (!d || !req || !req->agent_id || !req->reward || !req->now || !req->stats) WRSN_FAIL("req / its agent_id, reward, now or stats is NULL");
-    if (!agent_prev || !last || !resets_seen || !agent_next || !link_next || !new_episode_next || !reward_next || !now_next)
-        WRSN_FAIL("a record pointer is NULL");
-    if (d->B <= 0 || d->M <= 0) WRSN_FAIL("bad dims");
-    k_record_transitions<<<(d->B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        d->B, d->M, *req, (long long)t, (const long long *)agent_prev, (long long *)last, resets_seen,
-        (long long *)agent_next, (long long *)link_next, new_episode_next, reward_next, now_next);
-    WRSN_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int wrsn_fitness(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state,
-                 double *fitness, double *fit_min, void *stream) {
-    KParams P = base_params(d, scen, scen_id, state, nullptr);
-    P.fitness = fitness; P.fit_min = fit_min;
-    return launch_env<MODE_FITNESS>(P, stream);
 }
 
 int wrsn_observe(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
@@ -1281,23 +1015,6 @@ int wrsn_k_charge(const wrsn_dims *d, const void *scen, const int32_t *scen_id, 
     k_charge<<<(d->B + CHG_WARPS - 1) / CHG_WARPS, 32 * CHG_WARPS, 0, (cudaStream_t)stream>>>(P, charging, node_rate, mc_rate);
     WRSN_CUDA(cudaGetLastError());
     return 0;
-}
-
-int wrsn_k_bfs(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream) {
-    KParams P = base_params(d, scen, scen_id, state, nullptr);
-    return launch_env<MODE_K_BFS>(P, stream);
-}
-int wrsn_k_drain(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream) {
-    KParams P = base_params(d, scen, scen_id, state, nullptr);
-    return launch_env<MODE_K_DRAIN>(P, stream);
-}
-int wrsn_k_bookkeep(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream) {
-    KParams P = base_params(d, scen, scen_id, state, nullptr);
-    return launch_env<MODE_K_BOOK>(P, stream);
-}
-int wrsn_k_reward(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream) {
-    KParams P = base_params(d, scen, scen_id, state, nullptr);
-    return launch_env<MODE_K_REWARD>(P, stream);
 }
 
 }  /* extern "C" */

@@ -89,5 +89,45 @@ WRSN_HD void wrsn_make_layout(const wrsn_dims *d, WrsnLayout *L) {
 }
 
 
+/* ------------------------------------------------------------------ observation tables
+ * Output tile of a thread of the observation rasters (wrsn_kernels.cu: k_observe, k_observe_win): OBS_TI rows x OBS_TJ64 columns
+ * in the fp64 raster, x OBS_TJ32 in the fp32 one.  The node tables of the scenario record are padded to whole tiles. */
+#define OBS_TI 4
+#define OBS_TJ64 10
+#ifndef OBS_TJ32
+#define OBS_TJ32 20
+#endif
+
+WRSN_HD int32_t wrsn_obs_pitch(int S) {
+    const int ti = (S + OBS_TI - 1) / OBS_TI;
+    const int tj = (S + OBS_TJ64 - 1) / OBS_TJ64, tk = (S + OBS_TJ32 - 1) / OBS_TJ32;
+    const int pk = (tk * OBS_TJ32 + 3) & ~3;
+    int pi = ti * OBS_TI, pj = (tj * OBS_TJ64 + 3) & ~3;
+    if (pk > pj) pj = pk;
+    return pi > pj ? pi : pj;
+}
+
 /* request record of one environment, as the engine's entry points produce it */
 struct ReqOut { int agent; int terminal; double reward, now, act[3], detail[2]; int flags; };
+
+/* roll_out bookkeeping of row b (see include/wrsn_b200.h: wrsn_record_transitions) */
+WRSN_HD void record_transition(int b, int M, const wrsn_request &req, int64_t t, const int64_t *agent_prev, int64_t *last,
+                               double *resets_seen, int64_t *agent_next, int64_t *link_next, uint8_t *new_episode_next,
+                               double *reward_next, double *now_next) {
+    int64_t *row = last + (size_t)b * M;
+    const int64_t ap = agent_prev[b];
+    if (ap >= 0 && ap < M) row[ap] = t;
+    const double resets = req.stats[(size_t)b * 3 + 2];
+    const bool ended = resets != resets_seen[b];
+    resets_seen[b] = resets;
+    if (ended)
+        for (int a = 0; a < M; a++) row[a] = -1;
+    int an = req.agent_id[b];                        /* < 0: no request for this row (-4: its step is still in flight) */
+    if (an >= M) an = M - 1;
+    agent_next[b] = an < 0 ? -1 : an;
+    link_next[b] = an < 0 ? -1 : row[an];
+    new_episode_next[b] = ended ? 1 : 0;
+    const double r = req.reward[b];
+    reward_next[b] = (r == r) ? r : 0.0;
+    now_next[b] = req.now[b];
+}

@@ -1,7 +1,8 @@
 /*
  * wrsn_emu.cpp — TEST INFRASTRUCTURE.  Single-lane host build of the kernel source
- * (multi_agent_rl_wrsn_b200/csrc/wrsn_engine.cuh with WRSN_HOST_EMU): the same event logic the
- * sm_100a kernels run, with one "thread" per environment, on host memory.  It exists so the
+ * (multi_agent_rl_wrsn_b200/csrc/wrsn_engine.cuh with WRSN_HOST_EMU): the same event logic, the same per-environment
+ * driver (wrsn_env_kernel.cuh: env_run) and the same host side of the ABI (wrsn_abi_host.h) as the sm_100a library,
+ * with one "thread" per environment, on host memory.  It exists so the
  * `-m "not gpu"` tests can check the engine's event ordering and arithmetic against the oracle on a box
  * without a GPU.  It is built only by tests/ (tests/emu/Makefile), exports the C ABI of
  * include/wrsn_b200.h, and is never loaded by the product package, which has no CPU path.
@@ -13,171 +14,31 @@
 #include <stdlib.h>
 #include <vector>
 
-#include "wrsn_layout.h"
+#include "wrsn_launch.h"
 static thread_local char *wrsn_smem_host = nullptr;
 #define WRSN_GFIX 1
 #include "wrsn_engine.cuh"
 
-static thread_local char g_err[512] = "";
-#define WRSN_FAIL(...) do { snprintf(g_err, sizeof(g_err), __VA_ARGS__); return -1; } while (0)
+#include "wrsn_env_kernel.cuh"
+#include "wrsn_abi_host.h"
 
-enum { MODE_INIT = 0, MODE_RUN_UNTIL, MODE_RESET_FINISH, MODE_RESTORE_RESET, MODE_STEP, MODE_FITNESS, MODE_K_BFS,
-       MODE_K_DRAIN, MODE_K_BOOK, MODE_K_REWARD, MODE_STEP_BATCH };
-
-struct Args {
-    const wrsn_dims *d; const char *scen; const int32_t *scen_id; char *state; const char *snap; const uint8_t *mask;
-    const double *t_until; const int32_t *agent_in; const double *action_in; wrsn_request *req;
-    double *fitness, *fit_min; int with_reward; int mask_mode; int resume_only;
-};
-
-static int run_mode(int mode, const Args &A) {
-    const wrsn_dims &d = *A.d;
-    if (d.Npad < d.N || (d.Npad & 15) || d.state_bytes <= 0) WRSN_FAIL("dims not finalized");
-    WrsnLayout L; wrsn_make_layout(&d, &L);
-    std::vector<char> smem((size_t)L.smem_total + 64);
-    for (int b = 0; b < d.B; b++) {
-        if (A.mask && !A.mask[b]) continue;
-        if (A.mask_mode == 1 && A.req->agent_id[b] < 0 && A.req->agent_id[b] != -4) continue;
-        if (A.mask_mode == 2 && (A.req->agent_id[b] >= 0 || A.req->agent_id[b] == -4)) continue;
-        if (A.resume_only && A.req->agent_id[b] != -4) continue;
-        char *row = A.state + (size_t)b * L.total;
-        const bool split = d.step_budget > 0 && d.step_rounds > 0;
-        const double infl = reinterpret_cast<const double *>(row + L.off[WRSN_F_HDR])[WRSN_H_INFLIGHT];
-        if (mode == MODE_STEP && split && A.req && A.req->agent_id && A.req->agent_id[b] == -4 && infl == 2.0) continue;
-        if (mode == MODE_STEP_BATCH && (A.req->agent_id[b] != -4 || infl != 2.0)) continue;
-        const char *scen_row = A.scen + (size_t)A.scen_id[b] * L.scen_total;
-        Ctx c;
-        wrsn_smem_host = smem.data();
-        ctx_bind(c, d, L, scen_row, row, 0, 1);
-        if (mode == MODE_RESTORE_RESET) {
-            const char *src = A.snap + (size_t)A.scen_id[b] * L.total;
-            memcpy(row + L.resident, src + L.resident, (size_t)(L.total - L.resident));
-            memcpy(smem.data(), src, (size_t)L.resident);
-        } else if (mode != MODE_INIT) memcpy(smem.data(), row, (size_t)L.resident);
-        else memset(smem.data(), 0, (size_t)L.resident);
-        for (int i = 0; i < c.Npad; i++) c.own[i] = i < c.N ? (uint16_t)(c.tgt_ptr[i + 1] - c.tgt_ptr[i]) : 0;
-        const double now_before = c.hdr[WRSN_H_NOW];
-        ReqOut r; memset(&r, 0, sizeof(r)); r.agent = -3;
-        switch (mode) {
-        case MODE_INIT: entry_init_network(c, A.with_reward); break;
-        case MODE_RUN_UNTIL: entry_run_until(c, A.t_until[b]); break;
-        case MODE_RESET_FINISH: case MODE_RESTORE_RESET: entry_reset_finish(c, &r); break;
-        case MODE_STEP: entry_step(c, A.agent_in ? A.agent_in[b] : -1, A.action_in ? A.action_in + 3 * (size_t)b : nullptr, &r, d.step_budget, split ? 1 : 0); break;
-        case MODE_STEP_BATCH: entry_batches(c, &r, d.step_budget); break;
-        case MODE_FITNESS: { double mn = do_fitness(c, A.fitness ? A.fitness + (size_t)b * d.T : nullptr); if (A.fit_min) A.fit_min[b] = mn; break; }
-        case MODE_K_BFS: do_bfs(c); break;
-        case MODE_K_DRAIN: ev_nodes_drain(c); break;
-        case MODE_K_BOOK: ev_nodes_book(c); break;
-        case MODE_K_REWARD: ev_update_reward(c); break;
-        }
-        if (mode != MODE_FITNESS) memcpy(row, smem.data(), (size_t)L.resident);
-        if (mode == MODE_RESET_FINISH || mode == MODE_RESTORE_RESET || mode == MODE_STEP || mode == MODE_STEP_BATCH) {
-            wrsn_request &q = *A.req;
-            if (q.agent_id) q.agent_id[b] = r.agent;
-            if (q.terminal) q.terminal[b] = (uint8_t)r.terminal;
-            if (q.reward) q.reward[b] = r.reward;
-            if (q.now) q.now[b] = r.now;
-            if (q.action) for (int k = 0; k < 3; k++) q.action[3 * b + k] = r.act[k];
-            if (q.detail) { q.detail[2 * b] = r.detail[0]; q.detail[2 * b + 1] = r.detail[1]; }
-            if (q.flags) q.flags[b] = r.flags;
-            if (q.sticky && r.flags) q.sticky[b] |= r.flags;
-            if (q.stats) { if (r.agent >= 0) q.stats[3 * b] += 1.0; if (mode == MODE_STEP || mode == MODE_STEP_BATCH) q.stats[3 * b + 1] += r.now - now_before;
-                           if (mode == MODE_RESTORE_RESET || mode == MODE_RESET_FINISH) q.stats[3 * b + 2] += 1.0; }
-        }
-    }
+/* one "launch": every row of the batch in turn, on one lane, in the image the engine addresses as its shared memory */
+template <int MODE>
+static int launch_env(KParams &P, void *) {
+    if (prepare_launch(P)) return -1;
+    std::vector<char> smem((size_t)P.L.smem_total + 64);
+    wrsn_smem_host = smem.data();
+    for (int b = 0; b < P.d.B; b++) env_run<MODE>(P, b, 0, 1);
     return 0;
 }
 
-static int run_step(Args A) {                       /* launch_step of wrsn_kernels.cu */
-    const wrsn_dims &d = *A.d;
-    if (!(d.step_budget > 0 && d.step_rounds > 0)) return run_mode(MODE_STEP, A);
-    for (int r = 0; r < d.step_rounds; r++) {
-        if (run_mode(MODE_STEP, A)) return -1;
-        Args Q = A; Q.agent_in = nullptr; Q.action_in = nullptr;
-        if (run_mode(MODE_STEP_BATCH, Q)) return -1;
-        A.resume_only = 1;
-    }
-    return 0;
-}
+static int order_rows(KParams &, void *) { return 0; }   /* rows run one after the other: the order changes nothing */
 
 extern "C" {
-const char *wrsn_last_error(void) { return g_err; }
-int wrsn_abi_version(void) { return WRSN_ABI_VERSION; }
 int wrsn_is_emulation(void) { return 1; }
-int wrsn_field_count(int which) {
-    switch (which) {
-    case 0: return WRSN_P_LEN; case 1: return WRSN_H_LEN; case 2: return WRSN_MC_LEN; case 3: return WRSN_PR_LEN;
-    case 4: return WRSN_F_COUNT; case 5: return WRSN_S_COUNT; default: return -1;
-    }
-}
-int wrsn_dims_finalize(wrsn_dims *d) {
-    d->Npad = (d->N + 15) & ~15; d->W = (d->N + 31) / 32; d->Tw = (d->T + 31) / 32; if (d->Tw < 1) d->Tw = 1;
-    d->n_slot = d->M + 3; if (d->Emax < 1) d->Emax = 1; if (d->TEmax < 1) d->TEmax = 1;
-    d->threads = 32;
-    { const int ti = (d->S + 3) / 4, tj = (d->S + 9) / 10, tk = (d->S + 19) / 20; const int pi = ti * 4, pk = (tk * 20 + 3) & ~3; int pj = (tj * 10 + 3) & ~3; if (pk > pj) pj = pk; d->obs_pitch = pi > pj ? pi : pj; }
-    WrsnLayout L; wrsn_make_layout(d, &L);
-    d->state_bytes = (int32_t)L.total; d->state_resident_bytes = (int32_t)L.resident;
-    d->scen_bytes = (int32_t)L.scen_total; d->smem_bytes = (int32_t)L.smem_total;
-    return 0;
-}
-int wrsn_state_layout(const wrsn_dims *d, int64_t *o) { WrsnLayout L; wrsn_make_layout(d, &L); for (int k = 0; k < WRSN_F_COUNT; k++) o[k] = L.off[k]; return 0; }
-int wrsn_scen_layout(const wrsn_dims *d, int64_t *o) { WrsnLayout L; wrsn_make_layout(d, &L); for (int k = 0; k < WRSN_S_COUNT; k++) o[k] = L.soff[k]; return 0; }
 int wrsn_device_ok(void) { return 0; }
 int wrsn_build_obs_tables(const wrsn_dims *, void *, void *) { return 0; }   /* only the CUDA raster reads them */
 
-int wrsn_init_network(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, const uint8_t *m, int wr, void *) {
-    Args A = {d, (const char *)scen, scen_id, (char *)state, nullptr, m, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, wr};
-    return run_mode(MODE_INIT, A);
-}
-int wrsn_run_until(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, const uint8_t *m, const double *t, void *) {
-    Args A = {d, (const char *)scen, scen_id, (char *)state, nullptr, m, t, nullptr, nullptr, nullptr, nullptr, nullptr, 0};
-    return run_mode(MODE_RUN_UNTIL, A);
-}
-int wrsn_reset_finish(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, const uint8_t *m, wrsn_request *req, void *) {
-    Args A = {d, (const char *)scen, scen_id, (char *)state, nullptr, m, nullptr, nullptr, nullptr, req, nullptr, nullptr, 0};
-    return run_mode(MODE_RESET_FINISH, A);
-}
-int wrsn_reset_from_snapshot(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, const void *snap, const uint8_t *m, wrsn_request *req, void *) {
-    Args A = {d, (const char *)scen, scen_id, (char *)state, (const char *)snap, m, nullptr, nullptr, nullptr, req, nullptr, nullptr, 0};
-    return run_mode(MODE_RESTORE_RESET, A);
-}
-int wrsn_step(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, const uint8_t *m, const int32_t *ag, const double *act, wrsn_request *req, void *) {
-    Args A = {d, (const char *)scen, scen_id, (char *)state, nullptr, m, nullptr, ag, act, req, nullptr, nullptr, 0};
-    return run_step(A);
-}
-int wrsn_rollout_step(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, const void *snap,
-                      const double *act, wrsn_request *req, void *obs, int obs_f64, void *) {
-    Args A = {d, (const char *)scen, scen_id, (char *)state, nullptr, nullptr, nullptr, req->agent_id, act, req, nullptr, nullptr, 0, 1};
-    if (run_step(A)) return -1;
-    Args R = {d, (const char *)scen, scen_id, (char *)state, (const char *)snap, nullptr, nullptr, nullptr, nullptr, req, nullptr, nullptr, 0, 2};
-    if (run_mode(MODE_RESTORE_RESET, R)) return -1;
-    return obs ? wrsn_observe(d, scen, scen_id, state, req->agent_id, obs, obs_f64, nullptr) : 0;
-}
-int wrsn_record_transitions(const wrsn_dims *d, const wrsn_request *req, int64_t t, const int64_t *agent_prev, int64_t *last,
-                            double *resets_seen, int64_t *agent_next, int64_t *link_next, uint8_t *new_episode_next,
-                            double *reward_next, double *now_next, void *) {
-    if (!d || !req || !agent_prev || !last || !resets_seen || !agent_next || !link_next || !new_episode_next || !reward_next || !now_next)
-        WRSN_FAIL("a record pointer is NULL");
-    const int M = d->M;
-    for (int b = 0; b < d->B; b++) {                    /* host restatement of k_record_transitions, row by row */
-        int64_t *row = last + (size_t)b * M;
-        if (agent_prev[b] >= 0 && agent_prev[b] < M) row[agent_prev[b]] = t;
-        const double resets = req->stats[(size_t)b * 3 + 2];
-        const bool ended = resets != resets_seen[b];
-        resets_seen[b] = resets;
-        if (ended) for (int a = 0; a < M; a++) row[a] = -1;
-        int an = req->agent_id[b];
-        if (an >= M) an = M - 1;
-        agent_next[b] = an < 0 ? -1 : an; link_next[b] = an < 0 ? -1 : row[an]; new_episode_next[b] = ended ? 1 : 0;
-        reward_next[b] = req->reward[b] == req->reward[b] ? req->reward[b] : 0.0;
-        now_next[b] = req->now[b];
-    }
-    return 0;
-}
-int wrsn_fitness(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, double *fit, double *fmin_, void *) {
-    Args A = {d, (const char *)scen, scen_id, (char *)state, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, fit, fmin_, 0};
-    return run_mode(MODE_FITNESS, A);
-}
 /* WRSN.get_state (rl_env/WRSN.py:130-186), host restatement of the fp64 parity raster k_observe<double> (same source order,
  * same rounding: (w * gx) * gy added term by term; channel 4 as ((gx * gy) * w) / moving_time_max).  float output = the fp64
  * map rounded once (the GPU's fp32 raster accumulates in fp32: equal to ~1e-6 of the channel maximum, not bit for bit). */
@@ -287,10 +148,4 @@ int wrsn_k_charge(const wrsn_dims *d, const void *scen, const int32_t *scen_id, 
     }
     return 0;
 }
-#define EMU_K(NAME, MODE) int NAME(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *) { \
-    Args A = {d, (const char *)scen, scen_id, (char *)state, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0}; return run_mode(MODE, A); }
-EMU_K(wrsn_k_bfs, MODE_K_BFS)
-EMU_K(wrsn_k_drain, MODE_K_DRAIN)
-EMU_K(wrsn_k_bookkeep, MODE_K_BOOK)
-EMU_K(wrsn_k_reward, MODE_K_REWARD)
-}
+}  /* extern "C" */

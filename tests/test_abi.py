@@ -59,6 +59,33 @@ def test_layout_and_enums(cuda_so):
     assert b"bad dims" in L.wrsn_last_error()
 
 
+def test_emulation_dims_and_layouts_equal_the_cuda_library(cuda_so):
+    """Both libraries compile the same host side of the ABI: the same dims, thread counts and layouts, the same rejections."""
+    libs = [_lib._bind(cuda_so), _lib._bind(ctypes.CDLL(os.path.join(REPO, "tests", "emu", "libwrsn_emu.so")))]
+    e = _lib.enums()
+
+    def finalize(L, N, T, M, S, rounds=0):
+        d = _lib.Dims()
+        d.B, d.N, d.T, d.M, d.S, d.Emax, d.TEmax, d.n_scen = 8, N, T, M, S, 6 * N, 2 * T, 2
+        rc = L.wrsn_dims_finalize(ctypes.byref(d))
+        d.step_budget, d.step_rounds = 60, rounds
+        off = (ctypes.c_int64 * e["WRSN_F_COUNT"])()
+        soff = (ctypes.c_int64 * e["WRSN_S_COUNT"])()
+        rcs = (rc, L.wrsn_state_layout(ctypes.byref(d), off), L.wrsn_scen_layout(ctypes.byref(d), soff))
+        return rcs, {f: getattr(d, f) for f, _ in d._fields_}, list(off), list(soff)
+
+    for N in (50, 100, 150, 500, 1000):
+        for T, M, S in ((N, 3, 100), (2 * N, 10, 64), (7, 1, 37)):
+            got = [finalize(L, N, T, M, S) for L in libs]
+            assert got[0] == got[1], (N, T, M, S)
+            assert got[0][0] == (0, 0, 0)
+    assert [finalize(L, 150, 150, 3, 100)[1]["threads"] for L in libs] == [64, 64]
+    for kw, msg in ((dict(M=e["WRSN_MAX_MC"] + 1), b"bad dims"), (dict(M=3, rounds=-1), b"step_rounds")):
+        for L in libs:
+            rcs = finalize(L, N=100, T=100, S=100, **kw)[0]
+            assert rcs[1] != 0 and rcs[2] != 0 and msg in L.wrsn_last_error()
+
+
 def test_no_cpu_path():
     """Without a GPU the product host layer must refuse loudly, not fall back."""
     import torch

@@ -202,25 +202,6 @@ def test_step_budget_only_cuts_steps_into_launches(threads, budget, rounds):
     pc.check_budget_equals_unbudgeted(scs, DEV, num_envs=8, calls=60, seed=6, budget=budget, scale2=0.3, threads=threads, rounds=rounds)
 
 
-@pytest.mark.parametrize("budget", [0, 40, 100])
-def test_phase_synchronous_step_kernel(budget):
-    """wrsn_dims.step_rounds < 0 (k_env_sync: one persistent launch, sixteen environments per CTA, event phase / batch phase): same
-    requests and same records as one CTA per environment, with and without a step budget; more environments than one wave of
-    warps, so that the queue hands out several environments per warp."""
-    scs = [synthetic(num_nodes=100, num_targets=100, seed=s) for s in BENCH_SCENARIOS]
-    n = pc.check_budget_equals_unbudgeted(scs, DEV, num_envs=80, calls=60, seed=7, budget=budget, scale2=0.1, threads=32, rounds=-1)
-    assert n > 10 or budget == 0
-    scs = [synthetic(num_nodes=40, num_targets=120, seed=s, num_gateways=2) for s in (3, 4)]
-    pc.check_budget_equals_unbudgeted(scs, DEV, num_envs=8, calls=60, seed=6, budget=budget, scale2=0.3, threads=32, rounds=-1)
-
-
-def test_phase_synchronous_step_kernel_vs_oracle():
-    """The headline workload (RandomController maps decoded on the device) through k_env_sync against the C restatement."""
-    scs = [synthetic(num_nodes=100, num_targets=100, seed=s) for s in BENCH_SCENARIOS]
-    n_dec, cnt = pc.check_vs_oracle(scs, DEV, num_envs=64, steps=40, seed=13, controller=True, obs32=True, rounds=-1)
-    assert n_dec > 64 * 25
-
-
 def test_sharded_equals_unsharded_records():
     """Two / three simulators holding contiguous blocks of the environments == one simulator holding all of them, byte for
     byte (SURVEY 8e: environments shard by index, nothing is exchanged) — also with a step budget."""
@@ -228,7 +209,6 @@ def test_sharded_equals_unsharded_records():
     pc.check_sharded_equals_unsharded(scs, DEV, num_envs=50, steps=60, seed=2, world=2)
     pc.check_sharded_equals_unsharded(scs, DEV, num_envs=50, steps=60, seed=3, world=3, budget=40)
     pc.check_sharded_equals_unsharded(scs, DEV, num_envs=50, steps=60, seed=4, world=2, budget=60, rounds=2)
-    pc.check_sharded_equals_unsharded(scs, DEV, num_envs=50, steps=60, seed=5, world=2, budget=60, rounds=-1)
 
 
 @pytest.mark.parametrize("name,t_from,t_to", [("net_hanoi1000n200", 512, 524), ("net_hanoi1000n100", 1598, 1608)])

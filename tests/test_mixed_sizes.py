@@ -131,8 +131,7 @@ def _check_golden_mixed(names, device):
 def test_golden_episodes_mixed(dev, rows):
     """All five fixtures (largest 132 nodes: 64 threads per environment), and the first four (largest 98: one warp)."""
     env = _check_golden_mixed(GOLDEN_MIXED[:rows], dev)
-    if dev != "cpu":
-        assert env.dims.threads == (64 if rows == 5 else 32)
+    assert env.dims.threads == (64 if rows == 5 else 32)
 
 
 # ------------------------------------------------------------------ 2. mixed batch == one batch per scenario, byte for byte
@@ -221,14 +220,6 @@ def test_mixed_equals_homogeneous(dev, kind, threads, budget, rounds):
 
 
 @pytest.mark.gpu
-def test_mixed_equals_homogeneous_persistent_kernel(dev):
-    """step_rounds < 0: the persistent one-warp kernel (k_env_sync) keeps one image per warp."""
-    if dev == "cpu":
-        pytest.skip("the persistent kernel runs on the GPU only")
-    _check_mixed_equals_homogeneous(dev, _scenarios("small"), B=96, steps=40, threads=32, budget=60, rounds=-1)
-
-
-@pytest.mark.gpu
 @pytest.mark.parametrize("kind,threads", [("small", 32), ("large", 64)])
 def test_mixed_equals_homogeneous_reordered_launch(dev, kind, threads):
     """2304 rows in one launch: k_step_order reorders the mixed batch's CTAs (longest step first), not the smaller ones'."""
@@ -309,19 +300,16 @@ def test_mixed_shards_equal_whole(dev):
 
 
 # ------------------------------------------------------------------ 5. API
-def _expected_dims(N, T, gpu):
-    threads = 32                                     # (the emulation runs one lane whatever the batch)
-    if gpu:
-        per = (N + 3) // 4
-        while threads < per and threads < 128:
-            threads *= 2
-        if N > 9 * threads:
-            threads = 256
+def _expected_dims(N, T):
+    threads, per = 32, (N + 3) // 4
+    while threads < per and threads < 128:
+        threads *= 2
+    if N > 9 * threads:
+        threads = 256
     return dict(Npad=(N + 15) // 16 * 16, W=(N + 31) // 32, Tw=max((T + 31) // 32, 1), threads=threads)
 
 
 def test_dims_and_counts(dev):
-    gpu = dev != "cpu"
     # a homogeneous batch: the dims of its one size, as before mixed sizes existed
     for n, t in ((100, 100), (60, 70), (150, 170)):
         scs = [synthetic(num_nodes=n, num_targets=t, seed=s, num_gateways=4) for s in (1, 2)]
@@ -329,7 +317,7 @@ def test_dims_and_counts(dev):
         d = _lib.Dims()
         d.B, d.N, d.T, d.M, d.S, d.Emax, d.TEmax, d.n_scen = 4, n, t, 3, 100, env.dims.Emax, env.dims.TEmax, 2
         assert env.L.wrsn_dims_finalize(ctypes.byref(d)) == 0
-        want = _expected_dims(n, t, gpu)
+        want = _expected_dims(n, t)
         got = {k: getattr(env.dims, k) for k in want}
         assert got == want and env.dims.state_bytes == d.state_bytes and env.dims.smem_bytes == d.smem_bytes, (n, t)
         assert (env.N, env.T) == (n, t) and _np(env.num_nodes).tolist() == [n] * 4 and _np(env.num_targets).tolist() == [t] * 4
@@ -338,7 +326,7 @@ def test_dims_and_counts(dev):
     assert _np(env.num_nodes).tolist() == [82, 82, 82, 98, 132] and _np(env.num_targets).tolist() == [50, 50, 50, 100, 200]
     assert env.num_nodes.dtype == torch.int32 and env.num_nodes.device == env.device and env.num_targets.dtype == torch.int32
     assert (env.N, env.T) == (132, 200)
-    assert {k: getattr(env.dims, k) for k in ("Npad", "W", "Tw", "threads")} == _expected_dims(132, 200, gpu)
+    assert {k: getattr(env.dims, k) for k in ("Npad", "W", "Tw", "threads")} == _expected_dims(132, 200)
     env.reset()
     assert tuple(env.view("energy").shape) == (5, 132) and tuple(env.targets_active().shape) == (5, 200)
     assert tuple(env.get_network_fitness()[0].shape) == (5, 200) and tuple(env.charge_rates()[0].shape) == (5, 132)

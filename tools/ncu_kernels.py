@@ -1,8 +1,8 @@
 """Launch every kernel of the library a few times on realistic states, for `ncu --set full` (one capture per kernel, see
 profiles/r02_kernels.md): python tools/ncu_kernels.py [B].  Kernels: k_env<STEP> (rollout), k_env<RESTORE_RESET>, k_decode_map,
 k_decode_locate, k_observe (chunked, synthetic fields) / k_observe_win (hanoi1000n100: narrow sources), k_observe<double>,
-k_charge, k_record_transitions, the per-tick kernels k_env<K_BFS / K_DRAIN / K_BOOK / K_REWARD>, k_env<FITNESS>, k_step_order,
-k_env_sync (step_rounds < 0) and gany::k_env<STEP> on 1000-node environments (256 threads)."""
+k_charge, k_record_transitions, the per-tick kernels k_env<K_BFS / K_DRAIN / K_BOOK / K_REWARD>, k_env<FITNESS>, k_step_order
+and gany::k_env<STEP> on 1000-node environments (256 threads)."""
 import os, sys
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -41,16 +41,6 @@ torch.cuda.profiler.start()
 hn.get_state(out=o2)                                      # k_observe_win
 torch.cuda.synchronize()
 torch.cuda.profiler.stop()
-# the phase-synchronous persistent step kernel (step_rounds < 0) on the same rolled-out states
-env.dims.step_rounds = -1
-for k in range(3):
-    env.rollout_step(env.linear_controller_action(obs, (1.0, 1.0, -10.0, 1.0)), obs)
-torch.cuda.synchronize()
-torch.cuda.profiler.start()
-env.rollout_step(env.linear_controller_action(obs, (1.0, 1.0, -10.0, 1.0)), obs)       # k_env_sync
-torch.cuda.synchronize()
-torch.cuda.profiler.stop()
-env.dims.step_rounds = 0
 # BASELINE.json configs[4]: 1000 nodes / 10 chargers, 256 threads per environment (gany::k_env)
 if os.environ.get("WRSN_NCU_C5", "1") == "1":
     big = [synthetic(num_nodes=1000, num_targets=1000, seed=1000 + k, num_gateways=25) for k in range(4)]
