@@ -241,7 +241,9 @@ int wrsn_observe(const wrsn_dims *d, const void *scen, const int32_t *scen_id, c
 /* WRSN.density_map_to_action (:229-287) with the map normalisation of WRSN.step (:293-296): dmap[b][S][S] (float, or
  * double when dmap_f64 != 0) -> action_out[b][3] = (x-frac, y-frac, charge-time frac) for every row with
  * agent_id[b] >= 0; other rows are left untouched.  The location search replaces scipy's L-BFGS-B (see the kernel's
- * comment for what is reproduced exactly and what within tolerance). */
+ * comment for what is reproduced exactly and what within tolerance).  Map sizes 1 to 176: the 99.9th percentile of a
+ * larger map needs more order statistics than the decoder keeps, and such a map_size fails with an error (here and in
+ * wrsn_decode_linear_controller).  A map that is -inf everywhere decodes to the box of cell 0, as np.argmax gives it. */
 int wrsn_decode_density_map(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
                             const int32_t *agent_id, const void *dmap, int dmap_f64, double *action_out, void *stream);
 /* The same decode for a controller whose density map is a LINEAR COMBINATION of the observation's channels — the reference's

@@ -29,6 +29,26 @@ static int check_dims(const wrsn_dims *d) {
     return 0;
 }
 
+/* The density-map decoder (k_decode_map) keeps the WRSN_DEC_MAX_RANK largest values of a map: np.percentile(., 99.9) needs the
+ * R-th largest, R = n - floor(0.999 n - 0.999) with n = S * S (the kernel's own expression), so maps up to 176 x 176 (R = 32).
+ * A larger map is refused here instead of being ranked wrongly. */
+#define WRSN_DEC_MAX_RANK 32
+static int wrsn_decode_rank(int S) {
+    const int n = S * S;
+    const double qf = 99.9 / 100.0;
+    const double vidx = (double)n * qf + (1.0 + qf * (1.0 - 1.0 - 1.0)) - 1.0;
+    return n - (int)floor(vidx);
+}
+static int check_decode_size(const wrsn_dims *d) {
+    if (d->S > 46340 || wrsn_decode_rank(d->S) > WRSN_DEC_MAX_RANK) {
+        int smax = 1;
+        while (wrsn_decode_rank(smax + 1) <= WRSN_DEC_MAX_RANK) smax++;
+        WRSN_FAIL("map_size = %d: the density-map decoder supports map sizes up to %d (np.percentile(., 99.9) of a larger map "
+                  "needs more than the %d largest values it keeps)", d->S, smax, WRSN_DEC_MAX_RANK);
+    }
+    return 0;
+}
+
 /* every launch of the environment kernel: valid dims, the layout they imply, the buffers every mode reads */
 static int prepare_launch(KParams &P) {
     if (check_dims(&P.d)) return -1;

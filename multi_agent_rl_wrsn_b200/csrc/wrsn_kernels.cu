@@ -518,8 +518,10 @@ __global__ void __launch_bounds__(DEC_THREADS, 4) k_decode_map(const KParams P, 
     for (int k = tid; k < n; k += DEC_THREADS) {
         const MapT v = at(k);
         mn = v < mn ? v : mn; mx = v > mx ? v : mx; sm += (double)v;
-        if (v > h1v) { h2v = h1v; h2i = h1i; h1v = v; h1i = k; }
-        else if (v > h2v) { h2v = v; h2i = k; }
+        /* an empty head also takes a -inf cell (k ascending: the first one, as np.argmax does for a map that is -inf
+           everywhere); NaN cells never become heads */
+        if (v > h1v || (h1i == 0x7fffffff && v == h1v)) { h2v = h1v; h2i = h1i; h1v = v; h1i = k; }
+        else if (v > h2v || (h2i == 0x7fffffff && v == h2v)) { h2v = v; h2i = k; }
     }
     double dmn = (double)mn, dmx = (double)mx;
     for (int o = 16; o > 0; o >>= 1) {
@@ -531,8 +533,8 @@ __global__ void __launch_bounds__(DEC_THREADS, 4) k_decode_map(const KParams P, 
     const double vidx = (double)n * qf + (1.0 + qf * (1.0 - 1.0 - 1.0)) - 1.0;
     const int lo_idx = (int)floor(vidx);
     const double tq = vidx - (double)lo_idx;
-    int R = n - lo_idx;                              /* the R-th largest value is sorted[lo_idx] */
-    if (R > DEC_MAXR - 2) R = DEC_MAXR - 2;          /* map sizes up to ~175 x 175 */
+    int R = n - lo_idx;                              /* the R-th largest value is sorted[lo_idx]; R <= DEC_MAXR - 2: the host
+                                                        refuses larger maps (wrsn_abi_host.h: check_decode_size) */
     const int rounds = R + 1 < n ? R + 1 : n;        /* one more: does anything tie with sorted[lo_idx] beyond the selection? */
     /* every warp selects ITS `rounds` largest (shuffles only): the block's `rounds` largest are among those */
     {
@@ -543,8 +545,8 @@ __global__ void __launch_bounds__(DEC_THREADS, 4) k_decode_map(const KParams P, 
                 for (int k = tid; k < n; k += DEC_THREADS) {
                     const MapT v = at(k);
                     if (!(v < lastv || (v == lastv && k > lasti))) continue;
-                    if (v > h1v) { h2v = h1v; h2i = h1i; h1v = v; h1i = k; }
-                    else if (v > h2v) { h2v = v; h2i = k; }
+                    if (v > h1v || (h1i == 0x7fffffff && v == h1v)) { h2v = h1v; h2i = h1i; h1v = v; h1i = k; }
+                    else if (v > h2v || (h2i == 0x7fffffff && v == h2v)) { h2v = v; h2i = k; }
                 }
                 taken = 0;
             }
@@ -857,6 +859,7 @@ __global__ void k_record_transitions(int B, int M, wrsn_request req, int64_t t, 
 }
 
 #include "wrsn_abi_host.h"
+static_assert(WRSN_DEC_MAX_RANK == DEC_MAXR - 2, "the host refuses the map sizes whose rank k_decode_map cannot hold");
 
 template <int MODE>
 static int launch_env(KParams &P, void *stream) {
@@ -977,7 +980,7 @@ int wrsn_decode_density_map(const wrsn_dims *d, const void *scen, const int32_t 
     if (!agent_id || !dmap || !action_out || !scen || !scen_id || !state) WRSN_FAIL("NULL argument");
     KParams P = base_params(d, scen, scen_id, const_cast<void *>(state), nullptr);
     wrsn_make_layout(&P.d, &P.L);
-    if ((int64_t)d->S * d->S > (1 << 30)) WRSN_FAIL("map_size too large for the density-map decoder");
+    if (check_decode_size(d)) return -1;
     LinMap lin; memset(&lin, 0, sizeof(lin));
     if (dmap_f64) k_decode_map<double, 0><<<d->B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, (const double *)dmap, action_out, lin);
     else k_decode_map<float, 0><<<d->B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, (const float *)dmap, action_out, lin);
@@ -994,7 +997,7 @@ int wrsn_decode_linear_controller(const wrsn_dims *d, const void *scen, const in
     if (channels < 1 || channels > 8) WRSN_FAIL("1 to 8 channels");
     KParams P = base_params(d, scen, scen_id, const_cast<void *>(state), nullptr);
     wrsn_make_layout(&P.d, &P.L);
-    if ((int64_t)d->S * d->S > (1 << 30)) WRSN_FAIL("map_size too large for the density-map decoder");
+    if (check_decode_size(d)) return -1;
     LinMap lin; memset(&lin, 0, sizeof(lin));
     lin.C = channels;
     for (int k = 0; k < channels; k++) lin.w[k] = weights[k];

@@ -7,7 +7,7 @@
  * without a GPU.  It is built only by tests/ (tests/emu/Makefile), exports the C ABI of
  * include/wrsn_b200.h, and is never loaded by the product package, which has no CPU path.
  * wrsn_observe is a plain host restatement of the fp64 parity raster (the raster kernels themselves are checked on the GPU);
- * wrsn_decode_density_map is not emulated.
+ * wrsn_decode_density_map is not emulated (it only checks its dims and map size, as the CUDA library does).
  */
 #define WRSN_HOST_EMU 1
 #include <stdio.h>
@@ -63,7 +63,7 @@ int wrsn_observe(const wrsn_dims *d, const void *scen, const int32_t *scen_id, c
                  void *obs, int obs_f64, void *) {
     if (!d || !scen || !scen_id || !state || !agent_id || !obs) WRSN_FAIL("NULL argument");
     WrsnLayout L; wrsn_make_layout(d, &L);
-    const int S = d->S, N = d->N, M = d->M;
+    const int S = d->S, M = d->M;
     const size_t SS = (size_t)S * S;
     for (int b = 0; b < d->B; b++) {
         const int ag = agent_id[b];
@@ -81,7 +81,8 @@ int wrsn_observe(const wrsn_dims *d, const void *scen, const int32_t *scen_id, c
         for (int ch = 0; ch < 4; ch++) {
             std::vector<double> out(SS, 0.0);
             if (ch == 0) {
-                for (int s = 0; s < N; s++) {
+                const int Nrow = (int)par[WRSN_P_NNODES];        /* this row's own nodes, as the kernels read them */
+                for (int s = 0; s < Nrow; s++) {
                     if (status[s] == 0) continue;
                     const double w = (cs[s] / par[WRSN_P_MC_AB2]) / ((energy[s] - par[WRSN_P_THR]) / par[WRSN_P_CAPMTHR]);
                     if (w == 0.0) continue;
@@ -112,11 +113,14 @@ int wrsn_observe(const wrsn_dims *d, const void *scen, const int32_t *scen_id, c
     }
     return 0;
 }
-int wrsn_decode_linear_controller(const wrsn_dims *, const void *, const int32_t *, const void *, const int32_t *, const float *, int, const float *,
+/* the decoder is not emulated; its entry points refuse what the CUDA library refuses first, with the same message */
+int wrsn_decode_linear_controller(const wrsn_dims *d, const void *, const int32_t *, const void *, const int32_t *, const float *, int, const float *,
                                   double *, void *) {
+    if (check_dims(d) || check_decode_size(d)) return -1;
     WRSN_FAIL("wrsn_decode_linear_controller is not available in the host emulation");
 }
-int wrsn_decode_density_map(const wrsn_dims *, const void *, const int32_t *, const void *, const int32_t *, const void *, int, double *, void *) {
+int wrsn_decode_density_map(const wrsn_dims *d, const void *, const int32_t *, const void *, const int32_t *, const void *, int, double *, void *) {
+    if (check_dims(d) || check_decode_size(d)) return -1;
     WRSN_FAIL("wrsn_decode_density_map is not available in the host emulation");
 }
 int wrsn_k_charge(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state, const uint8_t *charging,

@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from multi_agent_rl_wrsn_b200 import BatchedWRSN, _lib, synthetic
+from multi_agent_rl_wrsn_b200 import BatchedWRSN, Scenario, _lib, synthetic
 from oracle import decode_oracle as do
 from oracle.wrsn_oracle import OracleWRSN, scenario_from_dict
 from tests import helpers, parity_cases as pc
@@ -264,3 +264,231 @@ def test_random_controller_rollout_stays_on_the_host_decode_trajectory(cuda_libr
           % (n_dec, n_centre, n_close, n_far, float(np.median(far)) if far else 0.0, n_nan))
     assert n_dec >= B * steps // 3
     assert n_centre + n_close >= 0.9 * (n_dec - n_nan), (n_dec, n_centre, n_close, n_far, n_nan)
+
+
+# ------------------------------------------------------------------ map sizes, map kinds and the decoder's edge paths
+DEC_SIZES = [1, 2, 4, 7, 17, 32, 64, 100, 128, 175, 176]
+DEC_MAX_S = 176                                       # the largest map whose percentile rank the decoder holds
+
+
+def _rank(S):
+    """R of np.percentile(., 99.9) over S * S cells (the R-th largest value is the lower interpolation point), with the
+    kernel's own expression."""
+    n = S * S
+    return n - int(np.floor(n * 0.999 + (1.0 + 0.999 * (1.0 - 1.0 - 1.0)) - 1.0))
+
+
+def _fraction_at_rank(dm, r):
+    """The charge fraction of density_map_to_action with the percentile taken between the r-th and (r-1)-th largest
+    values instead of the R-th and (R-1)-th."""
+    flat = np.sort(dm.ravel())
+    n = flat.size
+    vidx = n * 0.999 + (1.0 + 0.999 * (1.0 - 1.0 - 1.0)) - 1.0
+    tq = vidx - np.floor(vidx)
+    lo = n - r
+    a, b = flat[lo], flat[min(lo + 1, n - 1)]
+    thr = a + (b - a) * tq if tq < 0.5 else b - (b - a) * (1.0 - tq)
+    return dm.max() / dm.ravel()[dm.ravel() >= thr].sum()
+
+
+def test_decoder_rank_limit():
+    assert _rank(100) == 11 and _rank(DEC_MAX_S) == 32 and _rank(DEC_MAX_S + 1) == 33 and _rank(200) == 41
+
+
+@pytest.fixture()
+def host_library():
+    import os
+    import subprocess
+    subprocess.check_call(["make", "-C", os.path.join(helpers.REPO, "tests", "emu"), "libwrsn_emu.so"], stdout=subprocess.DEVNULL)
+    helpers.use_host_build()
+    yield
+    helpers.use_cuda_build_lazy()
+
+
+def _refuses_large_maps(dev):
+    for S in (DEC_MAX_S + 1, 200):
+        env = BatchedWRSN(synthetic(num_nodes=40, num_targets=40, seed=2), num_agent=3, num_envs=2, map_size=S, device=dev)
+        env.reset()
+        aid = torch.zeros(2, dtype=torch.int32, device=env.state.device)
+        with pytest.raises(RuntimeError, match=r"map_size = %d: .* up to %d" % (S, DEC_MAX_S)):
+            env.density_map_to_action(torch.zeros((2, S, S), dtype=torch.float32, device=env.state.device), agent_id=aid)
+        with pytest.raises(RuntimeError, match=r"map_size = %d: .* up to %d" % (S, DEC_MAX_S)):
+            env.linear_controller_action(torch.zeros((2, 4, S, S), dtype=torch.float32, device=env.state.device), (1, 1, -10, 1), agent_id=aid)
+
+
+def test_decoder_refuses_large_maps_host_build(host_library):
+    """Both libraries share the check (wrsn_abi_host.h); the host build's decode entry points run it before they report that
+    the decoder is not emulated."""
+    _refuses_large_maps("cpu")
+    env = BatchedWRSN(synthetic(num_nodes=40, num_targets=40, seed=2), num_agent=3, num_envs=2, map_size=DEC_MAX_S, device="cpu")
+    with pytest.raises(RuntimeError, match="not available in the host emulation"):
+        env.density_map_to_action(torch.zeros((2, DEC_MAX_S, DEC_MAX_S)), agent_id=torch.zeros(2, dtype=torch.int32))
+
+
+@pytest.mark.gpu
+def test_decoder_refuses_large_maps(cuda_library):
+    _refuses_large_maps(DEV)
+
+
+MAP_KINDS = ("bump", "logits", "masked", "masked_few", "ties", "onehot", "uniform")
+
+
+def _make_map(kind, S, rng, cx, cy):
+    ii = (np.arange(S) + 0.5) / S
+    n = S * S
+    if kind == "bump":                                # a distribution, at least two cells wide: on a small map a narrower
+        w = max(0.03, 2.0 / S)                        # bump is one-hot in all but name, and no rank near the top shows
+        m = np.exp(-((ii[:, None] - cx) ** 2 + (ii[None, :] - cy) ** 2) / (2 * w ** 2))
+        return m / m.sum()
+    if kind == "logits":
+        return rng.normal(0, 2.0, (S, S))
+    if kind in ("masked", "masked_few"):              # -inf in most cells; "few": fewer finite cells than R + 1
+        m = np.full(n, -np.inf)
+        k = max(1, n // 20) if kind == "masked" else max(1, min(n, _rank(S)) // 2)
+        m[rng.choice(n, k, replace=False)] = rng.normal(0, 2.0, k)
+        return m.reshape(S, S)
+    if kind == "ties":                                # quantised: values tie at the percentile (second pass)
+        return np.round(rng.uniform(0, 3, (S, S))) / 2
+    if kind == "onehot":
+        m = np.zeros(n); m[rng.integers(0, n)] = 1.0
+        return m.reshape(S, S)
+    return np.full((S, S), 1.0 / n)                   # uniform
+
+
+def _locate_counts(env, got, ref, b, res, x0, counts):
+    par = env.statics[int(env.scen_id[b])]["par"]
+    loc = np.array([got[0] * (par["F1"] - par["F0"]) + par["F0"], got[1] * (par["F3"] - par["F2"]) + par["F2"]])
+    if np.array_equal(res.x, x0):                     # scipy stopped at the centre: pgtol
+        np.testing.assert_allclose(got[:2], ref[:2], rtol=1e-14, atol=1e-15)
+        counts["exact"] += 1
+    else:
+        counts["moved"] += 1
+        counts["close"] += int(np.hypot(*(loc - res.x)) <= 1e-3)
+    return loc
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
+def test_decode_map_sizes_and_kinds(cuda_library, dtype):
+    """Maps of seven kinds at every size from 1 x 1 to 176 x 176 against the restatement: charge fraction 1e-12 (float64 maps) /
+    1e-6 (float32); location identical where scipy stops at the box centre, otherwise within 1e-3 m in at least 90 % of the
+    decodes.  For every map without ties, the restatement's fraction at rank R - 1 and R + 1 differs from the one at R by more
+    than the tolerance: a rank slip cannot pass."""
+    rng = np.random.default_rng(17)
+    tol = 1e-12 if dtype == torch.float64 else 1e-6
+    counts = dict(exact=0, moved=0, close=0)
+    rank_checked = 0
+    for S in DEC_SIZES:
+        B = 2 * len(MAP_KINDS)
+        env = BatchedWRSN(synthetic(num_nodes=100, num_targets=100, seed=1000 + S), num_agent=3, num_envs=B, map_size=S, device=DEV)
+        env.reset()
+        maps = []
+        for b in range(B):
+            st = env.statics[0]; par = st["par"]
+            n = rng.integers(0, env.N)
+            cx = (st["x"][n] - par["F0"]) / (par["F1"] - par["F0"]); cy = (st["y"][n] - par["F2"]) / (par["F3"] - par["F2"])
+            maps.append(_make_map(MAP_KINDS[b % len(MAP_KINDS)], S, rng, cx, cy))
+        dm = torch.as_tensor(np.stack(maps), device=DEV).to(dtype).contiguous()
+        aid = torch.zeros(B, dtype=torch.int32, device=DEV)
+        got = env.density_map_to_action(dm, agent_id=aid).cpu().numpy()
+        host = dm.cpu().numpy().astype(np.float64)
+        for b in range(B):
+            kind = MAP_KINDS[b % len(MAP_KINDS)]
+            with np.errstate(all="ignore"):
+                ref, res, x0, objective = _oracle_decode(env, None, b, host[b])
+            np.testing.assert_allclose(got[b, 2], ref[2], rtol=tol, err_msg=str((S, kind)))
+            _locate_counts(env, got[b], ref, b, res, x0, counts)
+            norm = do.normalise_map(host[b])
+            R = _rank(S)
+            top = np.sort(norm.ravel())[::-1][:R + 2]
+            if kind in ("bump", "logits") and 2 <= R < S * S and np.unique(top).size == top.size:   # no ties near the percentile
+                np.testing.assert_allclose(_fraction_at_rank(norm, R), ref[2], rtol=1e-12)
+                for r in (R - 1, R + 1):          # (ranks 1 and 2 keep the same single value: below 1000 cells the
+                    if 2 <= r <= S * S:           #  interpolation weight puts the percentile above the second largest)
+                        assert abs(_fraction_at_rank(norm, r) - ref[2]) > tol * abs(ref[2]), (S, kind, r)
+                        rank_checked += 1
+    print("map sizes 1..176 (%s): %d decodes at scipy's box centre exactly, %d of %d others within 1e-3 m; %d rank slips detectable"
+          % (dtype, counts["exact"], counts["close"], counts["moved"], rank_checked))
+    assert counts["exact"] >= 20 and rank_checked >= 30
+    assert counts["close"] >= 0.9 * counts["moved"], counts
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
+def test_decode_all_minus_inf_map(cuda_library, dtype):
+    """A map that is -inf everywhere (a fully masked log-density): numpy's argmax gives cell 0, so the box is cell 0's; the
+    charge fraction is NaN (0 / 0 after the normalisation) on both paths."""
+    for S in (7, 100):
+        B = 4
+        env = BatchedWRSN(synthetic(num_nodes=100, num_targets=100, seed=1100 + S), num_agent=3, num_envs=B, map_size=S, device=DEV)
+        env.reset()
+        dm = torch.full((B, S, S), -float("inf"), dtype=dtype, device=DEV)
+        got = env.density_map_to_action(dm, agent_id=torch.zeros(B, dtype=torch.int32, device=DEV)).cpu().numpy()
+        counts = dict(exact=0, moved=0, close=0)
+        for b in range(B):
+            with np.errstate(all="ignore"):
+                ref, res, x0, objective = _oracle_decode(env, None, b, dm[b].cpu().numpy().astype(np.float64))
+            assert np.isnan(ref[2]) and np.isnan(got[b, 2])
+            assert abs(got[b, 0]) <= 1.0 and abs(got[b, 1]) <= 1.0, (S, got[b])       # near cell 0, not far off the field
+            _locate_counts(env, got[b], ref, b, res, x0, counts)
+        assert counts["close"] == counts["moved"], counts
+
+
+@pytest.mark.gpu
+def test_linear_controller_rolled_path(cuda_library):
+    """wrsn_decode_linear_controller with 1, 2, 3, 5 and 8 channels (the rolled path) and 4 (unrolled) == the decoder on the map
+    torch forms left to right, bit for bit."""
+    B, S = 64, 100
+    env, scs = _rolled_env(B, 20, seed=9)
+    g = torch.Generator(device=DEV); g.manual_seed(4)
+    agents = torch.zeros(B, dtype=torch.int32, device=DEV)
+    weights = (0.5, -2.0, 3.0, 0.25, 1.5, -0.75, 2.0, -1.25)
+    same = lambda x, y: bool(((x == y) | (torch.isnan(x) & torch.isnan(y))).all())
+    for C in (1, 2, 3, 4, 5, 8):
+        obs = torch.randn((B, C, S, S), dtype=torch.float32, device=DEV, generator=g).contiguous()
+        w = weights[:C]
+        dm = w[0] * obs[:, 0]
+        for c in range(1, C):
+            dm = dm + w[c] * obs[:, c]
+        want = env.density_map_to_action(dm.contiguous(), agent_id=agents)
+        got = env.linear_controller_action(obs, w, agent_id=agents)
+        assert same(want, got), C
+
+
+@pytest.mark.gpu
+def test_decode_locate_dense_field(cuda_library):
+    """200 nodes in a 150 m square: about 120 alive nodes within reach of the box, more than the 64 the locate kernel lists in
+    shared memory, so it reads the nodes from HBM.  Against scipy with the criteria above; every returned point lies in the
+    box, with an objective at least the centre's."""
+    rng = np.random.default_rng(3)
+    nodes = rng.uniform(0, 150, (200, 2))
+    sc = Scenario(nodes=nodes, targets=rng.uniform(0, 150, (50, 2)), base_station=np.array([75.0, 75.0]))
+    B = 32
+    env = BatchedWRSN(sc, num_agent=3, num_envs=B, device=DEV)
+    env.reset()
+    S = env.S
+    st = env.statics[0]; par = st["par"]
+    R = par["MC_R"]
+    maps = []
+    ii = (np.arange(S) + 0.5) / S
+    for b in range(B):
+        cx, cy = rng.uniform(0.3, 0.7, 2)
+        m = np.exp(-((ii[:, None] - cx) ** 2 + (ii[None, :] - cy) ** 2) / (2 * 0.03 ** 2))
+        maps.append(m / m.sum())
+    dm = torch.as_tensor(np.stack(maps), device=DEV)
+    got = env.density_map_to_action(dm, agent_id=torch.zeros(B, dtype=torch.int32, device=DEV)).cpu().numpy()
+    xy = np.stack([st["x"], st["y"]], 1)
+    alive = env.view("status").cpu().numpy()
+    counts = dict(exact=0, moved=0, close=0)
+    reach = []
+    for b in range(B):
+        ref, res, x0, objective = _oracle_decode(env, None, b, maps[b])
+        np.testing.assert_allclose(got[b, 2], ref[2], rtol=1e-12)
+        reach.append(int(((np.hypot(*(xy - x0).T) <= R * 2.4143) & (alive[b] != 0)).sum()))
+        loc = _locate_counts(env, got[b], ref, b, res, x0, counts)
+        assert np.all(np.abs(loc - x0) <= R * (1 + 1e-12)), (b, loc, x0)
+        assert -objective(loc) >= -objective(x0) * (1 - 1e-12), b
+    print("dense field: %d to %d alive nodes within reach; %d decodes at scipy's box centre exactly, %d of %d others within 1e-3 m"
+          % (min(reach), max(reach), counts["exact"], counts["close"], counts["moved"]))
+    assert min(reach) > 64
+    assert counts["close"] >= 0.9 * counts["moved"], counts
