@@ -4,7 +4,8 @@
  * launches the environment kernel.  Included once, after the kernels; the including file supplies
  *   launch_env<MODE>(P, stream)   one launch of env_run<MODE> (wrsn_env_kernel.cuh) over the rows of the batch;
  *   order_rows(P, stream)         before a step: the order in which the launch takes the rows (P.order; NULL = index order);
- * and the CUDA build the kernel k_record_transitions.
+ * and the CUDA build the kernel k_record_transitions.  The entry points of the raster, the decoder and the charging model:
+ * wrsn_abi_aux.h.
  */
 #pragma once
 #include <stdio.h>

@@ -50,25 +50,16 @@ namespace gany {                                     /* 64 ... 256 threads per e
 }
 
 /* ------------------------------------------------------------------ WRSN.get_state (rl_env/WRSN.py:130-186)
- * 4 x S x S map per environment.  Every source (alive node, charger) contributes w * G(x - x0; hX) * G(y - y0; hY)
- * with G(u; h) = exp(u^2 / (-2 h^2)) — separable, so the raster is a rank-(number of sources) outer-product sum.
- * A chunk of sources is expanded into two S-vectors each in shared memory (2 S exponentials per source instead of
- * S^2, always evaluated in fp64) and every thread accumulates a 4 x 10 register tile of output cells over the sources
+ * The sources and their weights: wrsn_layout.h (obs_source).  The raster is separable, so it is a rank-(number of sources)
+ * outer-product sum.  A chunk of sources is expanded into two S-vectors each in shared memory (2 S exponentials per source
+ * instead of S^2, always evaluated in fp64) and every thread accumulates a 4 x 10 register tile of output cells over the sources
  * IN SOURCE ORDER.  AccT = double: multiply and add rounded separately, exactly the reference's `map += w*gx*gy`
  * (parity path, float64 out).  AccT = float: the vectors are rounded to fp32 once and accumulated with FFMA (the
  * observation the policy networks consume is float32; error ~1e-6 of the channel maximum). */
 #define OBS_THREADS64 256           /* fp64 parity raster: 4 x 10 tiles (OBS_TI x OBS_TJ64, wrsn_layout.h) */
-#ifndef OBS_THREADS32
 #define OBS_THREADS32 128           /* fp32 raster: 4 x 20 tiles (OBS_TI x OBS_TJ32) */
-#endif
-#ifndef OBS_CH32
 #define OBS_CH32 32                 /* sources staged per pass (fp32 raster) */
-#endif
-#ifndef OBS_MINB32
 #define OBS_MINB32 4                /* CTAs per SM the fp32 raster is compiled for */
-#endif
-
-struct ObsSrc { double x0, y0, hx, hy, w; int mode; int node; };     /* mode 0: (w*gx)*gy ; 1: ((gx*gy)*w)/mtm ; node >= 0: table row */
 
 /* the node terms of get_state are static: one table row per node, float (the fp32 raster reads them, the fp64 parity
  * raster evaluates its exponentials itself) */
@@ -78,15 +69,13 @@ __global__ void k_obs_tables(const wrsn_dims d, const WrsnLayout L, char *scen) 
     const double *nx = (const double *)(row + L.soff[WRSN_S_NX]), *ny = (const double *)(row + L.soff[WRSN_S_NY]);
     float *gx = (float *)(row + L.soff[WRSN_S_OBS_GX]), *gy = (float *)(row + L.soff[WRSN_S_OBS_GY]);
     const int n = blockIdx.y, S = d.S, TP = d.obs_pitch;
-    const double f0 = par[WRSN_P_F0], f1 = par[WRSN_P_F1], f2 = par[WRSN_P_F2], f3 = par[WRSN_P_F3];
-    const double Wd = f1 - f0, Hd = f3 - f2, R = par[WRSN_P_MC_R];
-    const double unit = 1.0 / (double)S, start = unit / 2.0, delta = (start + unit) - start;
-    const double x0 = (nx[n] - f0) / Wd, y0 = (ny[n] - f2) / Hd, hx = R / Wd, hy = R / Hd;
+    const ObsGrid g(par, S);
+    const double x0 = g.cx(nx[n]), y0 = g.cy(ny[n]), hx = g.R / g.Wd, hy = g.R / g.Hd;
+    const double dnx = -2.0 * (hx * hx), dny = -2.0 * (hy * hy);
     for (int i = threadIdx.x; i < TP; i += blockDim.x) {
-        const double cc = start + (double)i * delta, ux = cc - x0, uy = cc - y0;
         const bool in = i < S && n < (int)par[WRSN_P_NNODES];
-        gx[(size_t)n * TP + i] = in ? (float)exp(ux * ux / (-2.0 * (hx * hx))) : 0.f;
-        gy[(size_t)n * TP + i] = in ? (float)exp(uy * uy / (-2.0 * (hy * hy))) : 0.f;
+        gx[(size_t)n * TP + i] = in ? (float)obs_gauss(g.cell(i), x0, dnx) : 0.f;
+        gy[(size_t)n * TP + i] = in ? (float)obs_gauss(g.cell(i), y0, dny) : 0.f;
     }
 }
 
@@ -104,22 +93,9 @@ __global__ void __launch_bounds__(THREADS, sizeof(AccT) == 4 ? OBS_MINB32 : 1) k
     const int b = blockIdx.x, tid = threadIdx.x;
     const int ag = agent_id[b];
     if (ag < 0) return;
-    const char *row = P.state + (size_t)b * P.L.total;
-    const char *scen_row = P.scen + (size_t)P.scen_id[b] * P.L.scen_total;
-    const double *par = (const double *)(scen_row + P.L.soff[WRSN_S_PAR]);
-    const int N = (int)par[WRSN_P_NNODES];                                    /* this scenario's nodes (P.d.N: the batch's largest) */
-    const double *nx = (const double *)(scen_row + P.L.soff[WRSN_S_NX]);
-    const double *ny = (const double *)(scen_row + P.L.soff[WRSN_S_NY]);
-    const double *energy = (const double *)(row + P.L.off[WRSN_F_ENERGY]);
-    const double *cs = (const double *)(row + P.L.off[WRSN_F_CS]);
-    const uint8_t *status = (const uint8_t *)(row + P.L.off[WRSN_F_STATUS]);
-    const double *mc = (const double *)(row + P.L.off[WRSN_F_MC]);
-    const float *tab_gx = (const float *)(scen_row + P.L.soff[WRSN_S_OBS_GX]), *tab_gy = (const float *)(scen_row + P.L.soff[WRSN_S_OBS_GY]);
-    const double f0 = par[WRSN_P_F0], f1 = par[WRSN_P_F1], f2 = par[WRSN_P_F2], f3 = par[WRSN_P_F3];
-    const double Wd = f1 - f0, Hd = f3 - f2;
-    const double unit = 1.0 / (double)S, start = unit / 2.0, delta = (start + unit) - start;   /* np.arange(unit/2, 1.0, unit) */
-    const double R = par[WRSN_P_MC_R], mtm = par[WRSN_P_MTM];
-    const double *me = mc + (size_t)ag * WRSN_MC_LEN;
+    const WrsnRow rw(P.L, P.state, P.scen, P.scen_id, b);
+    const ObsGrid g(rw.par, S);
+    const int N = rw.N;
     const int SS = S * S;
     AccT *out = obs + (size_t)b * 4 * SS;
     const int n_tiles = tiles_i * tiles_j;
@@ -139,39 +115,9 @@ __global__ void __launch_bounds__(THREADS, sizeof(AccT) == 4 ? OBS_MINB32 : 1) k
             for (int s0 = 0; s0 < total; s0 += CH) {
                 const int nq = total - s0 < CH ? total - s0 : CH;
                 __syncthreads();
-                /* the sources of this pass, one thread each, in id order; unused ones (dead node, wrong charger) get
-                   mode -1 and are skipped — the reference skips them too, and the sum order of the rest is unchanged */
-                for (int q = tid; q < nq; q += THREADS) {
-                    const int s = s0 + q;
-                    ObsSrc v; v.mode = -1; v.node = -1; v.x0 = v.y0 = v.w = 0.0; v.hx = v.hy = 1.0;
-                    if (ch == 0) {
-                        if (status[s] != 0) {
-                            v.mode = 0; v.node = s;
-                            v.x0 = (nx[s] - f0) / Wd; v.y0 = (ny[s] - f2) / Hd; v.hx = R / Wd; v.hy = R / Hd;
-                            v.w = (cs[s] / par[WRSN_P_MC_AB2]) / ((energy[s] - par[WRSN_P_THR]) / par[WRSN_P_CAPMTHR]);
-                            if (v.w == 0.0) v.mode = -1;     /* a node without traffic (energyCS == 0) adds exact zeros: skip it */
-                        }
-                    } else if (ch == 1) {
-                        double tmp = fmin(Hd, Wd);
-                        v.mode = 0;
-                        v.x0 = (me[WRSN_MC_X] - f0) / Wd; v.y0 = (me[WRSN_MC_Y] - f2) / Hd;
-                        v.hx = 0.5 * tmp / Wd; v.hy = 0.5 * tmp / Hd;
-                        v.w = me[WRSN_MC_ENERGY] / par[WRSN_P_MC_CAP];
-                    } else {
-                        const double *an = mc + (size_t)s * WRSN_MC_LEN;
-                        const bool charging = an[WRSN_MC_TYPE] != 0.0;
-                        if (s != ag && (ch == 2 ? charging : !charging)) {
-                            v.x0 = (an[WRSN_MC_CPA0] - f0) / Wd; v.y0 = (an[WRSN_MC_CPA1] - f2) / Hd; v.hx = R / Wd; v.hy = R / Hd;
-                            if (ch == 2) { v.mode = 0; v.w = an[WRSN_MC_CPA2] / par[WRSN_P_CTM]; }
-                            else {                   /* SURVEY Q5: the observer's destination y */
-                                double dx = an[WRSN_MC_X] - an[WRSN_MC_CPA0], dy = an[WRSN_MC_Y] - me[WRSN_MC_CPA1];
-                                v.w = sqrt(dx * dx + dy * dy) / par[WRSN_P_MC_V];
-                                v.mode = 1;
-                            }
-                        }
-                    }
-                    src[q] = v;
-                }
+                /* the sources of this pass, one thread each, in id order; unused ones are skipped — the reference skips them
+                   too, and the sum order of the rest is unchanged */
+                for (int q = tid; q < nq; q += THREADS) src[q] = obs_source(rw, g, ag, ch, s0 + q);
                 __syncthreads();
                 /* expand every source into its two S-vectors.  Node sources of the fp32 raster are a scaled copy of the
                    scenario's table (contiguous, independent loads); everything else is one fp64 exponential per entry. */
@@ -181,7 +127,7 @@ __global__ void __launch_bounds__(THREADS, sizeof(AccT) == 4 ? OBS_MINB32 : 1) k
                     const int node = src[q].node;
                     if (sizeof(AccT) == 4 && node >= 0) {
                         const float wq = (float)src[q].w;
-                        const float *rx = tab_gx + (size_t)node * TP, *ry = tab_gy + (size_t)node * TP;
+                        const float *rx = rw.tab_gx + (size_t)node * TP, *ry = rw.tab_gy + (size_t)node * TP;
                         /* TP is a multiple of 4 and every row starts 16-byte aligned: four entries per lane and instruction */
                         const float4 *rx4 = reinterpret_cast<const float4 *>(rx), *ry4 = reinterpret_cast<const float4 *>(ry);
                         float4 *gx4 = reinterpret_cast<float4 *>(gx + q * TP), *gy4 = reinterpret_cast<float4 *>(gy + q * TP);
@@ -195,13 +141,10 @@ __global__ void __launch_bounds__(THREADS, sizeof(AccT) == 4 ? OBS_MINB32 : 1) k
                         const double dnx = -2.0 * (src[q].hx * src[q].hx), dny = -2.0 * (src[q].hy * src[q].hy);
                         /* fp32 raster: the constant factor of the source (w, or w / moving_time_max for the travel-time
                            channel) is folded into the x-vector, so every channel shares the FFMA loop below */
-                        const double fold = mode == 0 ? src[q].w : (sizeof(AccT) == 4 ? src[q].w / mtm : 1.0);
+                        const double fold = mode == 0 ? src[q].w : (sizeof(AccT) == 4 ? src[q].w / g.mtm : 1.0);
                         for (int i = tid & 31; i < TP; i += 32) {
-                            const double cc = start + (double)i * delta;
-                            const double ux = cc - x0, uy = cc - y0;
-                            const double ax = ux * ux / dnx, ay = uy * uy / dny;
-                            const double ex = (i < S && ax > -745.2) ? exp(ax) : 0.0;   /* below: exp underflows to 0 anyway */
-                            const double ey = (i < S && ay > -745.2) ? exp(ay) : 0.0;
+                            const double ex = i < S ? obs_gauss(g.cell(i), x0, dnx) : 0.0;
+                            const double ey = i < S ? obs_gauss(g.cell(i), y0, dny) : 0.0;
                             gx[q * TP + i] = (AccT)((mode == 0 || sizeof(AccT) == 4) ? fold * ex : ex);
                             gy[q * TP + i] = (AccT)ey;
                         }
@@ -245,7 +188,7 @@ __global__ void __launch_bounds__(THREADS, sizeof(AccT) == 4 ? OBS_MINB32 : 1) k
                 } else {
                     for (int q = 0; q < nq; q++) {
                         if (src[q].mode < 0) continue;
-                        const AccT w = (AccT)src[q].w, d = (AccT)mtm;
+                        const AccT w = (AccT)src[q].w, d = (AccT)g.mtm;
 #pragma unroll
                         for (int r = 0; r < OBS_TI; r++)
 #pragma unroll
@@ -297,98 +240,56 @@ __global__ void __launch_bounds__(THREADS, sizeof(AccT) == 4 ? OBS_MINB32 : 1) k
  * tile, in source order.  Shared memory per source: OBW row entries and OBW column entries between two 16-entry zero
  * margins (a partly covered tile reads zeros instead of branching): 448 bytes at OBW = 40. */
 #define OBM 16                       /* zero margin on either side of the column window (a tile is 20 columns wide) */
+#define OBW 40                       /* window in cells (multiple of 4): >= 12.2 sigma + 6 */
 #define OBW_THREADS 128
 struct WinSrc { int sx, sy; };       /* first row / column of the window; sx < -1000: source unused */
-template <int OBW>                   /* window in cells (multiple of 4): >= 12.2 sigma + 6, chosen by the launcher */
-__global__ void __launch_bounds__(OBW_THREADS, OBW <= 40 ? 4 : (OBW <= 56 ? 3 : 2)) k_observe_win(const KParams P, const int32_t *agent_id, float *obs) {
+__global__ void __launch_bounds__(OBW_THREADS, 4) k_observe_win(const KParams P, const int32_t *agent_id, float *obs) {
     extern __shared__ uint4 smem_u4[];
     const int S = P.d.S, M = P.d.M, TP = P.d.obs_pitch;
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
     const int ag = agent_id[b];
     if (ag < 0) return;
-    const char *row = P.state + (size_t)b * P.L.total;
-    const char *scen_row = P.scen + (size_t)P.scen_id[b] * P.L.scen_total;
-    const double *par = (const double *)(scen_row + P.L.soff[WRSN_S_PAR]);
-    const int N = (int)par[WRSN_P_NNODES];                      /* this scenario's nodes (P.d.N, the batch's largest, sizes smem) */
+    const WrsnRow rw(P.L, P.state, P.scen, P.scen_id, b);
+    const ObsGrid g(rw.par, S);
+    const int N = rw.N;                                         /* (P.d.N, the batch's largest, sizes smem) */
     const int NS = N + 2 * M;                                   /* nodes | chargers as channel-3 sources | as channel-4 sources */
     float *gxw = reinterpret_cast<float *>(smem_u4);            /* [NS][OBW] */
     float *gyw = gxw + (size_t)NS * OBW;                        /* [NS][OBM + OBW + OBM] */
     float *own = gyw + (size_t)NS * (OBW + 2 * OBM);            /* [2][TP]: the observer's own position, full width */
     WinSrc *win = reinterpret_cast<WinSrc *>(own + 2 * TP);     /* [NS] */
-    const double *nx = (const double *)(scen_row + P.L.soff[WRSN_S_NX]);
-    const double *ny = (const double *)(scen_row + P.L.soff[WRSN_S_NY]);
-    const double *energy = (const double *)(row + P.L.off[WRSN_F_ENERGY]);
-    const double *cs = (const double *)(row + P.L.off[WRSN_F_CS]);
-    const uint8_t *status = (const uint8_t *)(row + P.L.off[WRSN_F_STATUS]);
-    const double *mc = (const double *)(row + P.L.off[WRSN_F_MC]);
-    const float *tab_gx = (const float *)(scen_row + P.L.soff[WRSN_S_OBS_GX]), *tab_gy = (const float *)(scen_row + P.L.soff[WRSN_S_OBS_GY]);
-    const double f0 = par[WRSN_P_F0], f1 = par[WRSN_P_F1], f2 = par[WRSN_P_F2], f3 = par[WRSN_P_F3];
-    const double Wd = f1 - f0, Hd = f3 - f2;
-    const double unit = 1.0 / (double)S, start = unit / 2.0, delta = (start + unit) - start;   /* np.arange(unit/2, 1.0, unit) */
-    const double R = par[WRSN_P_MC_R], mtm = par[WRSN_P_MTM];
-    const double *me = mc + (size_t)ag * WRSN_MC_LEN;
     /* ---- stage every source: one warp per source */
     for (int q = wrp; q < NS + 1; q += OBW_THREADS / 32) {
-        if (q == NS) {                                          /* channel 2: own position, bandwidth 0.5 min(W, H) / extent */
-            const double tmp = fmin(Hd, Wd);
-            const double x0 = (me[WRSN_MC_X] - f0) / Wd, y0 = (me[WRSN_MC_Y] - f2) / Hd;
-            const double hx = 0.5 * tmp / Wd, hy = 0.5 * tmp / Hd, w = me[WRSN_MC_ENERGY] / par[WRSN_P_MC_CAP];
-            const double dnx = -2.0 * (hx * hx), dny = -2.0 * (hy * hy);
+        if (q == NS) {                                          /* channel 2: own position */
+            const ObsSrc v = obs_source(rw, g, ag, 1, 0);
+            const double dnx = -2.0 * (v.hx * v.hx), dny = -2.0 * (v.hy * v.hy);
             for (int i = lane; i < TP; i += 32) {
-                const double cc = start + (double)i * delta, ux = cc - x0, uy = cc - y0;
-                const double ax = ux * ux / dnx, ay = uy * uy / dny;
-                own[i] = (float)((i < S && ax > -745.2) ? w * exp(ax) : 0.0);
-                own[TP + i] = (float)((i < S && ay > -745.2) ? exp(ay) : 0.0);
+                own[i] = (float)(i < S ? v.w * obs_gauss(g.cell(i), v.x0, dnx) : 0.0);
+                own[TP + i] = (float)(i < S ? obs_gauss(g.cell(i), v.y0, dny) : 0.0);
             }
             continue;
         }
-        bool used = false;
-        double x0 = 0.0, y0 = 0.0, w = 0.0;
-        int node = -1;
-        if (q < N) {                                            /* channel 1: alive nodes with traffic */
-            if (status[q] != 0) {
-                w = (cs[q] / par[WRSN_P_MC_AB2]) / ((energy[q] - par[WRSN_P_THR]) / par[WRSN_P_CAPMTHR]);
-                used = w != 0.0; node = q;
-                x0 = (nx[q] - f0) / Wd; y0 = (ny[q] - f2) / Hd;
-            }
-        } else {                                                /* channels 3 / 4: the other chargers at their destinations */
-            const int a = (q - N) % M, ch = q < N + M ? 2 : 3;
-            const double *an = mc + (size_t)a * WRSN_MC_LEN;
-            const bool charging = an[WRSN_MC_TYPE] != 0.0;
-            if (a != ag && (ch == 2 ? charging : !charging)) {
-                used = true;
-                x0 = (an[WRSN_MC_CPA0] - f0) / Wd; y0 = (an[WRSN_MC_CPA1] - f2) / Hd;
-                if (ch == 2) w = an[WRSN_MC_CPA2] / par[WRSN_P_CTM];
-                else {                                          /* SURVEY Q5: the observer's destination y; / moving_time_max folded in */
-                    const double dx = an[WRSN_MC_X] - an[WRSN_MC_CPA0], dy = an[WRSN_MC_Y] - me[WRSN_MC_CPA1];
-                    w = sqrt(dx * dx + dy * dy) / par[WRSN_P_MC_V] / mtm;
-                }
-            }
-        }
+        /* channel 1: alive nodes with traffic; channels 3 / 4: the other chargers at their destinations */
+        const ObsSrc v = q < N ? obs_source(rw, g, ag, 0, q) : obs_source(rw, g, ag, q < N + M ? 2 : 3, (q - N) % M);
+        const double w = v.mode == 1 ? v.w / g.mtm : v.w;
         int sx = -100000, sy = -100000;
-        if (used) {
-            sx = (((int)floor(x0 * (double)S) - OBW / 2) >> 2) << 2; sy = (((int)floor(y0 * (double)S) - OBW / 2) >> 2) << 2;
+        if (v.mode >= 0) {
+            sx = (((int)floor(v.x0 * (double)S) - OBW / 2) >> 2) << 2; sy = (((int)floor(v.y0 * (double)S) - OBW / 2) >> 2) << 2;
             sx = sx < 0 ? 0 : (sx > S - OBW ? S - OBW : sx); sy = sy < 0 ? 0 : (sy > S - OBW ? S - OBW : sy);
             float *gx = gxw + (size_t)q * OBW, *gy = gyw + (size_t)q * (OBW + 2 * OBM);
-            if (node >= 0) {                                    /* scaled copy of the scenario's table rows */
+            if (v.node >= 0) {                                  /* scaled copy of the scenario's table rows */
                 const float wq = (float)w;
-                const float *rx = tab_gx + (size_t)node * TP, *ry = tab_gy + (size_t)node * TP;
+                const float *rx = rw.tab_gx + (size_t)v.node * TP, *ry = rw.tab_gy + (size_t)v.node * TP;
                 for (int i = lane; i < OBW; i += 32) gx[i] = rx[sx + i] * wq;
                 for (int i = lane; i < OBW + 2 * OBM; i += 32) {
                     const int k = i - OBM;
                     gy[i] = (k >= 0 && k < OBW) ? ry[sy + k] : 0.f;
                 }
             } else {
-                const double hx = R / Wd, hy = R / Hd, dnx = -2.0 * (hx * hx), dny = -2.0 * (hy * hy);
-                for (int i = lane; i < OBW; i += 32) {
-                    const double ux = (start + (double)(sx + i) * delta) - x0, ax = ux * ux / dnx;
-                    gx[i] = (float)(ax > -745.2 ? w * exp(ax) : 0.0);
-                }
+                const double dnx = -2.0 * (v.hx * v.hx), dny = -2.0 * (v.hy * v.hy);
+                for (int i = lane; i < OBW; i += 32) gx[i] = (float)(w * obs_gauss(g.cell(sx + i), v.x0, dnx));
                 for (int i = lane; i < OBW + 2 * OBM; i += 32) {
                     const int k = i - OBM;
-                    float v = 0.f;
-                    if (k >= 0 && k < OBW) { const double uy = (start + (double)(sy + k) * delta) - y0, ay = uy * uy / dny; v = (float)(ay > -745.2 ? exp(ay) : 0.0); }
-                    gy[i] = v;
+                    gy[i] = (k >= 0 && k < OBW) ? (float)obs_gauss(g.cell(sy + k), v.y0, dny) : 0.f;
                 }
             }
         }
@@ -628,13 +529,10 @@ __global__ void __launch_bounds__(32 * LOC_WARPS) k_decode_locate(const KParams 
     const int flat0 = (int)action[3 * (size_t)b];
     double out_x, out_y;
     {
-        const char *row = P.state + (size_t)b * P.L.total;
-        const char *scen_row = P.scen + (size_t)P.scen_id[b] * P.L.scen_total;
-        const double *par = (const double *)(scen_row + P.L.soff[WRSN_S_PAR]);
-        const int N = (int)par[WRSN_P_NNODES];               /* this scenario's nodes */
-        const double *nx = (const double *)(scen_row + P.L.soff[WRSN_S_NX]), *ny = (const double *)(scen_row + P.L.soff[WRSN_S_NY]);
-        const double *energy = (const double *)(row + P.L.off[WRSN_F_ENERGY]), *cs = (const double *)(row + P.L.off[WRSN_F_CS]);
-        const uint8_t *status = (const uint8_t *)(row + P.L.off[WRSN_F_STATUS]);
+        const WrsnRow rw(P.L, P.state, P.scen, P.scen_id, b);
+        const double *par = rw.par, *nx = rw.nx, *ny = rw.ny, *energy = rw.energy, *cs = rw.cs;
+        const uint8_t *status = rw.status;
+        const int N = rw.N;
         const double f0 = par[WRSN_P_F0], f1 = par[WRSN_P_F1], f2 = par[WRSN_P_F2], f3 = par[WRSN_P_F3];
         const double R = par[WRSN_P_MC_R], alpha = par[WRSN_P_MC_ALPHA], beta = par[WRSN_P_MC_BETA], thr = par[WRSN_P_THR];
         const double unit = 1.0 / (double)S;
@@ -746,11 +644,8 @@ __global__ void __launch_bounds__(ORD_THREADS) k_step_order(const KParams P, int
         const int raid = P.req.agent_id ? P.req.agent_id[b] : 0;
         int bin = 4;
         if (!((P.mask && !P.mask[b]) || (P.mask_mode == 1 && raid < 0 && raid != -4))) {
-            const char *row = P.state + (size_t)b * P.L.total;
-            const double *hdr = reinterpret_cast<const double *>(row + P.L.off[WRSN_F_HDR]);
-            const double *mc = reinterpret_cast<const double *>(row + P.L.off[WRSN_F_MC]);
-            const double *proc = reinterpret_cast<const double *>(row + P.L.off[WRSN_F_PROC]);
-            const double *par = reinterpret_cast<const double *>(P.scen + (size_t)P.scen_id[b] * P.L.scen_total + P.L.soff[WRSN_S_PAR]);
+            const WrsnRow rw(P.L, P.state, P.scen, P.scen_id, b);
+            const double *hdr = rw.hdr, *mc = rw.mc, *proc = rw.proc, *par = rw.par;
             const double now = hdr[WRSN_H_NOW];
             const bool fresh = hdr[WRSN_H_INFLIGHT] == 0.0 && aid >= 0 && aid < M && P.action_in;
             double rem = INFINITY;
@@ -799,14 +694,11 @@ __global__ void __launch_bounds__(32 * CHG_WARPS) k_charge(const KParams P, cons
     const int b = blockIdx.x * CHG_WARPS + wrp;
     if (b >= P.d.B) return;                                   /* whole warps leave together; only __syncwarp below */
     const int NP = P.d.N, M = P.d.M;                          /* node_rate's row pitch: the batch's largest node count */
-    const char *row = P.state + (size_t)b * P.L.total;
-    const char *scen_row = P.scen + (size_t)P.scen_id[b] * P.L.scen_total;
-    const double *par = (const double *)(scen_row + P.L.soff[WRSN_S_PAR]);
-    const int N = (int)par[WRSN_P_NNODES];                    /* this scenario's nodes; node_rate[b][N..NP) is left untouched */
-    const double *nx = (const double *)(scen_row + P.L.soff[WRSN_S_NX]), *ny = (const double *)(scen_row + P.L.soff[WRSN_S_NY]);
-    const uint8_t *status = (const uint8_t *)(row + P.L.off[WRSN_F_STATUS]);
-    const double *mc = (const double *)(row + P.L.off[WRSN_F_MC]);
-    const double R = par[WRSN_P_MC_R], alpha = par[WRSN_P_MC_ALPHA], beta = par[WRSN_P_MC_BETA];
+    const WrsnRow rw(P.L, P.state, P.scen, P.scen_id, b);
+    const int N = rw.N;                                       /* this scenario's nodes; node_rate[b][N..NP) is left untouched */
+    const double *nx = rw.nx, *ny = rw.ny, *mc = rw.mc;
+    const uint8_t *status = rw.status;
+    const double R = rw.par[WRSN_P_MC_R], alpha = rw.par[WRSN_P_MC_ALPHA], beta = rw.par[WRSN_P_MC_BETA];
     for (int m = lane; m < M; m += 32) {                      /* stage the chargers of this environment */
         s_mx[wrp][m] = mc[(size_t)m * WRSN_MC_LEN + WRSN_MC_X];
         s_my[wrp][m] = mc[(size_t)m * WRSN_MC_LEN + WRSN_MC_Y];
@@ -859,6 +751,7 @@ __global__ void k_record_transitions(int B, int M, wrsn_request req, int64_t t, 
 }
 
 #include "wrsn_abi_host.h"
+#include "wrsn_abi_aux.h"
 static_assert(WRSN_DEC_MAX_RANK == DEC_MAXR - 2, "the host refuses the map sizes whose rank k_decode_map cannot hold");
 
 template <int MODE>
@@ -916,21 +809,16 @@ int wrsn_device_ok(void) {
     return 1;
 }
 
-int wrsn_build_obs_tables(const wrsn_dims *d, void *scen, void *stream) {
-    if (check_dims(d)) return -1;
-    if (!scen) WRSN_FAIL("scen is NULL");
-    WrsnLayout L; wrsn_make_layout(d, &L);
-    k_obs_tables<<<dim3(d->n_scen, d->Npad), 128, 0, (cudaStream_t)stream>>>(*d, L, (char *)scen);
+}  /* extern "C" */
+
+static int launch_obs_tables(KParams &P, void *stream) {
+    k_obs_tables<<<dim3(P.d.n_scen, P.d.Npad), 128, 0, (cudaStream_t)stream>>>(P.d, P.L, const_cast<char *>(P.scen));
     WRSN_CUDA(cudaGetLastError());
     return 0;
 }
 
-int wrsn_observe(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
-                 const int32_t *agent_id, void *obs, int obs_f64, void *stream) {
-    if (check_dims(d)) return -1;
-    if (!agent_id || !obs || !scen || !scen_id || !state) WRSN_FAIL("NULL argument");
-    KParams P = base_params(d, scen, scen_id, const_cast<void *>(state), nullptr);
-    wrsn_make_layout(&P.d, &P.L);
+static int launch_observe(KParams &P, const int32_t *agent_id, void *obs, int obs_f64, void *stream) {
+    const wrsn_dims *d = &P.d;
     if (obs_f64) {
         size_t smem = sizeof(double) * 2 * 16 * (size_t)d->obs_pitch;
         if (smem > 200 * 1024) WRSN_FAIL("map_size too large");
@@ -938,26 +826,18 @@ int wrsn_observe(const wrsn_dims *d, const void *scen, const int32_t *scen_id, c
         k_observe<double, OBS_TJ64, OBS_THREADS64><<<d->B, OBS_THREADS64, smem, (cudaStream_t)stream>>>(P, agent_id, (double *)obs);
     } else {
         /* the windowed raster: map sizes it is laid out for, sources narrow enough for its window (the host layer says so in
-           dims.obs_sigma_cells: the largest charging_range / extent * S over the scenarios; 0 = unknown), shared memory */
-        const float sg = d->obs_sigma_cells;
-        /* (measured: the 40-cell window — 4 CTAs per SM — beats the chunked raster; 56 / 72 cells leave 3 / 2 CTAs per SM and
+           dims.obs_sigma_cells: the largest charging_range / extent * S over the scenarios; 0 = unknown), shared memory
+           (measured: the 40-cell window — 4 CTAs per SM — beats the chunked raster; 56 / 72 cells leave 3 / 2 CTAs per SM and
            lose to it, 0.79 ms against 0.52 ms per 4096 maps at 72: wider sources stay with the chunked kernel) */
-        const int obw = (sg > 0.0f && sg <= 2.9f) ? 40 : 0;
-        const size_t wsmem = sizeof(float) * ((size_t)(d->N + 2 * d->M) * (obw + obw + 2 * OBM) + 2 * (size_t)d->obs_pitch) + sizeof(WinSrc) * (size_t)(d->N + 2 * d->M);
-        if (obw > 0 && OBS_TJ32 == 20 && d->S % 20 == 0 && d->S >= obw && (d->S / OBS_TI) * (d->S / OBS_TJ32) <= OBW_THREADS && wsmem <= 100 * 1024) {
+        const float sg = d->obs_sigma_cells;
+        const size_t wsmem = sizeof(float) * ((size_t)(d->N + 2 * d->M) * (OBW + OBW + 2 * OBM) + 2 * (size_t)d->obs_pitch) + sizeof(WinSrc) * (size_t)(d->N + 2 * d->M);
+        if (sg > 0.0f && sg <= 2.9f && d->S % 20 == 0 && d->S >= OBW && (d->S / OBS_TI) * (d->S / OBS_TJ32) <= OBW_THREADS && wsmem <= 100 * 1024) {
             static bool wattr[WRSN_MAX_DEVICES];
             int dev = 0;
             WRSN_CUDA(cudaGetDevice(&dev));
             if (dev < 0 || dev >= WRSN_MAX_DEVICES) WRSN_FAIL("device ordinal %d not supported", dev);
-            if (!wattr[dev]) {
-                WRSN_CUDA(cudaFuncSetAttribute(k_observe_win<40>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-                WRSN_CUDA(cudaFuncSetAttribute(k_observe_win<56>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-                WRSN_CUDA(cudaFuncSetAttribute(k_observe_win<72>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-                wattr[dev] = true;
-            }
-            if (obw == 40) k_observe_win<40><<<d->B, OBW_THREADS, wsmem, (cudaStream_t)stream>>>(P, agent_id, (float *)obs);
-            else if (obw == 56) k_observe_win<56><<<d->B, OBW_THREADS, wsmem, (cudaStream_t)stream>>>(P, agent_id, (float *)obs);
-            else k_observe_win<72><<<d->B, OBW_THREADS, wsmem, (cudaStream_t)stream>>>(P, agent_id, (float *)obs);
+            if (!wattr[dev]) { WRSN_CUDA(cudaFuncSetAttribute(k_observe_win, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024)); wattr[dev] = true; }
+            k_observe_win<<<d->B, OBW_THREADS, wsmem, (cudaStream_t)stream>>>(P, agent_id, (float *)obs);
             WRSN_CUDA(cudaGetLastError());
             return 0;
         }
@@ -974,50 +854,24 @@ int wrsn_observe(const wrsn_dims *d, const void *scen, const int32_t *scen_id, c
     return 0;
 }
 
-int wrsn_decode_density_map(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
-                            const int32_t *agent_id, const void *dmap, int dmap_f64, double *action_out, void *stream) {
-    if (check_dims(d)) return -1;
-    if (!agent_id || !dmap || !action_out || !scen || !scen_id || !state) WRSN_FAIL("NULL argument");
-    KParams P = base_params(d, scen, scen_id, const_cast<void *>(state), nullptr);
-    wrsn_make_layout(&P.d, &P.L);
-    if (check_decode_size(d)) return -1;
-    LinMap lin; memset(&lin, 0, sizeof(lin));
-    if (dmap_f64) k_decode_map<double, 0><<<d->B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, (const double *)dmap, action_out, lin);
-    else k_decode_map<float, 0><<<d->B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, (const float *)dmap, action_out, lin);
-    k_decode_locate<<<(d->B + LOC_WARPS - 1) / LOC_WARPS, 32 * LOC_WARPS, 0, (cudaStream_t)stream>>>(P, agent_id, action_out);
-    WRSN_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int wrsn_decode_linear_controller(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
-                                  const int32_t *agent_id, const float *obs, int channels, const float *weights,
-                                  double *action_out, void *stream) {
-    if (check_dims(d)) return -1;
-    if (!agent_id || !obs || !weights || !action_out || !scen || !scen_id || !state) WRSN_FAIL("NULL argument");
-    if (channels < 1 || channels > 8) WRSN_FAIL("1 to 8 channels");
-    KParams P = base_params(d, scen, scen_id, const_cast<void *>(state), nullptr);
-    wrsn_make_layout(&P.d, &P.L);
-    if (check_decode_size(d)) return -1;
+/* channels = 0: dmap is the map (float64 if dmap_f64); otherwise the float observations, combined with weights[channels] */
+static int launch_decode(KParams &P, const int32_t *agent_id, const void *dmap, int dmap_f64, int channels, const float *weights,
+                         double *action_out, void *stream) {
+    const int B = P.d.B;
     LinMap lin; memset(&lin, 0, sizeof(lin));
     lin.C = channels;
     for (int k = 0; k < channels; k++) lin.w[k] = weights[k];
-    if (channels == 4) k_decode_map<float, 4><<<d->B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, obs, action_out, lin);
-    else k_decode_map<float, -1><<<d->B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, obs, action_out, lin);
-    k_decode_locate<<<(d->B + LOC_WARPS - 1) / LOC_WARPS, 32 * LOC_WARPS, 0, (cudaStream_t)stream>>>(P, agent_id, action_out);
+    if (channels == 0 && dmap_f64) k_decode_map<double, 0><<<B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, (const double *)dmap, action_out, lin);
+    else if (channels == 0) k_decode_map<float, 0><<<B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, (const float *)dmap, action_out, lin);
+    else if (channels == 4) k_decode_map<float, 4><<<B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, (const float *)dmap, action_out, lin);
+    else k_decode_map<float, -1><<<B, DEC_THREADS, 0, (cudaStream_t)stream>>>(P, agent_id, (const float *)dmap, action_out, lin);
+    k_decode_locate<<<(B + LOC_WARPS - 1) / LOC_WARPS, 32 * LOC_WARPS, 0, (cudaStream_t)stream>>>(P, agent_id, action_out);
     WRSN_CUDA(cudaGetLastError());
     return 0;
 }
 
-int wrsn_k_charge(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state, const uint8_t *charging,
-                  double *node_rate, double *mc_rate, void *stream) {
-    if (check_dims(d)) return -1;
-    if (!scen || !scen_id || !state || !node_rate || !mc_rate) WRSN_FAIL("NULL argument");
-    if (d->M <= 0) WRSN_FAIL("no chargers");
-    KParams P = base_params(d, scen, scen_id, const_cast<void *>(state), nullptr);
-    wrsn_make_layout(&P.d, &P.L);
-    k_charge<<<(d->B + CHG_WARPS - 1) / CHG_WARPS, 32 * CHG_WARPS, 0, (cudaStream_t)stream>>>(P, charging, node_rate, mc_rate);
+static int launch_charge(KParams &P, const uint8_t *charging, double *node_rate, double *mc_rate, void *stream) {
+    k_charge<<<(P.d.B + CHG_WARPS - 1) / CHG_WARPS, 32 * CHG_WARPS, 0, (cudaStream_t)stream>>>(P, charging, node_rate, mc_rate);
     WRSN_CUDA(cudaGetLastError());
     return 0;
 }
-
-}  /* extern "C" */

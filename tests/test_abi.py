@@ -86,6 +86,62 @@ def test_emulation_dims_and_layouts_equal_the_cuda_library(cuda_so):
             assert rcs[1] != 0 and rcs[2] != 0 and msg in L.wrsn_last_error()
 
 
+def test_emulation_entry_point_checks_equal_the_cuda_library(cuda_so):
+    """wrsn_observe, wrsn_k_charge and both decode entry points check their arguments in the shared host side of the ABI: both
+    libraries refuse the same inputs with the same message.  No input here passes the checks, so nothing is launched."""
+    import numpy as np
+    libs = [_lib._bind(cuda_so), _lib._bind(ctypes.CDLL(os.path.join(REPO, "tests", "emu", "libwrsn_emu.so")))]
+    max_mc = _lib.enums()["WRSN_MAX_MC"]
+
+    def dims(L, M=3, S=100, finalize=True):
+        d = _lib.Dims()
+        d.B, d.N, d.T, d.M, d.S, d.Emax, d.TEmax, d.n_scen = 2, 100, 100, M, S, 600, 200, 1
+        if finalize:
+            assert L.wrsn_dims_finalize(ctypes.byref(d)) == 0
+        return d
+
+    # zeroed buffers large enough for every case, and no row with an observer: an entry point that skipped its checks would
+    # return 0 instead of touching memory it does not own
+    big = dims(libs[0], M=max_mc + 1, S=177)
+    B, N, M, S = big.B, big.N, big.M, big.S
+    arrays = dict(scen=np.zeros(big.scen_bytes * big.n_scen, np.uint8), scen_id=np.zeros(B, np.int32),
+                  state=np.zeros(big.state_bytes * B, np.uint8), agent=np.full(B, -1, np.int32),
+                  obs=np.zeros(B * 4 * S * S, np.float64), map=np.zeros(B * S * S, np.float64),
+                  action=np.zeros(B * 3, np.float64), node=np.zeros(B * N, np.float64), mc=np.zeros(B * M, np.float64))
+    weights = (ctypes.c_float * 9)(*([1.0] * 9))
+
+    def call(L, name, d, null=None, channels=4):
+        p = {k: (None if k == null else a.ctypes.data) for k, a in arrays.items()}
+        rd = ctypes.byref(d)
+        if name == "observe":
+            rc = L.wrsn_observe(rd, p["scen"], p["scen_id"], p["state"], p["agent"], p["obs"], 1, None)
+        elif name == "k_charge":
+            rc = L.wrsn_k_charge(rd, p["scen"], p["scen_id"], p["state"], None, p["node"], p["mc"], None)
+        elif name == "decode_density_map":
+            rc = L.wrsn_decode_density_map(rd, p["scen"], p["scen_id"], p["state"], p["agent"], p["map"], 1, p["action"], None)
+        else:
+            rc = L.wrsn_decode_linear_controller(rd, p["scen"], p["scen_id"], p["state"], p["agent"], p["obs"], channels, weights,
+                                                 p["action"], None)
+        return rc, L.wrsn_last_error()
+
+    every = ("observe", "k_charge", "decode_density_map", "decode_linear_controller")
+    cases = [(every, dict(finalize=False), {}, b"dims not finalized"),
+             (every, dict(M=max_mc + 1), {}, b"bad dims"),
+             (every, {}, dict(null="state"), b"NULL argument"),
+             (every, {}, dict(null="scen_id"), b"NULL argument"),
+             (("observe",), {}, dict(null="obs"), b"NULL argument"),
+             (("k_charge",), {}, dict(null="node"), b"NULL argument"),
+             (("decode_density_map",), {}, dict(null="map"), b"NULL argument"),
+             (("decode_linear_controller",), {}, dict(channels=0), b"1 to 8 channels"),
+             (("decode_linear_controller",), {}, dict(channels=9), b"1 to 8 channels"),
+             (("decode_density_map", "decode_linear_controller"), dict(S=177), {}, b"map_size = 177")]
+    for names, dkw, ckw, msg in cases:
+        for name in names:
+            got = [call(L, name, dims(L, **dkw), **ckw) for L in libs]
+            assert got[0] == got[1], (name, dkw, ckw, got)
+            assert got[0][0] == -1 and msg in got[0][1], (name, dkw, ckw, got)
+
+
 def test_no_cpu_path():
     """Without a GPU the product host layer must refuse loudly, not fall back."""
     import torch

@@ -238,6 +238,37 @@ def test_mixed_equals_homogeneous_random_controller(dev, kind, threads):
     assert cnt["decisions"] > 500
 
 
+def test_charge_rates_leave_padding_nodes_alone(dev):
+    """wrsn_k_charge on a mixed batch whose smaller scenarios' padding nodes are alive, with a charger on top of them (the
+    scenario record holds them at the origin): each row's rates are the reference's over its own nodes, and the padding columns
+    of node_rate keep what the caller put there."""
+    from oracle.wrsn_oracle import charge_rates_reference
+    gs, env = _golden_batch(("ep_basic_n50", "ep_full_n100", "ep_full_n200"), dev)      # 82 / 98 / 132 nodes
+    env.reset()
+    E, sid, Ns = env.E, _np(env.scen_id), _np(env.num_nodes)
+    assert Ns.min() < env.N
+    env.view("status")[:] = 1                                      # padding columns included
+    mc = env.view("mc")
+    for b in range(env.B):
+        nodes = env.scenarios[sid[b]].nodes
+        mc[b, 0, E["WRSN_MC_X"]], mc[b, 0, E["WRSN_MC_Y"]] = 0.0, 0.0
+        for a in range(1, env.M):                                  # a few metres off a node: several nodes within range
+            mc[b, a, E["WRSN_MC_X"]], mc[b, a, E["WRSN_MC_Y"]] = float(nodes[7 * a][0]) + 3.0, float(nodes[7 * a][1]) - 2.0
+    sentinel = -7.25
+    out = (torch.full((env.B, env.N), sentinel, dtype=torch.float64, device=env.device),
+           torch.zeros((env.B, env.M), dtype=torch.float64, device=env.device))
+    node_rate, mc_rate = (_np(t) for t in env.charge_rates(out=out))
+    status, mx, my, mcp = _np(env.view("status")), _np(env.mc("X")), _np(env.mc("Y")), env.mc_type
+    for b in range(env.B):
+        N = int(Ns[b])
+        rr, cr = charge_rates_reference(env.scenarios[sid[b]].nodes, status[b, :N], np.stack([mx[b], my[b]], 1), np.ones(env.M),
+                                        mcp["charging_range"], mcp["alpha"], mcp["beta"])
+        assert (rr != 0).sum() >= 2 and (cr[1:] != 0).all(), b
+        np.testing.assert_allclose(node_rate[b, :N], rr, rtol=1e-14, atol=0, err_msg=str(b))
+        np.testing.assert_allclose(mc_rate[b], cr, rtol=1e-14, atol=0, err_msg=str(b))
+        assert (node_rate[b, N:] == sentinel).all(), b
+
+
 # ------------------------------------------------------------------ 3. against the C oracle
 def test_mixed_vs_oracle(dev):
     scs = [synthetic(num_nodes=40, num_targets=120, seed=3, num_gateways=2), synthetic(num_nodes=60, num_targets=70, seed=11),

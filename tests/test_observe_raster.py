@@ -1,4 +1,4 @@
-"""Observation rasters (``wrsn_observe``: ``k_observe<double>``, ``k_observe<float>`` chunked, ``k_observe_win<40>``) against the
+"""Observation rasters (``wrsn_observe``: ``k_observe<double>``, ``k_observe<float>`` chunked, ``k_observe_win``) against the
 float64 restatement of ``WRSN.get_state`` (oracle/obs_oracle.py), across map sizes, field shapes, node and charger counts.
 
 The restatement is pinned first, against the golden episodes and against the C oracle.  Then every case builds a batch,
@@ -131,7 +131,7 @@ CASES = ([("size%d" % S, S, "square", 100, 3, False) for S in (1, 2, 3, 7, 17, 3
 
 
 def windowed_eligible(d):
-    """wrsn_observe's choice of k_observe_win<40> (wrsn_kernels.cu), restated: narrow sources, a map size the window's tiles
+    """wrsn_observe's choice of k_observe_win (wrsn_kernels.cu), restated: narrow sources, a map size the window's tiles
     cover, and the staged sources within 100 KB of shared memory."""
     sg = np.float32(d.obs_sigma_cells)
     wsmem = 4 * ((d.N + 2 * d.M) * (40 + 40 + 2 * 16) + 2 * d.obs_pitch) + 8 * (d.N + 2 * d.M)

@@ -1,4 +1,11 @@
-"""Time the fp32 observation raster of the tuning builds (tools/build_obs_variants.sh): python tools/time_observe.py <k> [B]"""
+"""Time the fp32 observation raster: python tools/time_observe.py <k> [B]
+
+k = "base" times the package's libwrsn_b200.so; any other k times multi_agent_rl_wrsn_b200/csrc/libwrsn_b200_obs<k>.so, another
+build of the library, such as the parent commit's, for an A/B comparison in one process:
+
+  nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -fmad=false -std=c++17 -Xcompiler -fPIC -shared -I include \
+       -o multi_agent_rl_wrsn_b200/csrc/libwrsn_b200_obs<k>.so <other tree>/multi_agent_rl_wrsn_b200/csrc/wrsn_kernels.cu
+"""
 import ctypes, os, sys
 import numpy as np, torch
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
