@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define WRSN_ABI_VERSION 20
+#define WRSN_ABI_VERSION 21
 #define WRSN_MAX_MC 16          /* chargers per environment */
 #define WRSN_RING 10            /* Node.operate keeps the last 10 per-second consumptions (Node.py:70-77) */
 
@@ -267,6 +267,19 @@ int wrsn_decode_linear_controller(const wrsn_dims *d, const void *scen, const in
 int wrsn_record_transitions(const wrsn_dims *d, const wrsn_request *req, int64_t t, const int64_t *agent_prev,
                             int64_t *last, double *resets_seen, int64_t *agent_next, int64_t *link_next,
                             uint8_t *new_episode_next, double *reward_next, double *now_next, void *stream);
+/* Copy the continuation state of n environments: for i < n, row src_rows[i] of (src_state, src_req, src_scen_id) is copied
+ * to row dst_rows[i] of (dst_state, dst_req, dst_scen_id): the whole state record (state_bytes), scen_id, and the request
+ * row (agent_id, terminal, reward, now, action[3], detail[2], flags; stats[3] and sticky when both sides have them; never
+ * `order`, which is launch scratch).  A row in flight (agent_id -4) stays in flight and continues at the next step call.
+ * Pairs whose index lies outside [0, src_B) / [0, dst_B) are skipped.  dst rows must be distinct, and when source and
+ * destination are the same buffers no row may be both (the result is undefined otherwise).
+ * Both sides share d's layout: a record is a pure function of its scenario and the actions it was given (SURVEY Q8), so a
+ * copied row continues exactly as its source would.  Fork (src = dst buffers), snapshot (dst = a compact buffer of n rows)
+ * and restore (src = such a buffer) are all this one call.  n == 0 does nothing. */
+int wrsn_copy_rows(const wrsn_dims *d, int32_t n,
+                   const void *src_state, const wrsn_request *src_req, const int32_t *src_scen_id, const int32_t *src_rows, int32_t src_B,
+                   void *dst_state, const wrsn_request *dst_req, int32_t *dst_scen_id, const int32_t *dst_rows, int32_t dst_B,
+                   void *stream);
 /* WRSN.get_network_fitness (:188-220): per-target values fitness[B][T] (may be NULL) and their minimum fit_min[B] over the row's own
  * targets; the columns beyond a row's own target count are not written. */
 int wrsn_fitness(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state,

@@ -5,10 +5,11 @@
 """
 from .scenario import Scenario, build_static, load_mc_type, synthetic  # noqa: F401
 from .batched import BatchedWRSN, Requests  # noqa: F401
+from .snapshot import EnvSnapshot  # noqa: F401
 from .wrsn import WRSN  # noqa: F401
 from .ippo import BatchedIPPO  # noqa: F401
 from .controllers import (BatchedRandomController, IPPORollout, PerAgentPolicy, allreduce_gradients, ppo_update,  # noqa: F401
                           rollout, select_batch)  # noqa: F401
 
-__all__ = ["Scenario", "build_static", "load_mc_type", "synthetic", "BatchedWRSN", "Requests", "WRSN", "BatchedIPPO",
+__all__ = ["Scenario", "build_static", "load_mc_type", "synthetic", "BatchedWRSN", "Requests", "EnvSnapshot", "WRSN", "BatchedIPPO",
            "BatchedRandomController", "IPPORollout", "PerAgentPolicy", "allreduce_gradients", "ppo_update", "rollout", "select_batch"]

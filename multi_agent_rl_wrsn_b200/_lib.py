@@ -74,6 +74,8 @@ def _bind(L):
     L.wrsn_rollout_step.argtypes = [dp, vp, vp, vp, vp, vp, C.POINTER(Request), vp, ip, vp]
     L.wrsn_observe.argtypes = [dp, vp, vp, vp, vp, vp, ip, vp]
     L.wrsn_record_transitions.argtypes = [dp, C.POINTER(Request), C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    L.wrsn_copy_rows.argtypes = [dp, C.c_int32, vp, C.POINTER(Request), vp, vp, C.c_int32, vp, C.POINTER(Request), vp, vp,
+                                 C.c_int32, vp]
     L.wrsn_fitness.argtypes = [dp, vp, vp, vp, vp, vp, vp]
     L.wrsn_k_charge.argtypes = [dp, vp, vp, vp, vp, vp, vp, vp]
     L.wrsn_decode_density_map.argtypes = [dp, vp, vp, vp, vp, vp, ip, vp, vp]

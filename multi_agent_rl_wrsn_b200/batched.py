@@ -12,6 +12,7 @@ import torch
 
 from . import _lib
 from .scenario import Scenario, build_static, load_mc_type
+from .snapshot import LAYOUT_DIMS, REQ_FIELDS, EnvSnapshot, c_request, check_layout, layout_meta, scenario_fingerprint
 
 _NP = {"f64": np.float64, "i32": np.int32, "u8": np.uint8}
 _S_FIELDS = (  # (enum, dtype, which size)
@@ -108,6 +109,8 @@ class BatchedWRSN:
         self._all = None
         self._snap = None
         self._agent_obs = None
+        self._fingerprints = None
+        self._counts = None
         self._make_snapshot()
 
     # ------------------------------------------------------------------ plumbing
@@ -293,6 +296,104 @@ class BatchedWRSN:
         self._call(self.L.wrsn_fitness, C.byref(self.dims), self.scen.data_ptr(), self.scen_id.data_ptr(),
                                        self.state.data_ptr(), fit.data_ptr(), mn.data_ptr(), self._stream())
         return fit[:, :self.T], mn
+
+    # ------------------------------------------------------------------ copies of running environments (wrsn_copy_rows)
+    def _rows(self, rows, what):
+        """Host copy of a row list, every index in [0, B)."""
+        r = np.asarray(rows.cpu() if isinstance(rows, torch.Tensor) else rows, np.int64).reshape(-1)
+        if r.size and (r.min() < 0 or r.max() >= self.B):
+            raise ValueError("%s: row indices must lie in [0, %d)" % (what, self.B))
+        return r
+
+    def _copy_rows(self, src, src_rows, dst, dst_rows):
+        """``wrsn_copy_rows`` from ``src`` to ``dst``, each (state, wrsn_request, scen_id); the host row lists are the caller's,
+        already checked."""
+        n = len(src_rows)
+        if n == 0:
+            return
+        sr = torch.as_tensor(src_rows.astype(np.int32), device=self.device)
+        dr = torch.as_tensor(dst_rows.astype(np.int32), device=self.device)
+        (ss, sq, si), (ds, dq, di) = src, dst
+        self._call(self.L.wrsn_copy_rows, C.byref(self.dims), n, ss.data_ptr(), C.byref(sq), si.data_ptr(), sr.data_ptr(),
+                   int(ss.shape[0]), ds.data_ptr(), C.byref(dq), di.data_ptr(), dr.data_ptr(), int(ds.shape[0]), self._stream())
+
+    def _refresh_counts(self):
+        if self._counts is None:                         # node and target count of every scenario
+            self._counts = torch.as_tensor([[st["N"] for st in self.statics], [st["T"] for st in self.statics]], dtype=torch.int32,
+                                           device=self.device)
+        sid = self.scen_id.long()
+        self.num_nodes.copy_(self._counts[0][sid])
+        self.num_targets.copy_(self._counts[1][sid])
+
+    @property
+    def fingerprints(self):
+        """One ``snapshot.scenario_fingerprint`` per scenario of the batch."""
+        if self._fingerprints is None:
+            self._fingerprints = [scenario_fingerprint(st) for st in self.statics]
+        return self._fingerprints
+
+    def fork(self, src, dst):
+        """Copy the running environments ``src[i]`` onto rows ``dst[i]`` (state record, scenario and request row: see
+        ``wrsn_copy_rows``); each copy then continues exactly as its source would with the same actions, including a step in
+        flight (``agent_id == -4``).  ``dst`` rows must be distinct and disjoint from ``src``.  A destination row of another
+        scenario takes the source's (``num_nodes`` / ``num_targets`` follow)."""
+        s, d = self._rows(src, "src"), self._rows(dst, "dst")
+        if len(s) != len(d):
+            raise ValueError("src and dst must have the same length (%d != %d)" % (len(s), len(d)))
+        if len(np.unique(d)) != len(d):
+            raise ValueError("dst: rows must be distinct")
+        if np.intersect1d(s, d).size:
+            raise ValueError("dst: rows %s are also in src" % np.intersect1d(s, d)[:8].tolist())
+        me = (self.state, self.req.c, self.scen_id)
+        self._copy_rows(me, s, me, d)
+        self._refresh_counts()
+
+    def snapshot(self, rows=None, base=0):
+        """The continuation state of ``rows`` (default all) as an ``EnvSnapshot`` on this batch's device.  ``base`` is the
+        global index of local row 0 (a shard passes the start of its ``sharding.shard_range``): the snapshot records global
+        row ids."""
+        r = np.arange(self.B, dtype=np.int64) if rows is None else self._rows(rows, "rows")
+        n = len(r)
+        q = Requests(n, self.device)
+        req = {f: getattr(q, f) for f in REQ_FIELDS}
+        state = torch.zeros((n, self.dims.state_bytes), dtype=torch.uint8, device=self.device)
+        scen = torch.zeros((n,), dtype=torch.int32, device=self.device)
+        self._copy_rows((self.state, self.req.c, self.scen_id), r, (state, c_request(req), scen), np.arange(n, dtype=np.int64))
+        meta = layout_meta(self.L, self.dims, self._foff, self.fingerprints)
+        return EnvSnapshot(meta, torch.as_tensor(r + int(base), dtype=torch.int64, device=self.device), scen, state, req)
+
+    def restore(self, snap, rows=None, base=0):
+        """Write the rows of ``snap`` into this batch.  ``rows=None``: every snapshot row whose global id lies in
+        [base, base + B) goes to local row id - base; otherwise ``rows[i]`` receives the snapshot's row i.  Scenarios are
+        matched by fingerprint (the batch may list them in another order).  Raises ValueError, naming the field, for a
+        snapshot this batch cannot continue exactly: another ABI version, layout dim or offset, a scenario the batch does not
+        have, bad lengths or indices.  Returns the request record."""
+        snap.validate()
+        check_layout(snap.meta, self.L.wrsn_abi_version(), {k: getattr(self.dims, k) for k in LAYOUT_DIMS}, list(self._foff))
+        if rows is None:
+            ids = snap.ids.cpu().numpy()
+            sel = (ids >= int(base)) & (ids < int(base) + self.B)
+            src, dst = np.nonzero(sel)[0], ids[sel] - int(base)
+        else:
+            dst = self._rows(rows, "rows")
+            if len(dst) != len(snap):
+                raise ValueError("rows: %d rows for a snapshot of %d" % (len(dst), len(snap)))
+            src = np.arange(len(snap), dtype=np.int64)
+        if len(np.unique(dst)) != len(dst):
+            raise ValueError("rows: a destination row is written twice (duplicate global ids or rows)")
+        mine = {fp: k for k, fp in enumerate(self.fingerprints)}
+        table = np.array([mine.get(fp, -1) for fp in snap.meta["fingerprints"]], np.int32)
+        used = np.unique(snap.scen.cpu().numpy()[src])
+        absent = [int(k) for k in used if table[k] < 0]
+        if absent:
+            raise ValueError("fingerprints: scenario %d of the snapshot (%s) is not in this batch"
+                             % (absent[0], snap.meta["fingerprints"][absent[0]][:16]))
+        if snap.device != self.device:
+            snap = snap.to(self.device)
+        scen = torch.as_tensor(table, device=self.device)[snap.scen.long()].contiguous()
+        self._copy_rows((snap.state, c_request(snap.req), scen), src, (self.state, self.req.c, self.scen_id), dst)
+        self._refresh_counts()
+        return self.req
 
     # ------------------------------------------------------------------ lower-level entry points (tests / profiling)
     def init_network(self, with_reward_process=True, mask=None):

@@ -4,7 +4,7 @@
  * launches the environment kernel.  Included once, after the kernels; the including file supplies
  *   launch_env<MODE>(P, stream)   one launch of env_run<MODE> (wrsn_env_kernel.cuh) over the rows of the batch;
  *   order_rows(P, stream)         before a step: the order in which the launch takes the rows (P.order; NULL = index order);
- * and the CUDA build the kernel k_record_transitions.  The entry points of the raster, the decoder and the charging model:
+ * and the CUDA build the kernels k_record_transitions and k_copy_rows.  The entry points of the raster, the decoder and the charging model:
  * wrsn_abi_aux.h.
  */
 #pragma once
@@ -206,6 +206,38 @@ int wrsn_record_transitions(const wrsn_dims *d, const wrsn_request *req, int64_t
 #else
     k_record_transitions<<<(d->B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
         d->B, d->M, *req, t, agent_prev, last, resets_seen, agent_next, link_next, new_episode_next, reward_next, now_next);
+    WRSN_CUDA(cudaGetLastError());
+#endif
+    return 0;
+}
+
+int wrsn_copy_rows(const wrsn_dims *d, int32_t n,
+                   const void *src_state, const wrsn_request *src_req, const int32_t *src_scen_id, const int32_t *src_rows, int32_t src_B,
+                   void *dst_state, const wrsn_request *dst_req, int32_t *dst_scen_id, const int32_t *dst_rows, int32_t dst_B,
+                   void *stream) {
+    if (check_dims(d)) return -1;
+    if (n < 0) WRSN_FAIL("n = %d: the number of rows to copy must not be negative", n);
+    if (src_B <= 0 || dst_B <= 0) WRSN_FAIL("src_B = %d, dst_B = %d: both must be positive", src_B, dst_B);
+    if (!src_state || !dst_state || !src_rows || !dst_rows || !src_scen_id || !dst_scen_id)
+        WRSN_FAIL("a state, row list or scen_id is NULL");
+    if (!src_req || !dst_req) WRSN_FAIL("src_req / dst_req is NULL");
+    for (int side = 0; side < 2; side++) {
+        const wrsn_request *q = side ? dst_req : src_req;
+        if (!q->agent_id || !q->terminal || !q->reward || !q->now || !q->action || !q->detail || !q->flags)
+            WRSN_FAIL("%s: agent_id, terminal, reward, now, action, detail and flags must not be NULL", side ? "dst_req" : "src_req");
+    }
+    if (n == 0) return 0;
+#if defined(WRSN_HOST_EMU)
+    (void)stream;
+    for (int i = 0; i < n; i++) {
+        const int s = src_rows[i], o = dst_rows[i];
+        if (s < 0 || s >= src_B || o < 0 || o >= dst_B) continue;
+        memcpy((char *)dst_state + (size_t)o * d->state_bytes, (const char *)src_state + (size_t)s * d->state_bytes, (size_t)d->state_bytes);
+        copy_row_request(*src_req, src_scen_id, s, *dst_req, dst_scen_id, o);
+    }
+#else
+    k_copy_rows<<<n, COPY_THREADS, 0, (cudaStream_t)stream>>>(d->state_bytes, (const char *)src_state, *src_req, src_scen_id, src_rows, src_B,
+                                                              (char *)dst_state, *dst_req, dst_scen_id, dst_rows, dst_B);
     WRSN_CUDA(cudaGetLastError());
 #endif
     return 0;

@@ -750,6 +750,36 @@ __global__ void k_record_transitions(int B, int M, wrsn_request req, int64_t t, 
     record_transition(b, M, req, t, agent_prev, last, resets_seen, agent_next, link_next, new_episode_next, reward_next, now_next);
 }
 
+/* wrsn_copy_rows: one CTA per (source, destination) pair.  The state record (state_bytes, a multiple of 16) moves in 16-byte
+ * vectors, COPY_UNROLL loads in flight per thread before their stores; thread 0 copies scen_id and the request row. */
+#define COPY_THREADS 128
+#define COPY_UNROLL 4
+__global__ void __launch_bounds__(COPY_THREADS) k_copy_rows(int32_t state_bytes, const char *__restrict__ src_state, wrsn_request src_req,
+                                                            const int32_t *__restrict__ src_scen_id, const int32_t *__restrict__ src_rows,
+                                                            int32_t src_B, char *__restrict__ dst_state, wrsn_request dst_req,
+                                                            int32_t *__restrict__ dst_scen_id, const int32_t *__restrict__ dst_rows,
+                                                            int32_t dst_B) {
+    const int s = src_rows[blockIdx.x], o = dst_rows[blockIdx.x];
+    if (s < 0 || s >= src_B || o < 0 || o >= dst_B) return;
+    const uint4 *__restrict__ a = reinterpret_cast<const uint4 *>(src_state + (size_t)s * state_bytes);
+    uint4 *__restrict__ z = reinterpret_cast<uint4 *>(dst_state + (size_t)o * state_bytes);
+    const int nv = state_bytes >> 4;
+    for (int base = 0; base < nv; base += COPY_THREADS * COPY_UNROLL) {
+        uint4 v[COPY_UNROLL];
+#pragma unroll
+        for (int u = 0; u < COPY_UNROLL; u++) {
+            const int i = base + u * COPY_THREADS + (int)threadIdx.x;
+            if (i < nv) v[u] = a[i];
+        }
+#pragma unroll
+        for (int u = 0; u < COPY_UNROLL; u++) {
+            const int i = base + u * COPY_THREADS + (int)threadIdx.x;
+            if (i < nv) z[i] = v[u];
+        }
+    }
+    if (threadIdx.x == 0) copy_row_request(src_req, src_scen_id, s, dst_req, dst_scen_id, o);
+}
+
 #include "wrsn_abi_host.h"
 #include "wrsn_abi_aux.h"
 static_assert(WRSN_DEC_MAX_RANK == DEC_MAXR - 2, "the host refuses the map sizes whose rank k_decode_map cannot hold");

@@ -217,3 +217,21 @@ WRSN_HD void record_transition(int b, int M, const wrsn_request &req, int64_t t,
     reward_next[b] = (r == r) ? r : 0.0;
     now_next[b] = req.now[b];
 }
+
+/* continuation state of row s outside its state record, copied to row d (see include/wrsn_b200.h: wrsn_copy_rows): scen_id and
+ * the request row.  `order` is launch scratch of the next step call (k_step_order rewrites it from the state records), so it is
+ * not part of a row's state. */
+WRSN_HD void copy_row_request(const wrsn_request &src, const int32_t *src_scen_id, int s, const wrsn_request &dst,
+                              int32_t *dst_scen_id, int d) {
+    dst_scen_id[d] = src_scen_id[s];
+    dst.agent_id[d] = src.agent_id[s];
+    dst.terminal[d] = src.terminal[s];
+    dst.reward[d] = src.reward[s];
+    dst.now[d] = src.now[s];
+    for (int k = 0; k < 3; k++) dst.action[(size_t)d * 3 + k] = src.action[(size_t)s * 3 + k];
+    for (int k = 0; k < 2; k++) dst.detail[(size_t)d * 2 + k] = src.detail[(size_t)s * 2 + k];
+    dst.flags[d] = src.flags[s];
+    if (src.stats && dst.stats)
+        for (int k = 0; k < 3; k++) dst.stats[(size_t)d * 3 + k] = src.stats[(size_t)s * 3 + k];
+    if (src.sticky && dst.sticky) dst.sticky[d] = src.sticky[s];
+}
