@@ -285,6 +285,29 @@ int wrsn_copy_rows(const wrsn_dims *d, int32_t n,
 int wrsn_fitness(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state,
                  double *fitness, double *fit_min, void *stream);
 
+/* ---- hand-written charging rules of wrsn_heuristic_action ---- */
+enum {
+    WRSN_HEUR_MIN_LIFETIME = 0,                        /* lowest lifetime first: the greedy on-demand rule */
+    WRSN_HEUR_NEAREST_URGENT = 1,                      /* the nearest node that dies within one charging round, else lowest lifetime first */
+    WRSN_HEUR_COUNT
+};
+/* A baseline charging decision for the deciding charger a = agent_id[b] of every row with 0 <= a < M, computed from the state
+ * record; other rows of action[B][3] are left untouched.  No reference function: the reference has no such controller.
+ * Over the row's own nodes i < par[WRSN_P_NNODES] (padding nodes are never chosen):
+ *   alive      status[i] == 1
+ *   lifetime   L_i = (energy[i] - par[THR]) / energyCS[i], +inf when energyCS[i] <= 0 (the terms of get_network_fitness, :188-220)
+ *   claimed    some living charger j != a (mc[j][STATUS] != 0) has d(node i, (mc[j][CPA0], mc[j][CPA1])) <= par[MC_R]
+ *   candidates the alive nodes that are not claimed; when there are none, every alive node
+ *   WRSN_HEUR_MIN_LIFETIME    the candidate with the smallest (L_i, i)
+ *   WRSN_HEUR_NEAREST_URGENT  among the candidates with L_i < par[MTM] + par[CTM], the one with the smallest (d(charger a, node i), i);
+ *                             when there is none, the choice of WRSN_HEUR_MIN_LIFETIME
+ * The action for node i: ((x_i - F0) / (F1 - F0), (y_i - F2) / (F3 - F2), min(1, max(0, (CAP - energy[i]) / par[CAPMTHR]))),
+ * a frame fraction being 0 where the frame's width or height is 0.  With no alive node: charger a's own position, charge 0.
+ * d() is the engine's Euclidean distance (products and sum rounded separately).  Every choice is a minimum of a total order on
+ * (key, id), so the device and the host emulation agree bit for bit.  kind outside [0, WRSN_HEUR_COUNT) is refused. */
+int wrsn_heuristic_action(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
+                          const int32_t *agent_id, int kind, double *action /* [B][3] */, void *stream);
+
 /* standalone per-tick kernels (the same device functions the fused step uses; unit parity + ncu evidence) */
 int wrsn_k_bfs(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream);      /* Network.setLevels + receivers + relay counts */
 int wrsn_k_drain(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream);    /* Node.operate k+0.5 tick */

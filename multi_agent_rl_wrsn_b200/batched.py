@@ -15,6 +15,7 @@ from .scenario import Scenario, build_static, load_mc_type
 from .snapshot import LAYOUT_DIMS, REQ_FIELDS, EnvSnapshot, c_request, check_layout, layout_meta, scenario_fingerprint
 
 _NP = {"f64": np.float64, "i32": np.int32, "u8": np.uint8}
+HEURISTICS = ("min_lifetime", "nearest_urgent")     # wrsn_heuristic_action's kinds, in enum order (WRSN_HEUR_*)
 _S_FIELDS = (  # (enum, dtype, which size)
     ("WRSN_S_PAR", "f64", "P"), ("WRSN_S_NX", "f64", "Npad"), ("WRSN_S_NY", "f64", "Npad"),
     ("WRSN_S_BS_ESEND", "f64", "Npad"), ("WRSN_S_NBR_DIST", "f64", "Emax"), ("WRSN_S_NBR_ESEND", "f64", "Emax"),
@@ -286,6 +287,28 @@ class BatchedWRSN:
             raise ValueError("out must be a contiguous float64 tensor [B, 3]")
         self._call(self.L.wrsn_decode_linear_controller, C.byref(self.dims), self.scen.data_ptr(), self.scen_id.data_ptr(),
                    self.state.data_ptr(), a.data_ptr(), obs.data_ptr(), int(obs.shape[1]), w, out.data_ptr(), self._stream())
+        return out
+
+    def heuristic_action(self, kind="min_lifetime", agent_id=None, out=None):
+        """A hand-written charging decision (``wrsn_heuristic_action``) for every environment with ``agent_id[b] >= 0`` (default:
+        the deciding charger of the last request), computed from the state record: ``kind`` is one of ``HEURISTICS``,
+        ``"min_lifetime"`` (the alive node with the lowest lifetime ``(energy - threshold) / energyCS`` that no other living
+        charger is headed for) or ``"nearest_urgent"`` (the nearest such node among those that die within one worst-case move
+        plus full charge; otherwise as ``"min_lifetime"``).  -> actions [B, 3] float64 (x-frac, y-frac, charge-time frac) on
+        the device, ready for ``step`` / ``rollout_step``; the other rows of ``out`` are left untouched."""
+        if kind not in HEURISTICS:
+            raise ValueError("kind must be one of %s, not %r" % (", ".join(HEURISTICS), kind))
+        if agent_id is None:
+            agent_id = self.req.agent_id
+        a = torch.as_tensor(agent_id, device=self.device).to(torch.int32).contiguous()
+        if a.shape != (self.B,):
+            raise ValueError("agent_id must be [B]")
+        if out is None:
+            out = torch.zeros((self.B, 3), dtype=torch.float64, device=self.device)
+        if out.dtype != torch.float64 or not out.is_contiguous() or out.shape != (self.B, 3) or out.device != self.state.device:
+            raise ValueError("out must be a contiguous float64 tensor [B, 3] on the simulator's device")
+        self._call(self.L.wrsn_heuristic_action, C.byref(self.dims), self.scen.data_ptr(), self.scen_id.data_ptr(),
+                   self.state.data_ptr(), a.data_ptr(), HEURISTICS.index(kind), out.data_ptr(), self._stream())
         return out
 
     def get_network_fitness(self):

@@ -13,6 +13,7 @@ import math
 import torch
 
 from . import _lib
+from .batched import HEURISTICS, BatchedWRSN
 from .sharding import reduce_stats
 
 
@@ -26,22 +27,51 @@ class BatchedRandomController:
         return state[:, 0] + state[:, 1] - 10.0 * state[:, 2] + state[:, 3]
 
 
+class HeuristicController:
+    """A hand-written charging rule as a controller: ``kind`` is one of ``HEURISTICS`` (``BatchedWRSN.heuristic_action``).
+    The decision is computed from the state record, not from the observation, so ``rollout`` and ``evaluate`` take it
+    directly (``heuristic``) and render no observation for it."""
+
+    def __init__(self, kind="min_lifetime"):
+        if kind not in HEURISTICS:
+            raise ValueError("kind must be one of %s, not %r" % (", ".join(HEURISTICS), kind))
+        self.heuristic = kind
+
+    def make_action(self, agent_id, state, info=None, wrsn=None):
+        """Actions [B, 3] for the requests ``agent_id`` of ``wrsn`` (a ``BatchedWRSN``), or the 3-vector of charger ``agent_id``
+        when ``wrsn`` is the single-environment ``WRSN``; ``state`` is not read."""
+        if wrsn is None:
+            raise ValueError("HeuristicController.make_action needs the environment (wrsn=)")
+        if isinstance(wrsn, BatchedWRSN):
+            return wrsn.heuristic_action(self.heuristic, agent_id=agent_id)
+        return wrsn.heuristic_action(agent_id, self.heuristic)
+
+
 def rollout(env, controller, steps, obs=None, group=None):
     """``steps`` rollout steps of every environment of ``env`` (a ``BatchedWRSN``) under ``controller``.
 
     Returns the observation tensor and job-wide statistics (summed over ranks when torch.distributed is initialised:
     the only collective of the whole path): decisions handed out, simulated seconds, episodes finished, sum of rewards.
+    A controller with ``heuristic`` (``HeuristicController``) decides from the state record: its steps render no observation,
+    and ``obs`` is filled once, after the last step.
     """
     B, S, dev = env.B, env.S, env.device
+    heuristic = getattr(controller, "heuristic", None)
     if obs is None:
         obs = torch.zeros((B, 4, S, S), dtype=torch.float32, device=dev)
-        env.get_state(out=obs)
+        if heuristic is None:
+            env.get_state(out=obs)
     action = torch.zeros((B, 3), dtype=torch.float64, device=dev)
     local = torch.zeros(2, dtype=torch.float64, device=dev)               # episodes finished, sum of rewards
     resets0 = env.req.stats[:, 2].sum()
     dec0, sim0 = reduce_stats(env, group)
     fused = getattr(controller, "weights", None) is not None and obs.dtype == torch.float32
     for _ in range(int(steps)):
+        if heuristic is not None:                                         # action straight from the state record
+            env.heuristic_action(heuristic, out=action)
+            env.rollout_step(action)
+            local[1] += torch.nan_to_num(env.req.reward, nan=0.0).sum()
+            continue
         if fused:                                                         # map formed inside the decoder, channel by channel
             env.linear_controller_action(obs, controller.weights, out=action)
             env.rollout_step(action, obs)
@@ -54,6 +84,8 @@ def rollout(env, controller, steps, obs=None, group=None):
             action.copy_(a)
         env.rollout_step(action, obs)
         local[1] += torch.nan_to_num(env.req.reward, nan=0.0).sum()
+    if heuristic is not None:
+        env.get_state(out=obs)
     local[0] = env.req.stats[:, 2].sum() - resets0                        # episodes that ended (and were reset) in these steps
     if torch.distributed.is_available() and torch.distributed.is_initialized() and torch.distributed.get_world_size(group) > 1:
         torch.distributed.all_reduce(local, group=group)
@@ -61,6 +93,85 @@ def rollout(env, controller, steps, obs=None, group=None):
     all_dead = env.raise_on_error()                                       # engine errors of any step of the window, reset or not
     return obs, dict(decisions=dec1 - dec0, simulated_seconds=sim1 - sim0, episodes=float(local[0].item()),
                      reward_sum=float(local[1].item()), environments_that_saw_every_charger_dead=all_dead)
+
+
+def evaluate(env, controller, episodes=1, max_decisions=None, check_every=16):
+    """Run every environment of ``env`` (a ``BatchedWRSN``) from a reset under ``controller`` until it has finished
+    ``episodes`` episodes, and report each one: the network lifetime and the return of a policy, as the papers compare them.
+
+    An episode ends at a request that names no charger (``agent_id == -1``: the network is dead, ``terminal``, or every
+    charger is), or — with ``max_decisions`` — at the first request after that many decisions (``truncated``).  Each row is
+    stepped with ``step(mask=running)``, so its terminal request is read before ``reset(mask=finished)`` starts the next
+    episode.  A request with no deciding charger that is not terminal (``agent_id == -2``) is stepped with agent -1; a step in
+    flight (-4) continues.  The decision comes from ``heuristic`` (``HeuristicController``) when the controller has one;
+    otherwise from ``make_action(agent_id, obs)`` on the float32 observation (``get_state`` into one reused buffer), its maps
+    decoded by ``density_map_to_action``, or by ``linear_controller_action`` when the controller has ``weights``.  A
+    ``make_action`` that returns ``(action, log_prob)`` (a ``PerAgentPolicy``) is accepted.  The loop synchronises with the
+    host once every ``check_every`` steps, to see whether any row is still running.
+
+    Returns tensors [B, episodes] on the device: ``lifetime`` (``now`` at the episode's last request minus
+    ``warm_up_time``), ``return`` (sum of the rewards of its requests, NaN counted as 0), ``decisions`` (actions handed to
+    ``step``) and ``truncated``.
+    """
+    B, dev, E = env.B, env.device, int(episodes)
+    if E < 1 or int(check_every) < 1:
+        raise ValueError("episodes and check_every must be at least 1")
+    cap = None if max_decisions is None else int(max_decisions)
+    heuristic = getattr(controller, "heuristic", None)
+    weights = getattr(controller, "weights", None)
+    obs = None if heuristic is not None else torch.zeros((B, 4, env.S, env.S), dtype=torch.float32, device=dev)
+    lifetime = torch.zeros((B, E), dtype=torch.float64, device=dev)
+    ret = torch.zeros((B, E), dtype=torch.float64, device=dev)
+    decisions = torch.zeros((B, E), dtype=torch.int64, device=dev)
+    truncated = torch.zeros((B, E), dtype=torch.bool, device=dev)
+    done = torch.zeros(B, dtype=torch.int64, device=dev)                 # episodes finished per row
+    cur_ret = torch.zeros(B, dtype=torch.float64, device=dev)
+    cur_dec = torch.zeros(B, dtype=torch.int64, device=dev)
+    action = torch.zeros((B, 3), dtype=torch.float64, device=dev)
+    cols = torch.arange(E, device=dev)
+    env.reset()
+    k = 0
+    while True:
+        req = env.req
+        running = done < E
+        fin_term = running & (req.agent_id == -1)
+        fin = fin_term
+        if cap is not None:
+            fin = fin | (running & (req.agent_id != -1) & (req.agent_id != -4) & (cur_dec >= cap))
+        hit = fin[:, None] & (cols[None, :] == done[:, None])            # this episode's column
+        lifetime.copy_(torch.where(hit, (req.now - env.warm_up_time)[:, None], lifetime))
+        ret.copy_(torch.where(hit, cur_ret[:, None], ret))
+        decisions.copy_(torch.where(hit, cur_dec[:, None], decisions))
+        truncated.copy_(truncated | (hit & ~fin_term[:, None]))
+        done += fin.to(torch.int64)
+        cur_ret.masked_fill_(fin, 0.0)
+        cur_dec.masked_fill_(fin, 0)
+        running = done < E
+        env.reset(mask=fin & running)
+        if k % int(check_every) == 0 and not bool(running.any()):      # the loop's only host synchronisation
+            break
+        k += 1
+        aid = req.agent_id
+        if heuristic is not None:
+            env.heuristic_action(heuristic, out=action)
+        else:
+            env.get_state(out=obs)
+            if weights is not None:
+                env.linear_controller_action(obs, weights, out=action)
+            else:
+                a = controller.make_action(aid, obs)
+                if isinstance(a, tuple):
+                    a = a[0]
+                if a.dim() == 3:
+                    env.density_map_to_action(a.contiguous(), out=action)
+                else:
+                    action.copy_(a)
+        decided = running & (aid >= 0)
+        env.step(torch.where(aid >= 0, aid, torch.full_like(aid, -1)), action, mask=running)
+        cur_dec += decided.to(torch.int64)
+        cur_ret += torch.where(running, torch.nan_to_num(req.reward, nan=0.0), torch.zeros_like(cur_ret))
+    env.raise_on_error()
+    return {"lifetime": lifetime, "return": ret, "decisions": decisions, "truncated": truncated}
 
 
 class IPPORollout:

@@ -1,13 +1,15 @@
 /*
  * wrsn_abi_aux.h — the entry points of the C ABI (include/wrsn_b200.h) outside the environment kernel: the observation raster,
- * the density-map decoder, the charging model and the raster's scenario tables.  The CUDA library (wrsn_kernels.cu) and the
+ * the density-map decoder, the charging model, the heuristic charging rules and the raster's scenario tables.  The CUDA library (wrsn_kernels.cu) and the
  * tests' host emulation (tests/emu/wrsn_emu.cpp) share their argument checks and KParams; included once, after
  * wrsn_abi_host.h, and the including file supplies the work on checked arguments:
  *   launch_obs_tables(P, stream)                                  wrsn_build_obs_tables;
  *   launch_observe(P, agent_id, obs, obs_f64, stream)             wrsn_observe;
  *   launch_decode(P, agent_id, dmap, dmap_f64, channels, weights, action_out, stream)
  *                                                                 both decode entry points (channels = 0: dmap is the map);
- *   launch_charge(P, charging, node_rate, mc_rate, stream)        wrsn_k_charge.
+ *   launch_charge(P, charging, node_rate, mc_rate, stream)        wrsn_k_charge;
+ *   launch_heuristic(P, agent_id, kind, action, stream)           wrsn_heuristic_action (the CUDA library only: the host
+ *                                                                 emulation's row-by-row loop is defined below).
  */
 #pragma once
 #include "wrsn_abi_host.h"
@@ -17,8 +19,35 @@ static int launch_observe(KParams &P, const int32_t *agent_id, void *obs, int ob
 static int launch_decode(KParams &P, const int32_t *agent_id, const void *dmap, int dmap_f64, int channels, const float *weights,
                          double *action_out, void *stream);
 static int launch_charge(KParams &P, const uint8_t *charging, double *node_rate, double *mc_rate, void *stream);
+static int launch_heuristic(KParams &P, const int32_t *agent_id, int kind, double *action, void *stream);
 
 /* once the arguments are checked: the dims and the layout they imply */
+#if defined(WRSN_HOST_EMU)
+/* the host emulation's wrsn_heuristic_action: k_heuristic's rule (wrsn_layout.h: heur_key, heur_action) row by row and node by
+ * node; the minimum of a total order on (key, id) does not depend on the order in which the nodes are seen */
+static int launch_heuristic(KParams &P, const int32_t *agent_id, int kind, double *action, void *) {
+    for (int b = 0; b < P.d.B; b++) {
+        const int a = agent_id[b];
+        if (a < 0 || a >= P.d.M) continue;
+        const WrsnRow rw(P.L, P.state, P.scen, P.scen_id, b);
+        HeurFleet f = HeurFleet();
+        f.M = P.d.M;
+        for (int j = 0; j < f.M; j++) heur_charger(rw, a, j, &f);
+        int pick = -1;
+        for (int pass = 0; pass < 2 && pick < 0; pass++) {
+            HeurPick p;
+            for (int i = 0; i < rw.N; i++) {
+                double key[2] = {0.0, 0.0};
+                p.add(heur_key(rw, f, kind, i, pass, key), key, i);
+            }
+            pick = p.choice();
+        }
+        heur_action(rw, a, pick, action + 3 * (size_t)b);
+    }
+    return 0;
+}
+#endif
+
 static KParams aux_params(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state) {
     KParams P = base_params(d, scen, scen_id, const_cast<void *>(state), nullptr);
     wrsn_make_layout(&P.d, &P.L);
@@ -69,6 +98,15 @@ int wrsn_k_charge(const wrsn_dims *d, const void *scen, const int32_t *scen_id, 
     if (d->M <= 0) WRSN_FAIL("no chargers");
     KParams P = aux_params(d, scen, scen_id, state);
     return launch_charge(P, charging, node_rate, mc_rate, stream);
+}
+
+int wrsn_heuristic_action(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
+                          const int32_t *agent_id, int kind, double *action, void *stream) {
+    if (check_dims(d)) return -1;
+    if (!agent_id || !action || !scen || !scen_id || !state) WRSN_FAIL("NULL argument");
+    if (kind < 0 || kind >= WRSN_HEUR_COUNT) WRSN_FAIL("heuristic kind %d: 0 (min_lifetime) or 1 (nearest_urgent)", kind);
+    KParams P = aux_params(d, scen, scen_id, state);
+    return launch_heuristic(P, agent_id, kind, action, stream);
 }
 
 }  /* extern "C" */

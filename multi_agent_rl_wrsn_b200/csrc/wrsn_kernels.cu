@@ -739,6 +739,45 @@ __global__ void __launch_bounds__(32 * CHG_WARPS) k_charge(const KParams P, cons
     for (int m = lane; m < M; m += 32) mc_rate[(size_t)b * M + m] = s_sum[wrp][m];
 }
 
+/* the hand-written charging rules (include/wrsn_b200.h: wrsn_heuristic_action; the rule itself: wrsn_layout.h, heur_key /
+ * heur_action): one warp per row.  The chargers are read once into shared memory; lanes stride the row's nodes, each keeps the
+ * smallest (key, id) of the candidates and of the urgent ones, and the warp reduces them by shuffles.  Every comparison is a
+ * total order on (key, id), so the result does not depend on how the nodes fall on the lanes.  Pass 1 (every alive node is a
+ * candidate) runs only when pass 0 found none.  3 CTAs per SM: at 4 ptxas caps the kernel at 64 registers and spills. */
+#define HEUR_WARPS 8
+__global__ void __launch_bounds__(32 * HEUR_WARPS, 3) k_heuristic(const KParams P, const int32_t *__restrict__ agent_id, int kind,
+                                                               double *__restrict__ action) {
+    __shared__ HeurFleet s_fleet[HEUR_WARPS];
+    const int wrp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int b = blockIdx.x * HEUR_WARPS + wrp;
+    if (b >= P.d.B) return;                                   /* whole warps leave together; only __syncwarp below */
+    const int a = agent_id[b];
+    if (a < 0 || a >= P.d.M) return;
+    const WrsnRow rw(P.L, P.state, P.scen, P.scen_id, b);
+    HeurFleet &f = s_fleet[wrp];
+    if (lane < P.d.M) heur_charger(rw, a, lane, &f);          /* M <= WRSN_MAX_MC = 16 */
+    if (lane == 0) f.M = P.d.M;
+    __syncwarp();
+    int pick = -1;
+    for (int pass = 0; pass < 2 && pick < 0; pass++) {        /* pick is warp-uniform after the butterfly */
+        HeurPick p;
+        for (int i = lane; i < rw.N; i += 32) {
+            double key[2] = {0.0, 0.0};
+            p.add(heur_key(rw, f, kind, i, pass, key), key, i);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+            for (int s = 0; s < 2; s++) {
+                const double k = __shfl_xor_sync(0xffffffffu, p.k[s], o);
+                const int id = __shfl_xor_sync(0xffffffffu, p.i[s], o);
+                p.take(s, k, id);
+            }
+        pick = p.choice();
+    }
+    if (lane == 0) heur_action(rw, a, pick, action + 3 * (size_t)b);
+}
+
 /* roll_out bookkeeping (IPPO.py:138-155): one thread per environment, see include/wrsn_b200.h */
 __global__ void k_record_transitions(int B, int M, wrsn_request req, int64_t t, const int64_t *__restrict__ agent_prev,
                                      int64_t *__restrict__ last, double *__restrict__ resets_seen,
@@ -902,6 +941,12 @@ static int launch_decode(KParams &P, const int32_t *agent_id, const void *dmap, 
 
 static int launch_charge(KParams &P, const uint8_t *charging, double *node_rate, double *mc_rate, void *stream) {
     k_charge<<<(P.d.B + CHG_WARPS - 1) / CHG_WARPS, 32 * CHG_WARPS, 0, (cudaStream_t)stream>>>(P, charging, node_rate, mc_rate);
+    WRSN_CUDA(cudaGetLastError());
+    return 0;
+}
+
+static int launch_heuristic(KParams &P, const int32_t *agent_id, int kind, double *action, void *stream) {
+    k_heuristic<<<(P.d.B + HEUR_WARPS - 1) / HEUR_WARPS, 32 * HEUR_WARPS, 0, (cudaStream_t)stream>>>(P, agent_id, kind, action);
     WRSN_CUDA(cudaGetLastError());
     return 0;
 }

@@ -193,6 +193,75 @@ WRSN_HD int32_t wrsn_obs_pitch(int S) {
     return pi > pj ? pi : pj;
 }
 
+/* ------------------------------------------------------------------ the hand-written charging rules (include/wrsn_b200.h:
+ * wrsn_heuristic_action).  k_heuristic and the host emulation state the rule only through these functions. */
+#define HEUR_NONE 0x7fffffff                        /* id of an empty set's best: sorts after every node */
+
+struct HeurFleet {                                  /* what the rule reads of a row's chargers, once per row */
+    double ax, ay;                                  /* the deciding charger's position */
+    double dx[WRSN_MAX_MC], dy[WRSN_MAX_MC];        /* every charger's destination (cur_phy_action) */
+    uint8_t on[WRSN_MAX_MC];                        /* 1: charger j can claim a node (alive, not the deciding one) */
+    int M;
+};
+
+WRSN_HD void heur_charger(const WrsnRow &rw, int a, int j, HeurFleet *f) {
+    const double *m = rw.mc + (size_t)j * WRSN_MC_LEN;
+    f->dx[j] = m[WRSN_MC_CPA0]; f->dy[j] = m[WRSN_MC_CPA1];
+    f->on[j] = (j != a && m[WRSN_MC_STATUS] != 0.0) ? 1 : 0;
+    if (j == a) { f->ax = m[WRSN_MC_X]; f->ay = m[WRSN_MC_Y]; }
+}
+
+/* euclid2's arithmetic (wrsn_engine.cuh): both builds compile without contraction, so products and sum round separately */
+WRSN_HD double heur_dist(double ax, double ay, double bx, double by) {
+    const double dx = ax - bx, dy = ay - by;
+    return sqrt(dx * dx + dy * dy);
+}
+
+/* Node i under the rule.  pass 0: claimed nodes are not candidates; pass 1 (when pass 0 has none): every alive node is.
+ * Returns 0 when i is not a candidate, 1 when it is, 2 when it is also urgent under WRSN_HEUR_NEAREST_URGENT.
+ * key[0]: the lifetime (min_lifetime's key, nearest_urgent's fallback); key[1] (urgent nodes): the distance from charger a. */
+WRSN_HD int heur_key(const WrsnRow &rw, const HeurFleet &f, int kind, int i, int pass, double key[2]) {
+    if (rw.status[i] != 1) return 0;
+    const double *par = rw.par;
+    const double x = rw.nx[i], y = rw.ny[i];
+    if (pass == 0)
+        for (int j = 0; j < f.M; j++)
+            if (f.on[j] && heur_dist(x, y, f.dx[j], f.dy[j]) <= par[WRSN_P_MC_R]) return 0;
+    const double cs = rw.cs[i];
+    key[0] = cs <= 0.0 ? (double)INFINITY : (rw.energy[i] - par[WRSN_P_THR]) / cs;   /* no traffic: never needs a charger */
+    if (kind == WRSN_HEUR_NEAREST_URGENT && key[0] < par[WRSN_P_MTM] + par[WRSN_P_CTM]) {
+        key[1] = heur_dist(f.ax, f.ay, x, y);
+        return 2;
+    }
+    return 1;
+}
+
+/* the smallest (key, id) of the candidates (k[0], i[0]) and of the urgent ones (k[1], i[1]) seen so far */
+struct HeurPick {
+    double k[2]; int i[2];
+    WRSN_HDM HeurPick() { k[0] = k[1] = (double)INFINITY; i[0] = i[1] = HEUR_NONE; }
+    WRSN_HDM void take(int s, double key, int id) {
+        if (key < k[s] || (key == k[s] && id < i[s])) { k[s] = key; i[s] = id; }
+    }
+    WRSN_HDM void add(int cls, const double key[2], int id) {
+        if (cls) take(0, key[0], id);
+        if (cls == 2) take(1, key[1], id);
+    }
+    WRSN_HDM int choice() const { return i[1] != HEUR_NONE ? i[1] : (i[0] != HEUR_NONE ? i[0] : -1); }
+};
+
+/* the action of charger a for node i (i < 0: no alive node, charger a stays where it is) */
+WRSN_HD void heur_action(const WrsnRow &rw, int a, int i, double *out) {
+    const double *par = rw.par, *m = rw.mc + (size_t)a * WRSN_MC_LEN;
+    const double W = par[WRSN_P_F1] - par[WRSN_P_F0], H = par[WRSN_P_F3] - par[WRSN_P_F2];
+    const double x = i >= 0 ? rw.nx[i] : m[WRSN_MC_X], y = i >= 0 ? rw.ny[i] : m[WRSN_MC_Y];
+    out[0] = W == 0.0 ? 0.0 : (x - par[WRSN_P_F0]) / W;
+    out[1] = H == 0.0 ? 0.0 : (y - par[WRSN_P_F2]) / H;
+    double c = 0.0;                                 /* time to refill at the peak rate alpha / beta^2, over charging_time_max */
+    if (i >= 0) { c = (par[WRSN_P_CAP] - rw.energy[i]) / par[WRSN_P_CAPMTHR]; c = c > 1.0 ? 1.0 : (c > 0.0 ? c : 0.0); }
+    out[2] = c;
+}
+
 /* request record of one environment, as the engine's entry points produce it */
 struct ReqOut { int agent; int terminal; double reward, now, act[3], detail[2]; int flags; };
 

@@ -188,6 +188,12 @@ class WRSN:
         aid = torch.tensor([int(id)], dtype=torch.int32, device=self._b.device)
         return self._b.density_map_to_action(dm, agent_id=aid)[0].cpu().numpy()
 
+    def heuristic_action(self, agent_id, kind="min_lifetime"):
+        """The hand-written charging decision of charger ``agent_id`` (``BatchedWRSN.heuristic_action``) -> the 3-vector
+        action, for ``step`` of an environment built with ``density_map=False``."""
+        aid = torch.tensor([int(agent_id)], dtype=torch.int32, device=self._b.device)
+        return self._b.heuristic_action(kind, agent_id=aid)[0].cpu().numpy()
+
     def _host(self, name):
         """Typed view of ONE host copy of the environment's record, fetched once per request (invalidated by reset / step)."""
         if self._row is None:
