@@ -114,12 +114,14 @@ def check_episode(name, device, check_obs=False, replicas=1):
 
 
 def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=None, check_obs=False, scale2=0.05,
-                    map_size=100, scenario_index=None, controller=False, obs32=False, threads=0, rounds=0):
+                    map_size=100, scenario_index=None, controller=False, obs32=False, threads=0, rounds=0, probe=None):
     """B environments with DIFFERENT action streams (and possibly different scenarios) vs B oracle runs (ladder L6).
     ``controller``: the actions are those of the reference's RandomController — the density map s0 + s1 - 10 s2 + s3 of the
     float32 observation, decoded ON THE DEVICE (wrsn_decode_density_map) — and the oracle is fed the decoded 3-vectors, so
     the simulation is compared on the trajectory the device controller drives (the decoder itself: tests/test_decode.py).
-    ``obs32``: also the float32 raster against the oracle's state at 1e-5 of the channel maximum."""
+    ``obs32``: also the float32 raster against the oracle's state at 1e-5 of the channel maximum.
+    ``probe(env, rows)``: called at every request with the boolean mask of the rows compared there (e.g. to count the
+    requests that reached a regime the test is about)."""
     if isinstance(scenarios, Scenario):
         scenarios = [scenarios]
     env = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, map_size=map_size,
@@ -159,6 +161,8 @@ def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=No
                 n_dec += 1
                 if k > 0:
                     np.testing.assert_allclose(float(_np(req.reward)[b]), r["reward"], rtol=1e-9, atol=1e-18)
+        if probe is not None:
+            probe(env, live.copy())
         if check_obs:
             obs = _np(env.get_state(dtype=torch.float64))
             for b in range(B):
@@ -194,10 +198,10 @@ def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=No
     return n_dec, env.counters()
 
 
-def check_network_after_operate_stopped(scenario, device, horizon, every=50.0):
+def check_network_after_operate_stopped(scenario, device, horizon, every=50.0, threads=0):
     """Nodes keep running after Network.operate has finished (alive == 0): levels stay stale, later deaths re-route
     through the stale levels (Node.find_receiver) — engine vs oracle far past the end of Network.operate."""
-    env = BatchedWRSN(scenario, num_agent=0, num_envs=1, device=device)
+    env = BatchedWRSN(scenario, num_agent=0, num_envs=1, device=device, threads=threads)
     env.init_network(with_reward_process=False)
     o = OracleWRSN(scenario_from_dict(scenario.to_dict()), num_agent=0)
     o.start_network_only()
@@ -275,14 +279,16 @@ def _state_diff_but_switch(a, b):
     return "padding bytes differ"
 
 
-def check_batches_equal_event_path(scenarios, device, num_envs, steps, seed, num_agent=3, scale2=0.3, threads=0):
+def check_batches_equal_event_path(scenarios, device, num_envs, steps, seed, num_agent=3, scale2=0.3, threads=0, mc=None,
+                                   probe=None):
     """Whole-cycle batches (nodes_batch) leave EVERY byte of the environment record — node rows, event clock with its
-    insertion counters, charger records — exactly as the event-by-event path does, over several episodes."""
+    insertion counters, charger records — exactly as the event-by-event path does, over several episodes.  ``probe(env)``:
+    called with the batched simulator after every step."""
     rng = np.random.default_rng(seed)
     acts = rng.uniform(0.0, 1.0, size=(steps, num_envs, 3))
     acts[..., 2] *= scale2
-    a = BatchedWRSN(scenarios, num_agent=num_agent, num_envs=num_envs, device=device, threads=threads)
-    b = BatchedWRSN(scenarios, num_agent=num_agent, num_envs=num_envs, device=device, threads=threads)
+    a = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, threads=threads)
+    b = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, threads=threads)
     _disable_batches(b)
     a.reset(); b.reset()
     ends = 0
@@ -295,6 +301,8 @@ def check_batches_equal_event_path(scenarios, device, num_envs, steps, seed, num
         assert np.array_equal(_np(a.req.reward), _np(b.req.reward), equal_nan=True), k
         diff = _state_diff_but_switch(a, b)
         assert not diff, (k, diff)
+        if probe is not None:
+            probe(a)
     ca, cb = a.counters(), b.counters()
     # (the warm-up snapshot of `b` was simulated before the switch was set: its counter is not zero)
     assert ca["batched_ticks"] > cb["batched_ticks"] and ca["ticks"] == cb["ticks"] and ca["events"] == cb["events"]
@@ -454,12 +462,13 @@ def check_ippo_rollout(scenarios, device, num_envs, steps, gamma=0.99, lam=0.95,
     return n_tr, episodes
 
 
-def check_charge_kernel(scenarios, device, num_envs, steps, seed, num_agent=3):
+def check_charge_kernel(scenarios, device, num_envs, steps, seed, num_agent=3, mc=None, probe=None):
     """wrsn_k_charge (dense node x charger charging model, one warp per environment) == the reference's statements
     (oracle.wrsn_oracle.charge_rates_reference), bit for bit, on states reached by a rollout whose actions send the chargers to
-    node positions (several nodes within range), with all chargers and with a random subset selected."""
+    node positions (several nodes within range), with all chargers and with a random subset selected.  ``probe(env)``: called
+    at every step whose rates are checked."""
     from oracle.wrsn_oracle import charge_rates_reference
-    env = BatchedWRSN(scenarios, num_agent=num_agent, num_envs=num_envs, device=device)
+    env = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device)
     sid = _np(env.scen_id)
     rng = np.random.default_rng(seed)
     env.reset()
@@ -477,6 +486,8 @@ def check_charge_kernel(scenarios, device, num_envs, steps, seed, num_agent=3):
         env.rollout_step(torch.as_tensor(act, device=env.device))
         if k % 3:
             continue
+        if probe is not None:
+            probe(env)
         for sel in (None, rng.integers(0, 2, size=(num_envs, num_agent)).astype(np.uint8)):
             node_rate, mc_rate = env.charge_rates(None if sel is None else torch.as_tensor(sel, device=env.device))
             node_rate, mc_rate = _np(node_rate), _np(mc_rate)
@@ -499,16 +510,18 @@ def check_charge_kernel(scenarios, device, num_envs, steps, seed, num_agent=3):
     return n_pairs
 
 
-def check_budget_equals_unbudgeted(scenarios, device, num_envs, calls, seed, budget, num_agent=3, scale2=0.3, threads=0, rounds=0):
+def check_budget_equals_unbudgeted(scenarios, device, num_envs, calls, seed, budget, num_agent=3, scale2=0.3, threads=0, rounds=0,
+                                   mc=None, probe=None):
     """A step budget (wrsn_dims.step_budget) only cuts a WRSN.step into several launches: every request an environment hands
     out — agent, time, reward, termination, clipped action — and every byte of its record at that moment are those of the
-    unbudgeted run answered with the same actions.  Returns how many interrupted launches it took."""
+    unbudgeted run answered with the same actions.  Returns how many interrupted launches it took.  ``probe(env)``: called with
+    the unbudgeted simulator after every step."""
     rng = np.random.default_rng(seed)
     acts = rng.uniform(0.0, 1.0, size=(calls, num_envs, 3))
     acts[..., 2] *= scale2
-    a = BatchedWRSN(scenarios, num_agent=num_agent, num_envs=num_envs, device=device, threads=threads)
-    b = BatchedWRSN(scenarios, num_agent=num_agent, num_envs=num_envs, device=device, threads=threads, step_budget=budget,
-                    step_rounds=rounds)
+    a = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, threads=threads)
+    b = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, threads=threads,
+                    step_budget=budget, step_rounds=rounds)
     end = int(a._foff[a.E["WRSN_F_SCRATCH"]])            # the engine's scratch field (last in the record) is not state
     hdr0 = int(a._foff[a.E["WRSN_F_HDR"]])
     skip = [hdr0 + 8 * a.E["WRSN_H_" + f] for f in ("NRESUME", "NBATCH")]   # (a split step may run a short batch event by event)
@@ -526,6 +539,8 @@ def check_budget_equals_unbudgeted(scenarios, device, num_envs, calls, seed, bud
         a.rollout_step(torch.as_tensor(acts[k], device=a.device))
         rec.append(({f: _np(getattr(a.req, f)) for f in fields}, rows(a)))
         assert not bool((a.req.agent_id == -4).any())
+        if probe is not None:
+            probe(a)
     count = np.zeros(num_envs, np.int64)
     interrupted = launches = 0
     while int(count.min()) < calls and launches < 400 * calls:
