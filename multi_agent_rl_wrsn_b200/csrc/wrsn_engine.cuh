@@ -407,7 +407,8 @@ WRSN_D double div_pos(double num, double den) { return num == 0.0 ? num : num / 
  * that is part of the simulated state (energies, energyCS, charger records) goes through these. */
 #if !defined(WRSN_HOST_EMU)
 WRSN_D double wrsn_fma(double a, double b, double c) { return __fma_rn(a, b, c); }
-WRSN_D double wrsn_rcp(double d) {                  /* 1 / d, d > 0 normal: <= 2 ulp */
+WRSN_D double wrsn_rcp(double d) {                  /* 1 / d, d > 0 with d and 1 / d normal (d <= 2^1022): <= 2 ulp;
+                                                        the seed flushes a subnormal 1 / d to zero */
     double r;
     asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r) : "d"(d));
     double e = __fma_rn(-d, r, 1.0);
@@ -461,8 +462,10 @@ WRSN_NOINLINE double euclid2(double ax, double ay, double bx, double by) {
  * n_single times (e -= a) followed by n_pair times (e -= b; e -= a), evaluated sequentially in fp64 by the
  * reference.  Inside one binade [2^k, 2^(k+1)) every representable value is a multiple of u = 2^(k-52), so
  * "e - x" rounds to e - rint(x/u)*u (ties aside): each step removes a fixed integer number of ulps and the
- * whole chain is one exact integer multiply.  If the chain would leave the binade (or x/u is an exact tie)
- * the literal loop runs instead.  Order of the steps does not matter inside the binade. */
+ * whole chain is one exact integer multiply.  The result must lie strictly above 2^k: a chain that ends exactly on
+ * 2^k has a last step whose exact value may fall below 2^k, where the spacing is u/2, and round to 2^k - u/2.  If the
+ * chain would reach 2^k or leave the binade (or x/u is an exact tie) the literal loop runs instead.  Order of the
+ * steps does not matter while the result stays above 2^k. */
 WRSN_D double wrsn_pow2_biased(int biased) {       /* 2^(biased - 1023) for 1 <= biased <= 2046 */
     uint64_t b = (uint64_t)biased << 52;
 #if !defined(WRSN_HOST_EMU)
@@ -483,7 +486,7 @@ WRSN_NOINLINE double sub_chain_literal(double e, double a, int n_single, double 
     for (int k = 0; k < n_pair; k++) { e -= b; e -= a; }
     return e;
 }
-/* the closed form alone: NaN when the chain would leave the binade, has an exact tie, or e is out of range */
+/* the closed form alone: NaN when the chain would reach 2^k or leave the binade, has an exact tie, or e is out of range */
 WRSN_D double sub_chain_fast(double e, double a, int n_single, double b, int n_pair) {
     int n_a = n_single + n_pair;
     if (n_a == 0) return e;
@@ -497,7 +500,7 @@ WRSN_D double sub_chain_fast(double e, double a, int n_single, double b, int n_p
         double total = ra * (double)n_a + rb * (double)n_pair;
         if (!tie && total < 4503599627370496.0) {
             double r = e - total * u;
-            if (r >= lo) return r;
+            if (r > lo) return r;
         }
     }
     return NAN;
@@ -515,7 +518,7 @@ WRSN_D double sub_chain(double e, double a, int n_single, double b, int n_pair) 
         double total = ra * (double)n_a + rb * (double)n_pair;
         if (!tie && total < 4503599627370496.0) {    /* < 2^52 ulps: products and sum are exact integers */
             double r = e - total * u;
-            if (r >= lo) return r;
+            if (r > lo) return r;
         }
     }
     return sub_chain_literal(e, a, n_single, b, n_pair);
@@ -976,7 +979,7 @@ WRSN_D void ev_nodes_drain(Ctx &c) {
         double e3 = NAN;
         if (rr == 0.0) {
             /* no top-up in between: the two chains are one multiset of subtractions; inside a binade their order does not
-               matter (sub_chain), so one closed form serves both — NaN when it would leave the binade */
+               matter (sub_chain), so one closed form serves both — NaN when it would reach the binade's floor or leave it */
             e3 = sub_chain_fast(e, es, ow, er, nb + na);
             if (e3 == e3 && nb + ow + na > 0 && !(e3 - thr >= slack)) slow = 1;   /* e1 >= e3: the first check is implied */
         }
@@ -1112,16 +1115,14 @@ WRSN_D double nan_with_payload(int slot) {
 #endif
 }
 
-/* table entry of node i at energy e (reward_loop / spec_second): inside e's binade the chain of relayed packets of lower
+/* the table entry's arithmetic for a node at energy e: inside e's binade [lo, 2 lo) the chain of relayed packets of lower
  * ids, the own packets + relays of higher ids and the top-up  min(e + energyRR * 0.5, cap)  move e by D1, D2 and H — whole
- * numbers of ulps — as long as e stays between the guards for the whole second (both top-ups, both chains) */
-WRSN_NOINLINE void spec_entry(Ctx &c, int i, int slot, double e) {
-    double *sp = c.spec + slot * WRSN_SPEC_LEN;
-    const double es = c.esend[i], er = c.par[WRSN_P_ERECV], rr = c.rr[i];
-    const int nb = c.nbef[i], na = c.naft[i];
-    const int ow = c.parent[i] != -1 ? (int)c.own[i] : 0;
+ * numbers of ulps — as long as glo <= e <= ghi at the start of the second (both top-ups, both chains).  glo keeps one ulp
+ * above lo + D1 + D2: a chain that ends exactly on lo may round to lo - u/2 (see sub_chain).  No closed form: glo = +inf. */
+struct SpecTerms { double D1, D2, H, glo, ghi; };
+WRSN_DI SpecTerms spec_terms(double e, double es, double er, double rr, int nb, int ow, int na) {
     const int n_a = nb + ow + na, n_b = nb + na;
-    double D1 = 0.0, D2 = 0.0, H = 0.0, glo = INFINITY, ghi = -INFINITY;
+    SpecTerms s = {0.0, 0.0, 0.0, INFINITY, -INFINITY};
     const int ex = wrsn_biased_exp(e);
     if (e > 0.0 && ex > 60 && ex < 1900) {
         const double lo = wrsn_pow2_biased(ex), inv_u = wrsn_pow2_biased(2098 - ex), u = wrsn_pow2_biased(ex - 52);
@@ -1130,11 +1131,18 @@ WRSN_NOINLINE void spec_entry(Ctx &c, int i, int slot, double e) {
         const bool tie = (n_a > 0 && fabs(qa - ra) == 0.5) || (n_b > 0 && fabs(qb - rb) == 0.5) || fabs(qh - rh) == 0.5;
         const double K1 = (ra + rb) * (double)nb, K2 = ra * (double)(ow + na) + rb * (double)na;
         if (!tie && K1 + K2 < 1125899906842624.0 && rh < 1125899906842624.0 && rr >= 0.0) {
-            D1 = K1 * u; D2 = K2 * u; H = rh * u;
-            glo = lo + (D1 + D2); ghi = (lo + lo) - (H + H) - (u + u);
+            s.D1 = K1 * u; s.D2 = K2 * u; s.H = rh * u;
+            s.glo = lo + (s.D1 + s.D2) + u; s.ghi = (lo + lo) - (s.H + s.H) - (u + u);
         }
     }
-    sp[0] = D1; sp[1] = D2; sp[2] = H; sp[3] = glo; sp[4] = ghi; sp[5] = (double)i;
+    return s;
+}
+/* table entry of node i at energy e (reward_loop / spec_second) */
+WRSN_NOINLINE void spec_entry(Ctx &c, int i, int slot, double e) {
+    double *sp = c.spec + slot * WRSN_SPEC_LEN;
+    const int ow = c.parent[i] != -1 ? (int)c.own[i] : 0;
+    const SpecTerms s = spec_terms(e, c.esend[i], c.par[WRSN_P_ERECV], c.rr[i], c.nbef[i], ow, c.naft[i]);
+    sp[0] = s.D1; sp[1] = s.D2; sp[2] = s.H; sp[3] = s.glo; sp[4] = s.ghi; sp[5] = (double)i;
 }
 
 /* one table node, one second: [the previous second's k+1.0 top-up,] [this second's k+0.5 tick] on c.energy[i] */
@@ -2100,6 +2108,38 @@ WRSN_NOINLINE double drain_node(double e, double rr, double es, double er, int n
     return sub_chain(e2, es, ow, er, na);
 }
 
+/* the per-cycle decrement dec = K u of a node without top-up (energyRR == 0) and with traffic: inside e's binade [lo, 2 lo)
+ * every cycle removes the same K whole ulps (sub_chain).  *m_out: how many cycles may be applied as  e - dec * m  (at most
+ * n_max); the count keeps one cycle of margin above lo and above the threshold.  NaN (and *m_out = 0): replay cycle by cycle. */
+WRSN_DI double batch_dec(double e, double es, double er, int nb, int ow, int na, double thr, int n_max, int *m_out) {
+    const double slack = 1e-6;
+    const int n_a = nb + ow + na, n_b = nb + na;
+    double dec = NAN;
+    int m = 0;
+    const int ex = wrsn_biased_exp(e);
+    if (e > 0.0 && ex > 60 && ex < 1900) {
+        const double lo = wrsn_pow2_biased(ex), inv_u = wrsn_pow2_biased(2098 - ex), u = wrsn_pow2_biased(ex - 52);
+        const double qa = es * inv_u, qb = er * inv_u;
+        const double ra = rint(qa), rb = rint(qb);
+        const bool tie = (fabs(qa - ra) == 0.5) || (n_b > 0 && fabs(qb - rb) == 0.5);
+        const double K = ra * (double)n_a + rb * (double)n_b;      /* ulps per cycle */
+        if (!tie && K * (double)n_max < 4503599627370496.0) {
+            dec = K * u;
+            if (K == 0.0) m = n_max;
+            else {
+                const double room = e - fmax(lo, thr + 2.0 * slack);
+                double q = room > 0.0 ? floor(room / dec) - 1.0 : 0.0;
+                q = fmin(fmax(q, 0.0), (double)n_max);
+                m = (int)q;
+                if (m > 0) { const double r = e - dec * (double)m; if (!(r >= lo) || !(r - thr >= slack)) m = 0; }
+            }
+        }
+    }
+    if (m == 0) dec = NAN;
+    *m_out = m;
+    return dec;
+}
+
 /* `n_active_max`: cap on the cycles of a batch in which update_reward is active (the step budget's granularity);
  * returns the cycles applied, + 2^30 when they were of the active kind */
 /* KIND 0: any batch; 2: only batches of the active kind (the batch kernel: the all-at-once branch is not even compiled in) */
@@ -2107,7 +2147,6 @@ template <int KIND>
 WRSN_NOINLINE int nodes_batch(Ctx &c, int n_max, int ur_on, double t_reward, int n_active_max) {
     const int N = c.N;
     const double thr = c.par[WRSN_P_THR], cap = c.par[WRSN_P_CAP], er = c.par[WRSN_P_ERECV];
-    const double slack = 1e-6;
     const double *h = c.hdr;
     WRSN_PROF_BEGIN();
     if (h[WRSN_H_OPT_NOBATCH] == 1.0 || h[WRSN_H_BFS_DIRTY] != 0.0 || h[WRSN_H_LOG_LITERAL] != 0.0 ||
@@ -2129,28 +2168,7 @@ WRSN_NOINLINE int nodes_batch(Ctx &c, int n_max, int ur_on, double t_reward, int
         double dec = NAN;
         int m = 0;
         if (rr == 0.0 && n_a == 0) { dec = 0.0; m = n_max; }
-        else if (rr == 0.0) {
-            const int ex = wrsn_biased_exp(e);
-            if (e > 0.0 && ex > 60 && ex < 1900) {
-                const double lo = wrsn_pow2_biased(ex), inv_u = wrsn_pow2_biased(2098 - ex), u = wrsn_pow2_biased(ex - 52);
-                const double qa = es * inv_u, qb = er * inv_u;
-                const double ra = rint(qa), rb = rint(qb);
-                const bool tie = (fabs(qa - ra) == 0.5) || (n_b > 0 && fabs(qb - rb) == 0.5);
-                const double K = ra * (double)n_a + rb * (double)n_b;      /* ulps per cycle */
-                if (!tie && K * (double)n_max < 4503599627370496.0) {
-                    dec = K * u;
-                    if (K == 0.0) m = n_max;
-                    else {
-                        const double room = e - fmax(lo, thr + 2.0 * slack);
-                        double q = room > 0.0 ? floor(room / dec) - 1.0 : 0.0;
-                        q = fmin(fmax(q, 0.0), (double)n_max);
-                        m = (int)q;
-                        if (m > 0) { const double r = e - dec * (double)m; if (!(r >= lo) || !(r - thr >= slack)) m = 0; }
-                    }
-                }
-            }
-            if (m == 0) dec = NAN;
-        }
+        else if (rr == 0.0) dec = batch_dec(e, es, er, nb, ow, na, thr, n_max, &m);
         if (dec != dec) {                            /* charged, near a binade edge or near the threshold: literal cycles */
             /* without any charging the node loses at most `cons` per cycle (plus a few ulps of rounding); if that cannot
                bring it within a joule of the threshold, no cycle of the batch can take the serial path because of it */

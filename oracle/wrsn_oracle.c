@@ -919,3 +919,5 @@ int orc_get_static(Oracle *o, int *nbr_ptr, int *nbr_idx, int *tgt_ptr, int *tgt
     if (direct) memcpy(direct, o->direct, sizeof(int) * o->N);
     return o->nbr_ptr[o->N];
 }
+/* test-only: overwrite node i's energy (the tests place energies on binade edges in both simulators) */
+void orc_set_node_energy(Oracle *o, int i, double e) { o->energy[i] = e; }

@@ -54,6 +54,7 @@ def lib():
         L.orc_get_consts.argtypes = [C.c_void_p, dp]
         L.orc_get_static.argtypes = [C.c_void_p, ip, ip, ip, ip, ip]
         L.orc_get_static.restype = C.c_int
+        L.orc_set_node_energy.argtypes = [C.c_void_p, C.c_int, C.c_double]
         _LIB = L
     return _LIB
 
@@ -153,6 +154,10 @@ class OracleWRSN:
 
     def set_event_budget(self, n):
         self.L.orc_set_event_budget(self.h, int(n))
+
+    def set_node_energy(self, i, e):
+        """TEST INFRASTRUCTURE: overwrite node i's energy (no event, no status check)."""
+        self.L.orc_set_node_energy(self.h, int(i), float(e))
 
     # -- accessors --------------------------------------------------------------------
     @property
