@@ -267,6 +267,10 @@ static void receive_package(Oracle *o, int i) {            /* Node.py:124-132 */
     }
     check_status(o, i);
 }
+/* Node.send_package's `d ** 2` / `d ** 4` are libm pow calls in the reference (and in scenario.py's e_send table).  A literal
+   pow(d, 2.0) is folded by gcc into d * d, the correctly rounded square, which glibc's pow misses by one ulp for some d (e.g.
+   61.71026423045482): the pointer keeps the call a call. */
+static double (*volatile libm_pow)(double, double) = pow;
 static void send_package(Oracle *o, int i) {               /* Node.py:106-122 */
     double d0 = pow(o->efs / o->emp, 0.5);
     int recv;                                               /* -2 = base station, -1 = none */
@@ -275,7 +279,7 @@ static void send_package(Oracle *o, int i) {               /* Node.py:106-122 */
     if (recv != -1) {
         double d = recv == -2 ? euclid(o->nx[i], o->ny[i], o->bsx, o->bsy)
                               : euclid(o->nx[i], o->ny[i], o->nx[recv], o->ny[recv]);
-        double e_send = ((d <= d0) ? (o->et + o->efs * pow(d, 2.0)) : (o->et + o->emp * pow(d, 4.0))) * o->package_size;
+        double e_send = ((d <= d0) ? (o->et + o->efs * libm_pow(d, 2.0)) : (o->et + o->emp * libm_pow(d, 4.0))) * o->package_size;
         if (o->energy[i] - o->threshold < e_send) o->energy[i] = o->threshold;
         else {
             o->energy[i] -= e_send;

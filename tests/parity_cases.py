@@ -3,8 +3,10 @@
 Every check drives ``BatchedWRSN`` through the C ABI and compares with either the committed golden
 fixtures (outputs of the unmodified reference, see oracle/gen_golden.py) or the C oracle run on the same
 inputs.  Discrete quantities (agent ids, termination, status / level / coverage sets, event times) must be
-identical; energies are compared at 1e-9 relative (spec: 1e-5; observed: bit-exact); rewards and
-observations, which go through exp(), at 1e-9 relative / 1e-9 absolute.
+identical.  Against the fixtures energies are compared at 1e-9 relative (spec: 1e-5); against the C oracle, which runs the
+same arithmetic, every float the record and the request carry is compared bit for bit (``compare_row_with_oracle``) except
+update_reward's outputs (reward, EXCL, detail[1]: 1e-9, DESIGN §5).  Observations, which go through exp(), at 1e-9
+relative / 1e-9 absolute.
 """
 import numpy as np
 import torch
@@ -67,6 +69,7 @@ def check_episode(name, device, check_obs=False, replicas=1):
             req = env.reset()
         else:
             req = env.step(np.full(replicas, int(g["fed_agent"][i]), np.int32), np.tile(g["fed_action"][i], (replicas, 1)))
+        fm = _np(env.get_network_fitness()[1])
         for b in range(replicas):
             tag = (name, i, b)
             aid = int(_np(req.agent_id)[b])
@@ -87,7 +90,14 @@ def check_episode(name, device, check_obs=False, replicas=1):
             assert np.array_equal(_np(env.mc("STATUS"))[b].astype(np.uint8), g["mc_status"][i]), tag
             assert np.array_equal(_np(env.mc("TYPE"))[b].astype(np.uint8), g["mc_type"][i]), tag
             assert np.array_equal(_np(env.mc("NCONN"))[b].astype(np.int32), g["mc_nconn"][i]), tag
+            np.testing.assert_allclose(_np(env.mc("CPA0"))[b], g["mc_cpa"][i][:, 0], rtol=1e-12)
+            np.testing.assert_allclose(_np(env.mc("CPA1"))[b], g["mc_cpa"][i][:, 1], rtol=1e-12)
             np.testing.assert_allclose(_np(env.mc("CPA2"))[b], g["mc_cpa"][i][:, 2], rtol=1e-12)
+            want_fm = float(g["fitness_min"][i])
+            if np.isfinite(want_fm):
+                np.testing.assert_allclose(fm[b], want_fm, rtol=1e-12, err_msg=str(tag))
+            else:
+                assert fm[b] == want_fm, (tag, fm[b], want_fm)
             np.testing.assert_allclose(_np(env.mc("EXCL"))[b], g["excl"][i], rtol=1e-9, atol=1e-15)
             if aid >= 0:
                 assert np.array_equal(_np(req.action)[b], g["action"][i]), tag
@@ -107,21 +117,97 @@ def check_episode(name, device, check_obs=False, replicas=1):
                 for ch in range(4):
                     tol = 1e-5 * max(float(np.abs(ref[ch]).max()), 1e-3)
                     assert float(np.abs(obs32[0][ch] - ref[ch]).max()) <= tol, (name, i, ch)
-    fm = _np(env.get_network_fitness()[1])
-    if np.isfinite(g["fitness_min"][n - 1]):
-        np.testing.assert_allclose(fm[0], g["fitness_min"][n - 1], rtol=1e-12)
     return env.counters()
 
 
+def _ordered(a):
+    """float64 -> int64 keys whose order is the order of the values (-0.0 and +0.0 one apart): ulp distances."""
+    i = np.ascontiguousarray(a, np.float64).view(np.int64).astype(np.int64)
+    return np.where(i < 0, np.int64(-2 ** 63) - i, i)
+
+
+def assert_bits(got, want, tag, what):
+    """float64 arrays equal bit for bit (a NaN equals any NaN: the reference's ``inf - inf`` is whichever NaN the hardware makes);
+    the failure names the worst ulp distance and where it is."""
+    g = np.atleast_1d(np.ascontiguousarray(got, np.float64))
+    w = np.atleast_1d(np.ascontiguousarray(want, np.float64))
+    assert g.shape == w.shape, (tag, what, g.shape, w.shape)
+    same = (g.view(np.int64) == w.view(np.int64)) | (np.isnan(g) & np.isnan(w))
+    if not same.all():
+        bad = np.nonzero(~same)[0]
+        ulp = [abs(int(a) - int(b)) for a, b in zip(_ordered(g[bad]), _ordered(w[bad]))]
+        k = int(np.argmax(ulp))
+        raise AssertionError("%s: %s differs in %d of %d entries; worst %d ulp at [%d]: got %r, want %r"
+                             % (tag, what, len(bad), g.size, ulp[k], bad[k], float(g[bad[k]]), float(w[bad[k]])))
+
+
+_MC_BITS = ("X", "Y", "ENERGY", "CPA0", "CPA1", "CPA2")
+_MC_INTS = (("TYPE", "type"), ("NCONN", "nconn"), ("STATUS", "status"))
+
+
+def _request_views(env):
+    """One host copy of everything check_vs_oracle compares, for all rows at once."""
+    fit, fmin = env.get_network_fitness()
+    v = {f: _np(env.view(f)) for f in ("status", "level", "energy", "cs", "rr", "mc", "hdr")}
+    v["tact"], v["fit"], v["fmin"] = _np(env.targets_active()), _np(fit), _np(fmin)
+    for f in ("agent_id", "terminal", "now", "action", "reward", "detail"):
+        v["req_" + f] = _np(getattr(env.req, f))
+    return v
+
+
+def compare_row_with_oracle(env, v, b, o, r, prev_fit, k):
+    """Row b of the host copy ``v`` (``_request_views``) against oracle ``o`` at its request ``r``, on the row's own columns.
+    Exact: ids, termination, time, status / level / coverage sets, ALIVE, and bit for bit node energy / energyCS / energyRR, the
+    chargers' X / Y / ENERGY / CPA0..2 / TYPE / NCONN / STATUS, per-target fitness and its minimum, the clipped action and the
+    fitness term of the reward (detail[0] = the minimum now minus the minimum when the deciding charger was last stepped,
+    ``prev_fit``).  To 1e-9: the reward, the
+    exclusive reward EXCL and its term detail[1] (DESIGN §5: update_reward's reciprocal, table exponential and per-thread sums).
+    Returns the oracle's fitness minimum."""
+    E, tag = env.E, (b, k)
+    aid = int(r["raw_agent_id"])
+    assert int(v["req_agent_id"][b]) == aid, tag
+    assert int(v["req_terminal"][b]) == int(r["terminal"]), tag
+    assert float(v["req_now"][b]) == r["now"], tag
+    nd = o.nodes()
+    n = len(nd["energy"])
+    assert np.array_equal(v["status"][b][:n], nd["status"]), tag
+    assert np.array_equal(v["level"][b][:n].astype(np.int32), nd["level"]), tag
+    assert np.array_equal(v["tact"][b][:o.T], o.targets_active()), tag
+    assert float(v["hdr"][b][E["WRSN_H_ALIVE"]]) == float(o.alive), tag
+    for f in ("energy", "cs", "rr"):
+        assert_bits(v[f][b][:n], nd[f], tag, "node " + f)
+    m, mcs = v["mc"][b][:o.M], o.mcs()
+    want = dict(X=mcs["loc"][:, 0], Y=mcs["loc"][:, 1], ENERGY=mcs["energy"], CPA0=mcs["cpa"][:, 0], CPA1=mcs["cpa"][:, 1],
+                CPA2=mcs["cpa"][:, 2])
+    for f in _MC_BITS:
+        assert_bits(m[:, E["WRSN_MC_" + f]], want[f], tag, "charger " + f)
+    for f, g in _MC_INTS:
+        assert np.array_equal(m[:, E["WRSN_MC_" + f]].astype(np.int64), mcs[g].astype(np.int64)), (tag, f)
+    np.testing.assert_allclose(m[:, E["WRSN_MC_EXCL"]], mcs["excl"], rtol=1e-9, atol=1e-15, err_msg=str((tag, "EXCL")))
+    omin, ofit = o.fitness()
+    assert_bits(v["fit"][b][:o.T], ofit, tag, "per-target fitness")
+    assert_bits(v["fmin"][b], omin, tag, "fitness minimum")
+    if aid >= 0:
+        assert_bits(v["req_action"][b], r["action"], tag, "clipped action")
+        if k > 0:
+            np.testing.assert_allclose(float(v["req_reward"][b]), r["reward"], rtol=1e-9, atol=1e-18, err_msg=str(tag))
+            assert_bits(v["req_detail"][b][0], omin - prev_fit[aid], tag, "detail[0] (fitness term)")
+            np.testing.assert_allclose(float(v["req_detail"][b][1]), mcs["excl"][aid] / o.consts()["avg_nodes_agent"], rtol=1e-9,
+                                       atol=1e-18, err_msg=str((tag, "detail[1]")))
+    return omin
+
+
 def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=None, check_obs=False, scale2=0.05,
-                    map_size=100, scenario_index=None, controller=False, obs32=False, threads=0, rounds=0, probe=None):
-    """B environments with DIFFERENT action streams (and possibly different scenarios) vs B oracle runs (ladder L6).
+                    map_size=100, scenario_index=None, controller=False, obs32=False, threads=0, rounds=0, probe=None, spread=0.0):
+    """B environments with DIFFERENT action streams (and possibly different scenarios) vs B oracle runs (ladder L6), every
+    row at every request as ``compare_row_with_oracle`` states.
     ``controller``: the actions are those of the reference's RandomController — the density map s0 + s1 - 10 s2 + s3 of the
     float32 observation, decoded ON THE DEVICE (wrsn_decode_density_map) — and the oracle is fed the decoded 3-vectors, so
     the simulation is compared on the trajectory the device controller drives (the decoder itself: tests/test_decode.py).
     ``obs32``: also the float32 raster against the oracle's state at 1e-5 of the channel maximum.
     ``probe(env, rows)``: called at every request with the boolean mask of the rows compared there (e.g. to count the
-    requests that reached a regime the test is about)."""
+    requests that reached a regime the test is about).  ``spread``: the uniform actions are drawn from [-spread, 1 + spread]
+    (before ``scale2``), so that the clipping of WRSN.step is exercised."""
     if isinstance(scenarios, Scenario):
         scenarios = [scenarios]
     env = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, map_size=map_size,
@@ -129,7 +215,7 @@ def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=No
     sid = _np(env.scen_id)
     B = num_envs
     rng = np.random.default_rng(seed)
-    acts = rng.uniform(0.0, 1.0, size=(steps, B, 3))
+    acts = rng.uniform(-spread, 1.0 + spread, size=(steps, B, 3))       # spread > 0: some components outside [0, 1] (clipped)
     acts[..., 2] *= scale2
     oracles = [OracleWRSN(scenario_from_dict(scenarios[sid[b]].to_dict()), num_agent=num_agent, mc=mc, map_size=map_size)
                for b in range(B)]
@@ -137,30 +223,20 @@ def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=No
         o.set_event_budget(3_000_000)
     req = env.reset()
     oreq = [o.reset(want_state=check_obs or obs32) for o in oracles]
+    prev_fit = [None] * B                                            # WRSN.reset :74-78: agents_prev_fitness
+    fmin = [None] * B
     live = np.ones(B, bool)
     n_dec = 0
     for k in range(steps + 1):
         aid = _np(req.agent_id)
+        v = _request_views(env)
         for b in range(B):
             if not live[b]:
                 continue
-            r = oreq[b]
-            tag = (b, k)
-            assert int(aid[b]) == r["raw_agent_id"], tag
-            assert int(_np(req.terminal)[b]) == int(r["terminal"]), tag
-            assert float(_np(req.now)[b]) == r["now"], tag
-            nd = oracles[b].nodes()
-            assert np.array_equal(_np(env.view("status"))[b], nd["status"]), tag
-            assert np.array_equal(_np(env.view("level"))[b].astype(np.int32), nd["level"]), tag
-            assert np.array_equal(_np(env.targets_active())[b], oracles[b].targets_active()), tag
-            np.testing.assert_allclose(_np(env.view("energy"))[b], nd["energy"], rtol=E_RTOL)
-            mcs = oracles[b].mcs()
-            np.testing.assert_allclose(_np(env.mc("ENERGY"))[b], mcs["energy"], rtol=E_RTOL)
-            assert np.array_equal(_np(env.mc("STATUS"))[b].astype(np.uint8), mcs["status"]), tag
-            if r["raw_agent_id"] >= 0:
-                n_dec += 1
-                if k > 0:
-                    np.testing.assert_allclose(float(_np(req.reward)[b]), r["reward"], rtol=1e-9, atol=1e-18)
+            fmin[b] = compare_row_with_oracle(env, v, b, oracles[b], oreq[b], prev_fit[b], k)
+            if k == 0:
+                prev_fit[b] = [fmin[b]] * num_agent
+            n_dec += int(oreq[b]["raw_agent_id"] >= 0)
         if probe is not None:
             probe(env, live.copy())
         if check_obs:
@@ -193,6 +269,8 @@ def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=No
         req = env.step(np.where(live, aid, -1).astype(np.int32), act_k, mask=mask)
         for b in range(B):
             if live[b]:
+                if aid[b] >= 0:
+                    prev_fit[b][int(aid[b])] = fmin[b]                # WRSN.step :299: the fitness before the step
                 oreq[b] = oracles[b].step(int(aid[b]), act_k[b], want_state=check_obs or obs32)
     assert float(_np(env.hdr("ERR")).max()) == 0.0
     return n_dec, env.counters()
