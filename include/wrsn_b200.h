@@ -308,6 +308,21 @@ enum {
 int wrsn_heuristic_action(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
                           const int32_t *agent_id, int kind, double *action /* [B][3] */, void *stream);
 
+#define WRSN_CAND_MAX 32        /* candidates per row of wrsn_heuristic_candidates */
+/* The rule's K best candidate actions, for a planner that tries each of them (a rollout over forked rows, wrsn_copy_rows).  For
+ * every row with 0 <= a = agent_id[b] < M: the first K nodes of the candidate set of wrsn_heuristic_action, in the rule's order,
+ * which is one total order on (class, key, id):
+ *   WRSN_HEUR_MIN_LIFETIME    class 1, key L_i
+ *   WRSN_HEUR_NEAREST_URGENT  the urgent candidates (L_i < par[MTM] + par[CTM]): class 0, key d(charger a, node i);
+ *                             the others: class 1, key L_i
+ * Slot k: node[b][k] = its node id, action[b][k] = wrsn_heuristic_action's 3-vector for that node, so slot 0 is bit for bit
+ * wrsn_heuristic_action's output.  When the row has fewer than K candidates, the remaining slots hold node -1 and a copy of
+ * slot 0's action; with no alive node at all, every slot has node -1 and slot 0 is the stay action.  Other rows are left
+ * untouched.  K outside [1, WRSN_CAND_MAX] and kind outside [0, WRSN_HEUR_COUNT) are refused. */
+int wrsn_heuristic_candidates(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
+                              const int32_t *agent_id, int kind, int K, double *action /* [B][K][3] */, int32_t *node /* [B][K] */,
+                              void *stream);
+
 /* standalone per-tick kernels (the same device functions the fused step uses; unit parity + ncu evidence) */
 int wrsn_k_bfs(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream);      /* Network.setLevels + receivers + relay counts */
 int wrsn_k_drain(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream);    /* Node.operate k+0.5 tick */

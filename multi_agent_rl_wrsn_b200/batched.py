@@ -6,6 +6,7 @@ environment axis and lives in HBM as a torch tensor.  All simulation work happen
 behind the C ABI of ``include/wrsn_b200.h``; torch is the allocator and the stream provider only.
 """
 import ctypes as C
+import math
 
 import numpy as np
 import torch
@@ -46,6 +47,28 @@ class Requests:
         self.c = _lib.Request(self.agent_id.data_ptr(), self.terminal.data_ptr(), self.reward.data_ptr(),
                               self.now.data_ptr(), self.action.data_ptr(), self.detail.data_ptr(), self.flags.data_ptr(),
                               self.stats.data_ptr(), self.sticky.data_ptr(), self.order.data_ptr())
+
+
+def episode_ends(req, running, decisions, cap):
+    """Which of the rows ``running`` end their episode at the request ``req`` (``controllers.evaluate``'s rule): -> (terminal,
+    ended).  Terminal: the request names no charger (``agent_id == -1``).  Ended: terminal, or (``cap`` not None) a request
+    that is not in flight after ``cap`` decisions."""
+    terminal = running & (req.agent_id == -1)
+    ended = terminal
+    if cap is not None:
+        ended = ended | (running & (req.agent_id != -1) & (req.agent_id != -4) & (decisions >= cap))
+    return terminal, ended
+
+
+def episode_step(env, running, action, decisions, returns):
+    """One ``step`` of the rows ``running`` of ``env`` and ``controllers.evaluate``'s accounting of it: a request with no deciding
+    charger (-2) is stepped with agent -1, a step in flight (-4) continues; ``decisions`` counts the actions handed to a deciding
+    charger, ``returns`` adds the reward of the next request (NaN counted as 0)."""
+    aid = env.req.agent_id
+    decided = running & (aid >= 0)
+    env.step(torch.where(aid >= 0, aid, torch.full_like(aid, -1)), action, mask=running)
+    decisions += decided.to(torch.int64)
+    returns += torch.where(running, torch.nan_to_num(env.req.reward, nan=0.0), torch.zeros_like(returns))
 
 
 class BatchedWRSN:
@@ -112,6 +135,7 @@ class BatchedWRSN:
         self._agent_obs = None
         self._fingerprints = None
         self._counts = None
+        self._branches = {}                              # lookahead's branch batches, one per width
         self._make_snapshot()
 
     # ------------------------------------------------------------------ plumbing
@@ -310,6 +334,99 @@ class BatchedWRSN:
         self._call(self.L.wrsn_heuristic_action, C.byref(self.dims), self.scen.data_ptr(), self.scen_id.data_ptr(),
                    self.state.data_ptr(), a.data_ptr(), HEURISTICS.index(kind), out.data_ptr(), self._stream())
         return out
+
+    def heuristic_candidates(self, kind="min_lifetime", width=8, agent_id=None, out=None, node=None):
+        """The rule's ``width`` best candidates (``wrsn_heuristic_candidates``) for every environment with a deciding charger
+        ``agent_id[b] >= 0`` (default: that of the last request): the first ``width`` nodes of ``heuristic_action``'s candidate
+        set in the rule's order (``"min_lifetime"``: lowest lifetime first; ``"nearest_urgent"``: the urgent nodes nearest
+        first, then the rest by lifetime).  -> (actions [B, width, 3] float64, nodes [B, width] int32), slot 0 being
+        ``heuristic_action``'s decision bit for bit.  Slots beyond the row's candidate count hold node -1 and slot 0's action;
+        the other rows of ``out`` / ``node`` are left untouched.  ``width``: 1 to ``WRSN_CAND_MAX`` (32)."""
+        if kind not in HEURISTICS:
+            raise ValueError("kind must be one of %s, not %r" % (", ".join(HEURISTICS), kind))
+        K = int(width)
+        if not 1 <= K <= self.E["WRSN_CAND_MAX"]:
+            raise ValueError("width must lie in [1, %d], not %d" % (self.E["WRSN_CAND_MAX"], K))
+        if agent_id is None:
+            agent_id = self.req.agent_id
+        a = torch.as_tensor(agent_id, device=self.device).to(torch.int32).contiguous()
+        if a.shape != (self.B,):
+            raise ValueError("agent_id must be [B]")
+        if out is None:
+            out = torch.zeros((self.B, K, 3), dtype=torch.float64, device=self.device)
+        if node is None:
+            node = torch.full((self.B, K), -1, dtype=torch.int32, device=self.device)
+        if out.dtype != torch.float64 or not out.is_contiguous() or out.shape != (self.B, K, 3) or out.device != self.state.device:
+            raise ValueError("out must be a contiguous float64 tensor [B, width, 3] on the simulator's device")
+        if node.dtype != torch.int32 or not node.is_contiguous() or node.shape != (self.B, K) or node.device != self.state.device:
+            raise ValueError("node must be a contiguous int32 tensor [B, width] on the simulator's device")
+        self._call(self.L.wrsn_heuristic_candidates, C.byref(self.dims), self.scen.data_ptr(), self.scen_id.data_ptr(),
+                   self.state.data_ptr(), a.data_ptr(), HEURISTICS.index(kind), K, out.data_ptr(), node.data_ptr(), self._stream())
+        return out, node
+
+    def _branch(self, K):
+        """The branch batch of ``lookahead`` for ``K`` candidates: B * K rows of this batch's scenarios and settings."""
+        br = self._branches.get(K)
+        if br is None:
+            d = self.dims
+            br = BatchedWRSN(self.scenarios, num_agent=self.num_agent, mc_type=self.mc_type, num_envs=self.B * K, map_size=self.map_size,
+                             warm_up_time=self.warm_up_time, device=self.device, threads=d.threads, step_budget=d.step_budget,
+                             step_rounds=d.step_rounds)
+            self._branches[K] = br
+        return br
+
+    def lookahead(self, candidates, horizon, rollout_kind="min_lifetime", valid=None):
+        """The value of each candidate action of each environment's deciding charger: for every row b whose request names a
+        charger and every slot k with ``valid[b, k]`` (default all), a copy of the row (``wrsn_copy_rows``) is stepped once with
+        ``candidates[b, k]`` ([B, K, 3] float64, any actions), then under the rule ``rollout_kind`` until it has made
+        ``horizon`` more decisions or its episode has ended, with ``controllers.evaluate``'s accounting (``episode_ends``,
+        ``episode_step``).  -> values [B, K] float64: the sum of the rewards of the branch's requests; -inf for a slot that is
+        not valid, NaN for every slot of a row without a deciding charger.  Those cost no branch work.
+
+        The branches are the rows of a second batch of B * K rows with this batch's scenarios and settings, built at the first
+        call with K candidates and reused.  This batch is not changed.  Host synchronisations: one per branch step after the
+        first ``horizon + 1``, and ``raise_on_error`` of the branch batch at the end."""
+        c = candidates
+        if c.dtype != torch.float64 or not c.is_contiguous() or c.dim() != 3 or c.shape[0] != self.B or c.shape[2] != 3 \
+                or not 1 <= c.shape[1] or c.device != self.state.device:
+            raise ValueError("candidates must be a contiguous float64 tensor [B, K, 3] on the simulator's device")
+        if rollout_kind not in HEURISTICS:
+            raise ValueError("rollout_kind must be one of %s, not %r" % (", ".join(HEURISTICS), rollout_kind))
+        H = int(horizon)
+        if H < 0:
+            raise ValueError("horizon must not be negative")
+        B, K = self.B, int(c.shape[1])
+        if valid is None:
+            valid = torch.ones((B, K), dtype=torch.bool, device=self.device)
+        valid = torch.as_tensor(valid, device=self.device).to(torch.bool)
+        if valid.shape != (B, K):
+            raise ValueError("valid must be [B, K]")
+        br = self._branch(K)
+        aid = self.req.agent_id
+        decider = (aid >= 0) & (aid < self.M)
+        running = (decider[:, None] & valid).reshape(B * K)
+        rows = torch.arange(B * K, dtype=torch.int32, device=self.device)
+        src = torch.where(running, rows // K, torch.full_like(rows, -1))     # -1: skipped by the copy
+        self._call(self.L.wrsn_copy_rows, C.byref(self.dims), B * K, self.state.data_ptr(), C.byref(self.req.c), self.scen_id.data_ptr(),
+                   src.data_ptr(), B, br.state.data_ptr(), C.byref(br.req.c), br.scen_id.data_ptr(), rows.data_ptr(), B * K,
+                   self._stream())
+        br._refresh_counts()
+        dec = torch.zeros(B * K, dtype=torch.int64, device=self.device)
+        ret = torch.zeros(B * K, dtype=torch.float64, device=self.device)
+        action = c.reshape(B * K, 3).clone()
+        cap, k = H + 1, 0
+        while True:
+            _, ended = episode_ends(br.req, running, dec, cap)
+            running &= ~ended
+            if k >= cap and not bool(running.any()):
+                break
+            if k > 0:
+                br.heuristic_action(rollout_kind, out=action)
+            episode_step(br, running, action, dec, ret)
+            k += 1
+        br.raise_on_error()
+        val = torch.where(valid, ret.view(B, K), torch.full_like(ret.view(B, K), -math.inf))
+        return torch.where(decider[:, None], val, torch.full_like(val, math.nan))
 
     def get_network_fitness(self):
         """``WRSN.get_network_fitness`` (:188-220): per-target values [B, T] and their minimum [B] over each row's own

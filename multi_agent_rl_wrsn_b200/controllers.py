@@ -13,7 +13,7 @@ import math
 import torch
 
 from . import _lib
-from .batched import HEURISTICS, BatchedWRSN
+from .batched import HEURISTICS, BatchedWRSN, episode_ends, episode_step
 from .sharding import reduce_stats
 
 
@@ -47,19 +47,63 @@ class HeuristicController:
         return wrsn.heuristic_action(agent_id, self.heuristic)
 
 
+class LookaheadController:
+    """A rollout planner over a hand-written rule: at every decision it ranks the rule's ``width`` best nodes
+    (``BatchedWRSN.heuristic_candidates``), tries each one at the rule's own charge fraction and then at each fraction of
+    ``charge_levels`` (absolute, in [0, 1]), values every try by ``BatchedWRSN.lookahead`` (one step with it, then ``horizon``
+    decisions of the rule ``kind``) and acts on the best.  Ties go to the lowest slot, so the rule's own decision (slot 0)
+    wins them; with ``width=1`` and no ``charge_levels`` it decides as ``HeuristicController(kind)``.  ``rollout`` and
+    ``evaluate`` take its action through ``plan``."""
+
+    def __init__(self, kind="min_lifetime", width=8, horizon=4, charge_levels=()):
+        if kind not in HEURISTICS:
+            raise ValueError("kind must be one of %s, not %r" % (", ".join(HEURISTICS), kind))
+        self.kind, self.width, self.horizon = kind, int(width), int(horizon)
+        self.charge_levels = tuple(float(c) for c in charge_levels)
+        if not all(0.0 <= c <= 1.0 for c in self.charge_levels):
+            raise ValueError("charge_levels must lie in [0, 1]")
+        self.last = None                                                  # (values, chosen slot) of the last plan
+
+    def candidates(self, env):
+        """-> (actions [B, K, 3], valid [B, K]) with K = width * (1 + len(charge_levels)): slot n * (1 + L) + l is the rule's
+        n-th node at its own charge fraction (l = 0) or at ``charge_levels[l - 1]``.  Slot 0 is valid even without a node
+        (the rule's stay action)."""
+        act, node = env.heuristic_candidates(self.kind, self.width)
+        L = len(self.charge_levels)
+        act = act[:, :, None, :].expand(env.B, self.width, 1 + L, 3).clone()
+        for l, c in enumerate(self.charge_levels):
+            act[:, :, l + 1, 2] = c
+        valid = (node >= 0)[:, :, None].expand(env.B, self.width, 1 + L).reshape(env.B, -1).clone()
+        valid[:, 0] = True
+        return act.reshape(env.B, -1, 3), valid
+
+    def plan(self, env, out):
+        """Write the planner's decision for every row of ``env`` (a ``BatchedWRSN``) with a deciding charger into ``out``
+        [B, 3]; the other rows are left untouched."""
+        cand, valid = self.candidates(env)
+        values = env.lookahead(cand, self.horizon, self.kind, valid)
+        best = torch.argmax(values, dim=1)                                # the first of equal maxima
+        chosen = cand.gather(1, best[:, None, None].expand(env.B, 1, 3))[:, 0]
+        out.copy_(torch.where((env.req.agent_id >= 0)[:, None], chosen, out))
+        self.last = (values, best)
+        return out
+
+
 def rollout(env, controller, steps, obs=None, group=None):
     """``steps`` rollout steps of every environment of ``env`` (a ``BatchedWRSN``) under ``controller``.
 
     Returns the observation tensor and job-wide statistics (summed over ranks when torch.distributed is initialised:
     the only collective of the whole path): decisions handed out, simulated seconds, episodes finished, sum of rewards.
-    A controller with ``heuristic`` (``HeuristicController``) decides from the state record: its steps render no observation,
-    and ``obs`` is filled once, after the last step.
+    A controller with ``plan`` (``LookaheadController``) or ``heuristic`` (``HeuristicController``) decides from the state
+    record: its steps render no observation, and ``obs`` is filled once, after the last step.
     """
     B, S, dev = env.B, env.S, env.device
+    plan = getattr(controller, "plan", None)
     heuristic = getattr(controller, "heuristic", None)
+    from_state = plan is not None or heuristic is not None
     if obs is None:
         obs = torch.zeros((B, 4, S, S), dtype=torch.float32, device=dev)
-        if heuristic is None:
+        if not from_state:
             env.get_state(out=obs)
     action = torch.zeros((B, 3), dtype=torch.float64, device=dev)
     local = torch.zeros(2, dtype=torch.float64, device=dev)               # episodes finished, sum of rewards
@@ -67,8 +111,11 @@ def rollout(env, controller, steps, obs=None, group=None):
     dec0, sim0 = reduce_stats(env, group)
     fused = getattr(controller, "weights", None) is not None and obs.dtype == torch.float32
     for _ in range(int(steps)):
-        if heuristic is not None:                                         # action straight from the state record
-            env.heuristic_action(heuristic, out=action)
+        if from_state:                                                    # action straight from the state record
+            if plan is not None:
+                plan(env, action)
+            else:
+                env.heuristic_action(heuristic, out=action)
             env.rollout_step(action)
             local[1] += torch.nan_to_num(env.req.reward, nan=0.0).sum()
             continue
@@ -84,7 +131,7 @@ def rollout(env, controller, steps, obs=None, group=None):
             action.copy_(a)
         env.rollout_step(action, obs)
         local[1] += torch.nan_to_num(env.req.reward, nan=0.0).sum()
-    if heuristic is not None:
+    if from_state:
         env.get_state(out=obs)
     local[0] = env.req.stats[:, 2].sum() - resets0                        # episodes that ended (and were reset) in these steps
     if torch.distributed.is_available() and torch.distributed.is_initialized() and torch.distributed.get_world_size(group) > 1:
@@ -103,7 +150,8 @@ def evaluate(env, controller, episodes=1, max_decisions=None, check_every=16):
     charger is), or — with ``max_decisions`` — at the first request after that many decisions (``truncated``).  Each row is
     stepped with ``step(mask=running)``, so its terminal request is read before ``reset(mask=finished)`` starts the next
     episode.  A request with no deciding charger that is not terminal (``agent_id == -2``) is stepped with agent -1; a step in
-    flight (-4) continues.  The decision comes from ``heuristic`` (``HeuristicController``) when the controller has one;
+    flight (-4) continues.  The decision comes from ``plan(env, out)`` (``LookaheadController``) when the controller has one,
+    else from ``heuristic`` (``HeuristicController``);
     otherwise from ``make_action(agent_id, obs)`` on the float32 observation (``get_state`` into one reused buffer), its maps
     decoded by ``density_map_to_action``, or by ``linear_controller_action`` when the controller has ``weights``.  A
     ``make_action`` that returns ``(action, log_prob)`` (a ``PerAgentPolicy``) is accepted.  The loop synchronises with the
@@ -117,9 +165,10 @@ def evaluate(env, controller, episodes=1, max_decisions=None, check_every=16):
     if E < 1 or int(check_every) < 1:
         raise ValueError("episodes and check_every must be at least 1")
     cap = None if max_decisions is None else int(max_decisions)
+    plan = getattr(controller, "plan", None)
     heuristic = getattr(controller, "heuristic", None)
     weights = getattr(controller, "weights", None)
-    obs = None if heuristic is not None else torch.zeros((B, 4, env.S, env.S), dtype=torch.float32, device=dev)
+    obs = None if heuristic is not None or plan is not None else torch.zeros((B, 4, env.S, env.S), dtype=torch.float32, device=dev)
     lifetime = torch.zeros((B, E), dtype=torch.float64, device=dev)
     ret = torch.zeros((B, E), dtype=torch.float64, device=dev)
     decisions = torch.zeros((B, E), dtype=torch.int64, device=dev)
@@ -134,10 +183,7 @@ def evaluate(env, controller, episodes=1, max_decisions=None, check_every=16):
     while True:
         req = env.req
         running = done < E
-        fin_term = running & (req.agent_id == -1)
-        fin = fin_term
-        if cap is not None:
-            fin = fin | (running & (req.agent_id != -1) & (req.agent_id != -4) & (cur_dec >= cap))
+        fin_term, fin = episode_ends(req, running, cur_dec, cap)
         hit = fin[:, None] & (cols[None, :] == done[:, None])            # this episode's column
         lifetime.copy_(torch.where(hit, (req.now - env.warm_up_time)[:, None], lifetime))
         ret.copy_(torch.where(hit, cur_ret[:, None], ret))
@@ -152,7 +198,9 @@ def evaluate(env, controller, episodes=1, max_decisions=None, check_every=16):
             break
         k += 1
         aid = req.agent_id
-        if heuristic is not None:
+        if plan is not None:
+            plan(env, action)
+        elif heuristic is not None:
             env.heuristic_action(heuristic, out=action)
         else:
             env.get_state(out=obs)
@@ -166,10 +214,7 @@ def evaluate(env, controller, episodes=1, max_decisions=None, check_every=16):
                     env.density_map_to_action(a.contiguous(), out=action)
                 else:
                     action.copy_(a)
-        decided = running & (aid >= 0)
-        env.step(torch.where(aid >= 0, aid, torch.full_like(aid, -1)), action, mask=running)
-        cur_dec += decided.to(torch.int64)
-        cur_ret += torch.where(running, torch.nan_to_num(req.reward, nan=0.0), torch.zeros_like(cur_ret))
+        episode_step(env, running, action, cur_dec, cur_ret)
     env.raise_on_error()
     return {"lifetime": lifetime, "return": ret, "decisions": decisions, "truncated": truncated}
 

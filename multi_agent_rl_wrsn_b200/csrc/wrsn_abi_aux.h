@@ -8,8 +8,9 @@
  *   launch_decode(P, agent_id, dmap, dmap_f64, channels, weights, action_out, stream)
  *                                                                 both decode entry points (channels = 0: dmap is the map);
  *   launch_charge(P, charging, node_rate, mc_rate, stream)        wrsn_k_charge;
- *   launch_heuristic(P, agent_id, kind, action, stream)           wrsn_heuristic_action (the CUDA library only: the host
- *                                                                 emulation's row-by-row loop is defined below).
+ *   launch_heuristic(P, agent_id, kind, action, stream)           wrsn_heuristic_action;
+ *   launch_candidates(P, agent_id, kind, K, action, node, stream) wrsn_heuristic_candidates (these two in the CUDA library
+ *                                                                 only: the host emulation's row-by-row loops are defined below).
  */
 #pragma once
 #include "wrsn_abi_host.h"
@@ -20,6 +21,7 @@ static int launch_decode(KParams &P, const int32_t *agent_id, const void *dmap, 
                          double *action_out, void *stream);
 static int launch_charge(KParams &P, const uint8_t *charging, double *node_rate, double *mc_rate, void *stream);
 static int launch_heuristic(KParams &P, const int32_t *agent_id, int kind, double *action, void *stream);
+static int launch_candidates(KParams &P, const int32_t *agent_id, int kind, int K, double *action, int32_t *node, void *stream);
 
 /* once the arguments are checked: the dims and the layout they imply */
 #if defined(WRSN_HOST_EMU)
@@ -43,6 +45,29 @@ static int launch_heuristic(KParams &P, const int32_t *agent_id, int kind, doubl
             pick = p.choice();
         }
         heur_action(rw, a, pick, action + 3 * (size_t)b);
+    }
+    return 0;
+}
+
+/* the host emulation's wrsn_heuristic_candidates: the K first nodes of the order (wrsn_layout.h: heur_rank, heur_insert), row by
+ * row and node by node, pass 1 only when pass 0 has no candidate */
+static int launch_candidates(KParams &P, const int32_t *agent_id, int kind, int K, double *action, int32_t *node, void *) {
+    for (int b = 0; b < P.d.B; b++) {
+        const int a = agent_id[b];
+        if (a < 0 || a >= P.d.M) continue;
+        const WrsnRow rw(P.L, P.state, P.scen, P.scen_id, b);
+        HeurFleet f = HeurFleet();
+        f.M = P.d.M;
+        for (int j = 0; j < f.M; j++) heur_charger(rw, a, j, &f);
+        HeurRank l[WRSN_CAND_MAX];
+        int n = 0;
+        for (int pass = 0; pass < 2 && n == 0; pass++)
+            for (int i = 0; i < rw.N; i++) {
+                HeurRank r;
+                if (heur_rank(rw, f, kind, i, pass, &r)) heur_insert(l, 1, n, K, r);
+            }
+        for (int k = 0; k < K; k++)
+            heur_slot(rw, a, k < n ? l[k].id : -1, n ? l[0].id : -1, action + 3 * ((size_t)b * K + k), node + (size_t)b * K + k);
     }
     return 0;
 }
@@ -107,6 +132,16 @@ int wrsn_heuristic_action(const wrsn_dims *d, const void *scen, const int32_t *s
     if (kind < 0 || kind >= WRSN_HEUR_COUNT) WRSN_FAIL("heuristic kind %d: 0 (min_lifetime) or 1 (nearest_urgent)", kind);
     KParams P = aux_params(d, scen, scen_id, state);
     return launch_heuristic(P, agent_id, kind, action, stream);
+}
+
+int wrsn_heuristic_candidates(const wrsn_dims *d, const void *scen, const int32_t *scen_id, const void *state,
+                              const int32_t *agent_id, int kind, int K, double *action, int32_t *node, void *stream) {
+    if (check_dims(d)) return -1;
+    if (!agent_id || !action || !node || !scen || !scen_id || !state) WRSN_FAIL("NULL argument");
+    if (kind < 0 || kind >= WRSN_HEUR_COUNT) WRSN_FAIL("heuristic kind %d: 0 (min_lifetime) or 1 (nearest_urgent)", kind);
+    if (K < 1 || K > WRSN_CAND_MAX) WRSN_FAIL("K = %d candidates: 1 to %d", K, WRSN_CAND_MAX);
+    KParams P = aux_params(d, scen, scen_id, state);
+    return launch_candidates(P, agent_id, kind, K, action, node, stream);
 }
 
 }  /* extern "C" */

@@ -778,6 +778,57 @@ __global__ void __launch_bounds__(32 * HEUR_WARPS, 3) k_heuristic(const KParams 
     if (lane == 0) heur_action(rw, a, pick, action + 3 * (size_t)b);
 }
 
+/* the rule's K best candidates (include/wrsn_b200.h: wrsn_heuristic_candidates; the order: wrsn_layout.h, heur_rank /
+ * heur_before): one warp per row, in the style of k_heuristic.  Lanes stride the row's nodes and each keeps the smallest entries
+ * of its own nodes in an ascending column of shared memory (heur_insert), so every node's key is computed once.  A lane sees
+ * at most ceil(N / 32) nodes, so a column holds cap = min(K, ceil(N / 32)) entries.  The warp then takes the K smallest of the
+ * columns' heads one at a time: a shuffle butterfly on the total order finds the smallest head, its lane moves to its next
+ * entry, and lane k keeps the node of rank k. */
+#define CAND_WARPS 4
+__global__ void __launch_bounds__(32 * CAND_WARPS) k_heuristic_candidates(const KParams P, const int32_t *__restrict__ agent_id, int kind,
+                                                                         int K, int cap, double *__restrict__ action,
+                                                                         int32_t *__restrict__ node) {
+    extern __shared__ HeurRank s_cand[];                      /* [CAND_WARPS][cap][32] */
+    __shared__ HeurFleet s_fleet[CAND_WARPS];
+    const int wrp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int b = blockIdx.x * CAND_WARPS + wrp;
+    if (b >= P.d.B) return;                                   /* whole warps leave together; only warp-level sync below */
+    const int a = agent_id[b];
+    if (a < 0 || a >= P.d.M) return;
+    const WrsnRow rw(P.L, P.state, P.scen, P.scen_id, b);
+    HeurFleet &f = s_fleet[wrp];
+    if (lane < P.d.M) heur_charger(rw, a, lane, &f);
+    if (lane == 0) f.M = P.d.M;
+    __syncwarp();
+    HeurRank *col = s_cand + (size_t)wrp * cap * 32 + lane;
+    int n = 0;
+    for (int pass = 0; pass < 2 && !__any_sync(0xffffffffu, n > 0); pass++)
+        for (int i = lane; i < rw.N; i += 32) {
+            HeurRank r;
+            if (heur_rank(rw, f, kind, i, pass, &r)) heur_insert(col, 32, n, cap, r);
+        }
+    int head = 0, mine = -1, first = -1;
+    for (int k = 0; k < K; k++) {
+        HeurRank h;
+        if (head < n) h = col[head * 32];
+        else { h.cls = 2; h.key = (double)INFINITY; h.id = HEUR_NONE; }   /* sorts after every candidate */
+        HeurRank w = h;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            HeurRank q;
+            q.key = __shfl_xor_sync(0xffffffffu, w.key, o);
+            q.cls = __shfl_xor_sync(0xffffffffu, w.cls, o);
+            q.id = __shfl_xor_sync(0xffffffffu, w.id, o);
+            if (heur_before(q, w)) w = q;
+        }
+        if (w.id == HEUR_NONE) break;                         /* warp-uniform: fewer than K candidates */
+        if (head < n && h.id == w.id) head++;
+        if (lane == k) mine = w.id;
+        if (k == 0) first = w.id;
+    }
+    if (lane < K) heur_slot(rw, a, mine, first, action + 3 * ((size_t)b * K + lane), node + (size_t)b * K + lane);
+}
+
 /* roll_out bookkeeping (IPPO.py:138-155): one thread per environment, see include/wrsn_b200.h */
 __global__ void k_record_transitions(int B, int M, wrsn_request req, int64_t t, const int64_t *__restrict__ agent_prev,
                                      int64_t *__restrict__ last, double *__restrict__ resets_seen,
@@ -947,6 +998,24 @@ static int launch_charge(KParams &P, const uint8_t *charging, double *node_rate,
 
 static int launch_heuristic(KParams &P, const int32_t *agent_id, int kind, double *action, void *stream) {
     k_heuristic<<<(P.d.B + HEUR_WARPS - 1) / HEUR_WARPS, 32 * HEUR_WARPS, 0, (cudaStream_t)stream>>>(P, agent_id, kind, action);
+    WRSN_CUDA(cudaGetLastError());
+    return 0;
+}
+
+static int launch_candidates(KParams &P, const int32_t *agent_id, int kind, int K, double *action, int32_t *node, void *stream) {
+    const int per_lane = (P.d.N + 31) / 32, cap = K < per_lane ? K : per_lane;
+    const size_t smem = sizeof(HeurRank) * CAND_WARPS * 32 * (size_t)cap;   /* at most 64 KB (K <= WRSN_CAND_MAX) */
+    static bool attr[WRSN_MAX_DEVICES];                       /* per device, see launch_env */
+    int dev = 0;
+    WRSN_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= WRSN_MAX_DEVICES) WRSN_FAIL("device ordinal %d not supported", dev);
+    if (!attr[dev]) {
+        WRSN_CUDA(cudaFuncSetAttribute(k_heuristic_candidates, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)(sizeof(HeurRank) * CAND_WARPS * 32 * WRSN_CAND_MAX)));
+        attr[dev] = true;
+    }
+    k_heuristic_candidates<<<(P.d.B + CAND_WARPS - 1) / CAND_WARPS, 32 * CAND_WARPS, smem, (cudaStream_t)stream>>>(P, agent_id, kind, K,
+                                                                                                                  cap, action, node);
     WRSN_CUDA(cudaGetLastError());
     return 0;
 }

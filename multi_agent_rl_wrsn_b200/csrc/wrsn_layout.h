@@ -262,6 +262,42 @@ WRSN_HD void heur_action(const WrsnRow &rw, int a, int i, double *out) {
     out[2] = c;
 }
 
+/* The rule's candidate order (include/wrsn_b200.h: wrsn_heuristic_candidates): one total order on (class, key, id), node ids
+ * being distinct.  heur_key's urgent nodes come first (class 0, key: the distance from charger a), then the rest (class 1,
+ * key: the lifetime), so the order's first node is HeurPick's choice.  k_heuristic_candidates and the host emulation state the
+ * order only through these functions. */
+struct HeurRank { double key; int cls, id; };
+
+/* node i's place in the order; false when i is not a candidate in this pass */
+WRSN_HD bool heur_rank(const WrsnRow &rw, const HeurFleet &f, int kind, int i, int pass, HeurRank *r) {
+    double key[2] = {0.0, 0.0};
+    const int c = heur_key(rw, f, kind, i, pass, key);
+    if (c == 0) return false;
+    r->cls = c == 2 ? 0 : 1;
+    r->key = key[c - 1];
+    r->id = i;
+    return true;
+}
+
+WRSN_HD bool heur_before(const HeurRank &p, const HeurRank &q) {
+    return p.cls < q.cls || (p.cls == q.cls && (p.key < q.key || (p.key == q.key && p.id < q.id)));
+}
+
+/* insert r into the ascending list l[0], l[s], ..., l[(n - 1) s] that keeps the cap smallest entries seen (stride s: one lane's
+ * column of k_heuristic_candidates' shared list, 1 on the host) */
+WRSN_HD void heur_insert(HeurRank *l, int s, int &n, int cap, const HeurRank &r) {
+    if (n == cap && !heur_before(r, l[(n - 1) * s])) return;
+    int p = n < cap ? n++ : cap - 1;
+    for (; p > 0 && heur_before(r, l[(p - 1) * s]); p--) l[p * s] = l[(p - 1) * s];
+    l[p * s] = r;
+}
+
+/* slot k of row b: the node of rank k (node_k < 0: fewer candidates than slots), with slot 0's action when it has none */
+WRSN_HD void heur_slot(const WrsnRow &rw, int a, int node_k, int node_0, double *action, int32_t *node) {
+    heur_action(rw, a, node_k >= 0 ? node_k : node_0, action);
+    *node = node_k;
+}
+
 /* request record of one environment, as the engine's entry points produce it */
 struct ReqOut { int agent; int terminal; double reward, now, act[3], detail[2]; int flags; };
 
