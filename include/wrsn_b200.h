@@ -323,6 +323,26 @@ int wrsn_heuristic_candidates(const wrsn_dims *d, const void *scen, const int32_
                               const int32_t *agent_id, int kind, int K, double *action /* [B][K][3] */, int32_t *node /* [B][K] */,
                               void *stream);
 
+#define WRSN_ROLL_MAX 65536     /* decisions per row and launch of wrsn_rule_rollout */
+/* Rule rollouts without the host: every row b with running[b] != 0 continues from its request under the rule `kind`
+ * (wrsn_heuristic_action's) inside one launch, request after request, with the accounting of an evaluation loop that calls
+ * wrsn_heuristic_action and wrsn_step once per request:
+ *   agent_id == -1                          the episode has ended: running[b] = 0
+ *   agent_id != -4, decisions[b] >= limit   cut by the limit: running[b] = 0
+ *   agent_id >= 0                           a step with first_action[b] (when first_action != NULL and decisions[b] == 0) or the
+ *                                           rule's action for that charger; decisions[b] += 1
+ *   agent_id == -2 or -3                    a step with agent -1;   agent_id == -4: the step in flight continues
+ * After every step returns[b] += the reward of the new request (NaN counted as 0, +-inf as +-DBL_MAX), and stats / sticky of req
+ * are kept as wrsn_step keeps them.  A row that is still running ends the launch when its step comes back in flight (the
+ * dims' step_budget, > 0, bounds the work of the whole launch, not of each step; step_rounds is not used: every step runs in
+ * one kernel) or when it has handed out launch_max decisions in this launch.  The request record then holds the row's last
+ * request; a row that ends without a step keeps its request.  Rows with running[b] == 0 are not touched.  Refused: kind
+ * outside [0, WRSN_HEUR_COUNT), limit < 0, launch_max outside [1, WRSN_ROLL_MAX], NULL running, decisions, returns or
+ * req->agent_id. */
+int wrsn_rule_rollout(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, uint8_t *running /* [B] in/out */,
+                      int kind, const double *first_action /* [B][3] or NULL */, int64_t limit, int32_t launch_max,
+                      int64_t *decisions /* [B] in/out */, double *returns /* [B] in/out */, wrsn_request *req, void *stream);
+
 /* standalone per-tick kernels (the same device functions the fused step uses; unit parity + ncu evidence) */
 int wrsn_k_bfs(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream);      /* Network.setLevels + receivers + relay counts */
 int wrsn_k_drain(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, void *stream);    /* Node.operate k+0.5 tick */

@@ -82,6 +82,7 @@ def _bind(L):
     L.wrsn_decode_linear_controller.argtypes = [dp, vp, vp, vp, vp, vp, ip, C.POINTER(C.c_float), vp, vp]
     L.wrsn_heuristic_action.argtypes = [dp, vp, vp, vp, vp, ip, vp, vp]
     L.wrsn_heuristic_candidates.argtypes = [dp, vp, vp, vp, vp, ip, ip, vp, vp, vp]
+    L.wrsn_rule_rollout.argtypes = [dp, vp, vp, vp, vp, ip, vp, C.c_int64, C.c_int32, vp, vp, C.POINTER(Request), vp]
     for k in ("wrsn_k_bfs", "wrsn_k_drain", "wrsn_k_bookkeep", "wrsn_k_reward"):
         getattr(L, k).argtypes = [dp, vp, vp, vp, vp]
     e = enums()

@@ -364,6 +364,52 @@ class BatchedWRSN:
                    self.state.data_ptr(), a.data_ptr(), HEURISTICS.index(kind), K, out.data_ptr(), node.data_ptr(), self._stream())
         return out, node
 
+    def rule_rollout(self, kind, limit, first_action=None, running=None, decisions=None, returns=None, launch_max=None):
+        """Continue the rows ``running`` (bool [B]; default: every row whose request names a deciding charger) under the rule
+        ``kind`` (one of ``HEURISTICS``) until each one's episode ends (``agent_id == -1``) or, at a request that is not in flight,
+        it has made ``limit`` decisions — ``controllers.evaluate``'s accounting (``episode_ends``, ``episode_step``), run on the
+        device by ``wrsn_rule_rollout``: the rule decides inside the step kernel and the row keeps stepping.  A row's first
+        decision (``decisions[b] == 0``) takes ``first_action[b]`` ([B, 3] float64) when given.  ``decisions`` (int64 [B]) counts
+        the actions handed out and ``returns`` (float64 [B]) adds the reward of every request after a step (NaN counted as 0);
+        both start at 0 unless given, and are updated in place when given.  Each launch hands out at most ``launch_max`` (default
+        1024) decisions per row; the dims' ``step_budget`` bounds the work of a whole launch.  One host synchronisation per
+        launch, then ``raise_on_error``.  -> (returns, decisions, running), ``running`` all False; the request record holds
+        every row's last request."""
+        if kind not in HEURISTICS:
+            raise ValueError("kind must be one of %s, not %r" % (", ".join(HEURISTICS), kind))
+        limit = int(limit)
+        lm = 1024 if launch_max is None else int(launch_max)
+        if limit < 0:
+            raise ValueError("limit must not be negative")
+        if not 1 <= lm <= self.E["WRSN_ROLL_MAX"]:
+            raise ValueError("launch_max must lie in [1, %d], not %d" % (self.E["WRSN_ROLL_MAX"], lm))
+        B, dev = self.B, self.state.device
+
+        def own(x, dtype, shape, name, default):
+            if x is None:
+                return default()
+            if x.dtype != dtype or not x.is_contiguous() or tuple(x.shape) != shape or x.device != dev:
+                raise ValueError("%s must be a contiguous %s tensor %s on the simulator's device" % (name, str(dtype)[6:], list(shape)))
+            return x
+
+        fa = None
+        if first_action is not None:
+            fa = own(first_action, torch.float64, (B, 3), "first_action", None)
+        dec = own(decisions, torch.int64, (B,), "decisions", lambda: torch.zeros(B, dtype=torch.int64, device=dev))
+        ret = own(returns, torch.float64, (B,), "returns", lambda: torch.zeros(B, dtype=torch.float64, device=dev))
+        if running is None:
+            run = (self.req.agent_id >= 0).to(torch.uint8)
+        else:
+            if running.shape != (B,) or running.device != dev or running.dtype not in (torch.bool, torch.uint8):
+                raise ValueError("running must be a bool / uint8 tensor [B] on the simulator's device")
+            run = running.to(torch.uint8).contiguous()
+        while bool(run.any()):                           # one host synchronisation per launch
+            self._call(self.L.wrsn_rule_rollout, C.byref(self.dims), self.scen.data_ptr(), self.scen_id.data_ptr(),
+                       self.state.data_ptr(), run.data_ptr(), HEURISTICS.index(kind), None if fa is None else fa.data_ptr(),
+                       limit, lm, dec.data_ptr(), ret.data_ptr(), C.byref(self.req.c), self._stream())
+        self.raise_on_error()
+        return ret, dec, run.to(torch.bool)
+
     def _branch(self, K):
         """The branch batch of ``lookahead`` for ``K`` candidates: B * K rows of this batch's scenarios and settings."""
         br = self._branches.get(K)
@@ -384,8 +430,9 @@ class BatchedWRSN:
         not valid, NaN for every slot of a row without a deciding charger.  Those cost no branch work.
 
         The branches are the rows of a second batch of B * K rows with this batch's scenarios and settings, built at the first
-        call with K candidates and reused.  This batch is not changed.  Host synchronisations: one per branch step after the
-        first ``horizon + 1``, and ``raise_on_error`` of the branch batch at the end."""
+        call with K candidates and reused, and run by one ``rule_rollout`` of ``horizon + 1`` decisions that starts with the
+        candidates.  This batch is not changed.  Host synchronisations: one per launch of the rollout (one when no branch runs
+        into the step budget or past 1024 decisions), and ``raise_on_error`` of the branch batch at the end."""
         c = candidates
         if c.dtype != torch.float64 or not c.is_contiguous() or c.dim() != 3 or c.shape[0] != self.B or c.shape[2] != 3 \
                 or not 1 <= c.shape[1] or c.device != self.state.device:
@@ -411,20 +458,7 @@ class BatchedWRSN:
                    src.data_ptr(), B, br.state.data_ptr(), C.byref(br.req.c), br.scen_id.data_ptr(), rows.data_ptr(), B * K,
                    self._stream())
         br._refresh_counts()
-        dec = torch.zeros(B * K, dtype=torch.int64, device=self.device)
-        ret = torch.zeros(B * K, dtype=torch.float64, device=self.device)
-        action = c.reshape(B * K, 3).clone()
-        cap, k = H + 1, 0
-        while True:
-            _, ended = episode_ends(br.req, running, dec, cap)
-            running &= ~ended
-            if k >= cap and not bool(running.any()):
-                break
-            if k > 0:
-                br.heuristic_action(rollout_kind, out=action)
-            episode_step(br, running, action, dec, ret)
-            k += 1
-        br.raise_on_error()
+        ret, _, _ = br.rule_rollout(rollout_kind, H + 1, first_action=c.reshape(B * K, 3), running=running)
         val = torch.where(valid, ret.view(B, K), torch.full_like(ret.view(B, K), -math.inf))
         return torch.where(decider[:, None], val, torch.full_like(val, math.nan))
 

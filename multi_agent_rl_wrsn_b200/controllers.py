@@ -150,8 +150,9 @@ def evaluate(env, controller, episodes=1, max_decisions=None, check_every=16):
     charger is), or — with ``max_decisions`` — at the first request after that many decisions (``truncated``).  Each row is
     stepped with ``step(mask=running)``, so its terminal request is read before ``reset(mask=finished)`` starts the next
     episode.  A request with no deciding charger that is not terminal (``agent_id == -2``) is stepped with agent -1; a step in
-    flight (-4) continues.  The decision comes from ``plan(env, out)`` (``LookaheadController``) when the controller has one,
-    else from ``heuristic`` (``HeuristicController``);
+    flight (-4) continues.  The decision comes from ``plan(env, out)`` (``LookaheadController``) when the controller has one;
+    a controller with ``heuristic`` (``HeuristicController``) runs each episode, for every row at once, as one
+    ``BatchedWRSN.rule_rollout`` from the reset, which takes the same decisions without the per-request loop;
     otherwise from ``make_action(agent_id, obs)`` on the float32 observation (``get_state`` into one reused buffer), its maps
     decoded by ``density_map_to_action``, or by ``linear_controller_action`` when the controller has ``weights``.  A
     ``make_action`` that returns ``(action, log_prob)`` (a ``PerAgentPolicy``) is accepted.  The loop synchronises with the
@@ -179,6 +180,15 @@ def evaluate(env, controller, episodes=1, max_decisions=None, check_every=16):
     action = torch.zeros((B, 3), dtype=torch.float64, device=dev)
     cols = torch.arange(E, device=dev)
     env.reset()
+    if plan is None and heuristic is not None:
+        for e in range(E):
+            if e:
+                env.reset()
+            r, d, _ = env.rule_rollout(heuristic, 1 << 62 if cap is None else cap, running=torch.ones(B, dtype=torch.bool, device=dev))
+            lifetime[:, e] = env.req.now - env.warm_up_time
+            ret[:, e], decisions[:, e] = r, d
+            truncated[:, e] = env.req.agent_id != -1
+        return {"lifetime": lifetime, "return": ret, "decisions": decisions, "truncated": truncated}
     k = 0
     while True:
         req = env.req
@@ -200,8 +210,6 @@ def evaluate(env, controller, episodes=1, max_decisions=None, check_every=16):
         aid = req.agent_id
         if plan is not None:
             plan(env, action)
-        elif heuristic is not None:
-            env.heuristic_action(heuristic, out=action)
         else:
             env.get_state(out=obs)
             if weights is not None:

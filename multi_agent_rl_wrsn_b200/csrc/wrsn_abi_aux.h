@@ -11,9 +11,15 @@
  *   launch_heuristic(P, agent_id, kind, action, stream)           wrsn_heuristic_action;
  *   launch_candidates(P, agent_id, kind, K, action, node, stream) wrsn_heuristic_candidates (these two in the CUDA library
  *                                                                 only: the host emulation's row-by-row loops are defined below).
+ *   launch_roll(P, R, stream)                                     wrsn_rule_rollout: env_run<MODE_RULE_ROLLOUT> with its
+ *                                                                 arguments R (the CUDA library's k_env_roll; the host
+ *                                                                 emulation's row-by-row loop is defined below as well).
  */
 #pragma once
 #include "wrsn_abi_host.h"
+#if defined(WRSN_HOST_EMU)
+#include <vector>
+#endif
 
 static int launch_obs_tables(KParams &P, void *stream);
 static int launch_observe(KParams &P, const int32_t *agent_id, void *obs, int obs_f64, void *stream);
@@ -22,6 +28,7 @@ static int launch_decode(KParams &P, const int32_t *agent_id, const void *dmap, 
 static int launch_charge(KParams &P, const uint8_t *charging, double *node_rate, double *mc_rate, void *stream);
 static int launch_heuristic(KParams &P, const int32_t *agent_id, int kind, double *action, void *stream);
 static int launch_candidates(KParams &P, const int32_t *agent_id, int kind, int K, double *action, int32_t *node, void *stream);
+static int launch_roll(KParams &P, const RollArgs &R, void *stream);
 
 /* once the arguments are checked: the dims and the layout they imply */
 #if defined(WRSN_HOST_EMU)
@@ -69,6 +76,15 @@ static int launch_candidates(KParams &P, const int32_t *agent_id, int kind, int 
         for (int k = 0; k < K; k++)
             heur_slot(rw, a, k < n ? l[k].id : -1, n ? l[0].id : -1, action + 3 * ((size_t)b * K + k), node + (size_t)b * K + k);
     }
+    return 0;
+}
+
+/* the host emulation's wrsn_rule_rollout: env_run<MODE_RULE_ROLLOUT> row by row on one lane, as its launch_env runs every mode */
+static int launch_roll(KParams &P, const RollArgs &R, void *) {
+    if (prepare_launch(P)) return -1;
+    std::vector<char> smem((size_t)P.L.smem_total + 64);
+    wrsn_smem_host = smem.data();
+    for (int b = 0; b < P.d.B; b++) env_run<MODE_RULE_ROLLOUT>(P, b, 0, 1, R);
     return 0;
 }
 #endif
@@ -142,6 +158,22 @@ int wrsn_heuristic_candidates(const wrsn_dims *d, const void *scen, const int32_
     if (K < 1 || K > WRSN_CAND_MAX) WRSN_FAIL("K = %d candidates: 1 to %d", K, WRSN_CAND_MAX);
     KParams P = aux_params(d, scen, scen_id, state);
     return launch_candidates(P, agent_id, kind, K, action, node, stream);
+}
+
+int wrsn_rule_rollout(const wrsn_dims *d, const void *scen, const int32_t *scen_id, void *state, uint8_t *running, int kind,
+                      const double *first_action, int64_t limit, int32_t launch_max, int64_t *decisions, double *returns,
+                      wrsn_request *req, void *stream) {
+    if (check_dims(d)) return -1;
+    if (!scen || !scen_id || !state || !running || !decisions || !returns || !req || !req->agent_id) WRSN_FAIL("NULL argument");
+    if (kind < 0 || kind >= WRSN_HEUR_COUNT) WRSN_FAIL("heuristic kind %d: 0 (min_lifetime) or 1 (nearest_urgent)", kind);
+    if (limit < 0) WRSN_FAIL("limit = %lld decisions: must not be negative", (long long)limit);
+    if (launch_max < 1 || launch_max > WRSN_ROLL_MAX) WRSN_FAIL("launch_max = %d decisions: 1 to %d", (int)launch_max, WRSN_ROLL_MAX);
+    KParams P = base_params(d, scen, scen_id, state, nullptr);
+    P.req = *req;
+    RollArgs R;
+    R.running = running; R.decisions = decisions; R.returns = returns; R.first = first_action;
+    R.limit = limit; R.kind = kind; R.launch_max = launch_max;
+    return launch_roll(P, R, stream);
 }
 
 }  /* extern "C" */

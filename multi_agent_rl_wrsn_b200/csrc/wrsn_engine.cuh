@@ -2287,7 +2287,7 @@ WRSN_D bool any_watched(Ctx &c) {                   /* a lazy move whose positio
  * batch of the active kind; the batch kernel (run_batches) takes it from there.  The hot second-by-second loop then runs in
  * launches that contain nothing else: its code stays in the SMs' instruction caches instead of competing with the event
  * machinery of the environments next door (profiles/r02*_icache.md). */
-WRSN_DI int run_loop(Ctx &c, int budget, int split) {
+WRSN_DI int run_loop(Ctx &c, int budget, int split, int *work = nullptr) {
     Clk k;
     clk_load(c, k);
     k.work = 0;
@@ -2374,6 +2374,7 @@ WRSN_DI int run_loop(Ctx &c, int budget, int split) {
     catch_up_many(c, k.now, 1);
     WRSN_PROFB_END(c, WRSN_H_PROF2); }
     clk_store(c, k);
+    if (work) *work = k.work;                        /* (the rule rollout's launch-wide budget) */
     return interrupted;
 }
 
@@ -2538,7 +2539,8 @@ WRSN_D void entry_batches(Ctx &c, ReqOut *r, int budget) {
     entry_in_flight(c, r, code);
 }
 
-WRSN_D void entry_step(Ctx &c, int agent_id, const double *input_action, ReqOut *r, int budget, int split) {
+/* `work` (may be NULL): the work units the call used, for a caller that spreads one budget over several steps */
+WRSN_D void entry_step(Ctx &c, int agent_id, const double *input_action, ReqOut *r, int budget, int split, int *work = nullptr) {
     const bool resume = c.hdr[WRSN_H_INFLIGHT] != 0.0;
     gsync(c);
     if (c.tid == 0 && !resume) {
@@ -2581,7 +2583,8 @@ WRSN_D void entry_step(Ctx &c, int agent_id, const double *input_action, ReqOut 
     gsync(c);
     const int watched = (int)c.hdr[WRSN_H_CHAIN_N];
     int interrupted = 0;
-    if (watched > 0) interrupted = run_loop(c, budget, split);
+    if (watched > 0) interrupted = run_loop(c, budget, split, work);
+    else if (work) *work = 0;
     gsync(c);
     if (interrupted) { entry_in_flight(c, r, interrupted); return; }
     int id = -1;

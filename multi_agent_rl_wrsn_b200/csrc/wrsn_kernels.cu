@@ -874,8 +874,9 @@ __global__ void __launch_bounds__(COPY_THREADS) k_copy_rows(int32_t state_bytes,
 #include "wrsn_abi_aux.h"
 static_assert(WRSN_DEC_MAX_RANK == DEC_MAXR - 2, "the host refuses the map sizes whose rank k_decode_map cannot hold");
 
+/* one launch of k_env<MODE>, or of k_env_roll with R for MODE_RULE_ROLLOUT */
 template <int MODE>
-static int launch_env(KParams &P, void *stream) {
+static int launch_env_kernel(KParams &P, void *stream, const RollArgs &R) {
     if (prepare_launch(P)) return -1;
     /* the opt-in dynamic shared-memory limit is a per-DEVICE attribute of the function: cache it per template instance, group
        build and device (a second GPU in the same process needs its own opt-in) */
@@ -889,16 +890,29 @@ static int launch_env(KParams &P, void *stream) {
     if (pad < 0) { const char *e = getenv("WRSN_SMEM_PAD"); pad = e ? atoll(e) : 0; if (pad < 0 || pad > 200 * 1024) pad = 0; }
     const int w = P.d.threads == 32 ? 0 : 1;
     const int64_t smem = P.L.smem_total + pad;
+    constexpr bool roll = MODE == MODE_RULE_ROLLOUT;
     if (smem > attr_cache[w][dev]) {
-        if (w == 0) WRSN_CUDA(cudaFuncSetAttribute(g32::k_env<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        else WRSN_CUDA(cudaFuncSetAttribute(gany::k_env<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const void *fn;
+        if constexpr (roll) fn = w == 0 ? (const void *)g32::k_env_roll : (const void *)gany::k_env_roll;
+        else fn = w == 0 ? (const void *)g32::k_env<MODE> : (const void *)gany::k_env<MODE>;
+        WRSN_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_cache[w][dev] = smem;
     }
-    if (w == 0) g32::k_env<MODE><<<P.d.B, 32, (size_t)smem, (cudaStream_t)stream>>>(P);
-    else gany::k_env<MODE><<<P.d.B, P.d.threads, (size_t)smem, (cudaStream_t)stream>>>(P);
+    if constexpr (roll) {
+        if (w == 0) g32::k_env_roll<<<P.d.B, 32, (size_t)smem, (cudaStream_t)stream>>>(P, R);
+        else gany::k_env_roll<<<P.d.B, P.d.threads, (size_t)smem, (cudaStream_t)stream>>>(P, R);
+    } else {
+        if (w == 0) g32::k_env<MODE><<<P.d.B, 32, (size_t)smem, (cudaStream_t)stream>>>(P);
+        else gany::k_env<MODE><<<P.d.B, P.d.threads, (size_t)smem, (cudaStream_t)stream>>>(P);
+    }
     WRSN_CUDA(cudaGetLastError());
     return 0;
 }
+
+template <int MODE>
+static int launch_env(KParams &P, void *stream) { return launch_env_kernel<MODE>(P, stream, RollArgs()); }
+
+static int launch_roll(KParams &P, const RollArgs &R, void *stream) { return launch_env_kernel<MODE_RULE_ROLLOUT>(P, stream, R); }
 
 /* Measured (4096 environments, RandomController law): one launch of 4096 rows 1.03 -> 1.13 M decisions/s with the order; four
    groups of 1024 rows on four streams 1.20 -> 1.23 M (the other groups' kernels already fill the tail, and the ordering kernel

@@ -3,6 +3,7 @@
  * (shared by the host side of the C ABI, the kernels and the tests' host emulation).
  */
 #pragma once
+#include <float.h>
 #include <math.h>
 #include <stdint.h>
 #include <string.h>
@@ -100,9 +101,10 @@ struct WrsnRow {
     const double *hdr, *mc, *proc, *energy, *cs;    /* environment record */
     const uint8_t *status;
     int N;                                          /* this scenario's nodes (dims.N: the batch's largest) */
-    WRSN_HDM WrsnRow(const WrsnLayout &L, const char *state, const char *scen, const int32_t *scen_id, int b) {
-        const char *row = state + (size_t)b * L.total;
-        const char *srow = scen + (size_t)scen_id[b] * L.scen_total;
+    WRSN_HDM WrsnRow(const WrsnLayout &L, const char *state, const char *scen, const int32_t *scen_id, int b)
+        : WrsnRow(L, state + (size_t)b * L.total, scen + (size_t)scen_id[b] * L.scen_total) {}
+    /* `row`: a record, or its resident image in shared memory (the fields read here are all resident); `srow`: its scenario's record */
+    WRSN_HDM WrsnRow(const WrsnLayout &L, const char *row, const char *srow) {
         par = (const double *)(srow + L.soff[WRSN_S_PAR]);
         nx = (const double *)(srow + L.soff[WRSN_S_NX]);
         ny = (const double *)(srow + L.soff[WRSN_S_NY]);
@@ -194,7 +196,8 @@ WRSN_HD int32_t wrsn_obs_pitch(int S) {
 }
 
 /* ------------------------------------------------------------------ the hand-written charging rules (include/wrsn_b200.h:
- * wrsn_heuristic_action).  k_heuristic and the host emulation state the rule only through these functions. */
+ * wrsn_heuristic_action).  k_heuristic, the rule rollout (wrsn_env_kernel.cuh: roll_pick) and the host emulation state the rule
+ * only through these functions. */
 #define HEUR_NONE 0x7fffffff                        /* id of an empty set's best: sorts after every node */
 
 struct HeurFleet {                                  /* what the rule reads of a row's chargers, once per row */
