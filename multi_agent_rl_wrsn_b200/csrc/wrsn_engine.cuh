@@ -1654,6 +1654,71 @@ WRSN_D int slot_lazy_ok(Ctx &c, double ur_t, double ur_key, int s) {
     return 2;
 }
 
+/* Far from the destination and from exhaustion a move span is always 1 s: min(mt, 1.0, (energy - threshold) / (pm v))
+ * with mt >= 1 and energy - threshold >= pm v (x / y >= 1 exactly when x >= y).  Then neither the square root nor the two
+ * divisions are needed to know the span, and the remaining time `mt` is only needed once, for the position the replay
+ * stops at (it is a pure function of the position: move :91).  The margin above v^2 keeps sqrt(d2) / v > 1 after both
+ * roundings, so that the skipped arrival check (mt - span <= 0) could not have fired; anything closer takes the literal
+ * arithmetic. */
+WRSN_DI bool move_span_is_one(double d2, double far, double en1, double thr, double pmv) {
+    return d2 > far && en1 - thr >= pmv;
+}
+WRSN_DI double move_far(double v) { return v * v * 1.000001; }
+
+/* A lazy charge: the charger's energy and CPA2, the charge's remaining time (tmp) and current span, the span event's time */
+struct ChargeRun { double en, cpa2, tmp, span, tf; };
+
+/* replay the charge spans of r whose event time is < limit, literally (charge_step :45-46, charge :63-69) or, `jumps`, m
+ * one-second spans at once; returns the number replayed and sets *t_end to the time of the span event at which the run
+ * stops being private (left alone if the limit came first) */
+WRSN_DI int charge_run(ChargeRun &r, double rate, double thr, double limit, bool jumps, double *t_end) {
+    double en = r.en, cpa2 = r.cpa2, tmp = r.tmp, span = r.span, tf = r.tf;
+    int n = 0;
+    while (tf < limit) {
+        if (on_grid(tf)) { *t_end = tf; break; }
+        /* m one-second spans at once.  While the span stays 1.0 every step subtracts the same `rate` from the energy (the
+           same integer number of ulps inside a binade: sub_chain), 1.0 from the two countdowns (exact below 2^53) and adds
+           1.0 to the event time (exact inside the time's binade, where on_grid() cannot change either: the fraction of
+           tf is preserved).  m is cut so that all of that holds and none of the loop's exits can fire inside the jump;
+           whatever is left runs through the literal step below. */
+        if (span == 1.0 && tmp > 2.0 && tmp < 1073741824.0 && cpa2 < 4503599627370496.0 && jumps) {
+            const double fl = floor(tmp);
+            double m = fl == tmp ? tmp - 1.0 : fl;                             /* spans of 1.0 before the last, shorter one */
+            m = fmin(m, floor(limit - tf));                                    /* (inf - tf = inf) */
+            const int ext = wrsn_biased_exp(tf);
+            if (tf > 0.0 && ext > 60 && ext < 1100) m = fmin(m, floor(wrsn_pow2_biased(ext + 1) - tf)); else m = 0.0;
+            double en_m = en;
+            if (rate != 0.0) {
+                const int ex = wrsn_biased_exp(en);
+                if (en > 0.0 && ex > 60 && ex < 1900) {
+                    const double lo = wrsn_pow2_biased(ex), inv_u = wrsn_pow2_biased(2098 - ex), u = wrsn_pow2_biased(ex - 52);
+                    const double q = rate * inv_u, rq = rint(q);
+                    const double room = en - fmax(lo, thr);
+                    if (fabs(q - rq) == 0.5 || !(rq > 0.0) || !(room > 0.0)) m = 0.0;
+                    else {
+                        m = fmin(m, floor(room / (rq * u)) - 1.0);
+                        if (m >= 2.0 && rq * m < 4503599627370496.0) en_m = en - (rq * m) * u; else m = 0.0;
+                    }
+                } else m = 0.0;
+            }
+            if (m >= 2.0) {
+                en = en_m; cpa2 = cpa2 >= m ? cpa2 - m : 0.0; tmp = tmp - m;
+                span = fmin(tmp, 1.0);
+                tf = (tf + (m - 1.0)) + span; n += (int)m;
+                continue;
+            }
+        }
+        const double en1 = en - rate * span;                                   /* charge_step :45 */
+        const double cpa21 = fmax(0.0, cpa2 - span);                           /* :46 */
+        const double tmp1 = tmp - span;                                        /* charge :69 */
+        if (tmp1 == 0.0 || en1 <= thr) { *t_end = tf; break; }
+        en = en1; cpa2 = cpa21; tmp = tmp1; span = fmin(tmp1, 1.0);            /* :63-68 (the rate is 0 there: no energy limiter, Q3) */
+        tf = tf + span; n++;
+    }
+    r.en = en; r.cpa2 = cpa2; r.tmp = tmp; r.span = span; r.tf = tf;
+    return n;
+}
+
 /* replay spans of slot s whose event time is < limit; returns the number replayed and, in *t_end, the time of the span
  * event at which the run stops being private (or +inf if the limit came first).
  * mode FF_DRY: nothing is stored.  FF_ALL: every thread of the environment makes the same call, the leader stores.
@@ -1682,13 +1747,8 @@ WRSN_NOINLINE int slot_ff(Ctx &c, int s, double limit, int mode, double *t_end) 
         const double destx = p[WRSN_PR_DESTX], desty = p[WRSN_PR_DESTY], vx = p[WRSN_PR_VX], vy = p[WRSN_PR_VY], total = p[WRSN_PR_TOTAL];
         double x = m[WRSN_MC_X], y = m[WRSN_MC_Y], en = m[WRSN_MC_ENERGY];
         double mt = p[WRSN_PR_MT], span = p[WRSN_PR_SPAN], svx = p[WRSN_PR_SVX], svy = p[WRSN_PR_SVY];
-        /* Far from the destination and from exhaustion a span is always 1 s: min(mt, 1.0, (energy - threshold) / (pm v))
-           with mt >= 1 and energy - threshold >= pm v (x / y >= 1 exactly when x >= y).  Then neither the square root nor
-           the two divisions are needed to know the span, and the remaining time `mt` is only needed once, for the
-           position the replay stops at (it is a pure function of the position: move :91).  `far` is a safe margin above
-           v^2; anything closer takes the literal arithmetic. */
         const double ux = vx / total, uy = vy / total;                            /* move_step :77 (vec / total) * span */
-        const double far = v * v * 1.000001;
+        const double far = move_far(v);
         bool mt_known = true;
         while (tf < limit) {
             /* (a span that fires exactly on the node grid is still private: a moving charger is not "charging", so no
@@ -1698,7 +1758,7 @@ WRSN_NOINLINE int slot_ff(Ctx &c, int s, double limit, int mode, double *t_end) 
             if (en1 <= thr) { *t_end = tf; break; }                               /* arrival / exhaustion: ev_slot's business */
             const double dx = destx - x1, dy = desty - y1, d2 = dx * dx + dy * dy;
             double span2;
-            if (d2 > far && en1 - thr >= pmv) { span2 = 1.0; mt_known = false; }
+            if (move_span_is_one(d2, far, en1, thr, pmv)) { span2 = 1.0; mt_known = false; }
             else {
                 mt = sqrt(d2) / v; mt_known = true;                               /* move :91-94 */
                 span2 = fmin(fmin(mt, 1.0), (en1 - thr) / pmv);
@@ -1716,55 +1776,16 @@ WRSN_NOINLINE int slot_ff(Ctx &c, int s, double limit, int mode, double *t_end) 
             }
         }
     } else {                                         /* PC_CS_FIRE: a charge whose disconnect / reconnect pairs change nothing */
-        double en = m[WRSN_MC_ENERGY], cpa2 = m[WRSN_MC_CPA2], tmp = p[WRSN_PR_CHTMP], span = p[WRSN_PR_CHSPAN];
+        ChargeRun r = { m[WRSN_MC_ENERGY], m[WRSN_MC_CPA2], p[WRSN_PR_CHTMP], p[WRSN_PR_CHSPAN], tf };
         const double rate = m[WRSN_MC_RATE];
         const bool jumps = c.hdr[WRSN_H_OPT_NOBATCH] != 1.0;                      /* (test switch: every span literally) */
-        while (tf < limit) {
-            if (on_grid(tf)) { *t_end = tf; break; }
-            /* m one-second spans at once.  While the span stays 1.0 every step subtracts the same `rate` from the energy (the
-               same integer number of ulps inside a binade: sub_chain), 1.0 from the two countdowns (exact below 2^53) and adds
-               1.0 to the event time (exact inside the time's binade, where on_grid() cannot change either: the fraction of
-               tf is preserved).  m is cut so that all of that holds and none of the loop's exits can fire inside the jump;
-               whatever is left runs through the literal step below. */
-            if (span == 1.0 && tmp > 2.0 && tmp < 1073741824.0 && cpa2 < 4503599627370496.0 && jumps) {
-                const double fl = floor(tmp);
-                double m = fl == tmp ? tmp - 1.0 : fl;                             /* spans of 1.0 before the last, shorter one */
-                m = fmin(m, floor(limit - tf));                                    /* (inf - tf = inf) */
-                const int ext = wrsn_biased_exp(tf);
-                if (tf > 0.0 && ext > 60 && ext < 1100) m = fmin(m, floor(wrsn_pow2_biased(ext + 1) - tf)); else m = 0.0;
-                double en_m = en;
-                if (rate != 0.0) {
-                    const int ex = wrsn_biased_exp(en);
-                    if (en > 0.0 && ex > 60 && ex < 1900) {
-                        const double lo = wrsn_pow2_biased(ex), inv_u = wrsn_pow2_biased(2098 - ex), u = wrsn_pow2_biased(ex - 52);
-                        const double q = rate * inv_u, rq = rint(q);
-                        const double room = en - fmax(lo, thr);
-                        if (fabs(q - rq) == 0.5 || !(rq > 0.0) || !(room > 0.0)) m = 0.0;
-                        else {
-                            m = fmin(m, floor(room / (rq * u)) - 1.0);
-                            if (m >= 2.0 && rq * m < 4503599627370496.0) en_m = en - (rq * m) * u; else m = 0.0;
-                        }
-                    } else m = 0.0;
-                }
-                if (m >= 2.0) {
-                    en = en_m; cpa2 = cpa2 >= m ? cpa2 - m : 0.0; tmp = tmp - m;
-                    span = fmin(tmp, 1.0);
-                    tf = (tf + (m - 1.0)) + span; n += (int)m;
-                    continue;
-                }
-            }
-            const double en1 = en - rate * span;                                   /* charge_step :45 */
-            const double cpa21 = fmax(0.0, cpa2 - span);                           /* :46 */
-            const double tmp1 = tmp - span;                                        /* charge :69 */
-            if (tmp1 == 0.0 || en1 <= thr) { *t_end = tf; break; }
-            en = en1; cpa2 = cpa21; tmp = tmp1; span = fmin(tmp1, 1.0);            /* :63-68 (the rate is 0 there: no energy limiter, Q3) */
-            tf = tf + span; n++;
-        }
+        n = charge_run(r, rate, thr, limit, jumps, t_end);
+        tf = r.tf;
         if (mode != FF_DRY && n > 0) {
             if (mode == FF_ALL) gsync(c);
             if (store) {
-                m[WRSN_MC_ENERGY] = en; m[WRSN_MC_CPA2] = cpa2; m[WRSN_MC_CHTIME] = tmp;
-                p[WRSN_PR_CHTMP] = tmp; p[WRSN_PR_CHSPAN] = span;
+                m[WRSN_MC_ENERGY] = r.en; m[WRSN_MC_CPA2] = r.cpa2; m[WRSN_MC_CHTIME] = r.tmp;
+                p[WRSN_PR_CHTMP] = r.tmp; p[WRSN_PR_CHSPAN] = r.span;
             }
         }
     }

@@ -925,3 +925,4 @@ int orc_get_static(Oracle *o, int *nbr_ptr, int *nbr_idx, int *tgt_ptr, int *tgt
 }
 /* test-only: overwrite node i's energy (the tests place energies on binade edges in both simulators) */
 void orc_set_node_energy(Oracle *o, int i, double e) { o->energy[i] = e; }
+void orc_set_mc_energy(Oracle *o, int a, double e) { o->mc[a].energy = e; }

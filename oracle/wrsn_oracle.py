@@ -55,6 +55,7 @@ def lib():
         L.orc_get_static.argtypes = [C.c_void_p, ip, ip, ip, ip, ip]
         L.orc_get_static.restype = C.c_int
         L.orc_set_node_energy.argtypes = [C.c_void_p, C.c_int, C.c_double]
+        L.orc_set_mc_energy.argtypes = [C.c_void_p, C.c_int, C.c_double]
         _LIB = L
     return _LIB
 
@@ -158,6 +159,10 @@ class OracleWRSN:
     def set_node_energy(self, i, e):
         """TEST INFRASTRUCTURE: overwrite node i's energy (no event, no status check)."""
         self.L.orc_set_node_energy(self.h, int(i), float(e))
+
+    def set_mc_energy(self, a, e):
+        """TEST INFRASTRUCTURE: overwrite charger a's energy (no event)."""
+        self.L.orc_set_mc_energy(self.h, int(a), float(e))
 
     # -- accessors --------------------------------------------------------------------
     @property

@@ -1,6 +1,7 @@
 /*
- * energy_probe.cu — TEST INFRASTRUCTURE (tests/test_energy_chains.py).  Scalar entry points into the engine's exact energy
- * arithmetic, so that the closed forms can be compared with literal fp64 chains one case at a time.
+ * energy_probe.cu — TEST INFRASTRUCTURE (tests/test_energy_chains.py, tests/test_charger_spans.py).  Scalar entry points into
+ * the engine's exact energy arithmetic and its lazy charger spans, so that the closed forms can be compared with literal fp64
+ * chains one case at a time.
  *
  * Built twice by the test, never by the package:
  *   - g++ -x c++ with the flags of tests/emu/Makefile: wrsn_engine.cuh under WRSN_HOST_EMU, WRSN_GFIX 1 (the host build);
@@ -30,10 +31,10 @@ namespace host1 {
 #endif
 
 #define PROBE_IN 10
-#define PROBE_OUT 6
+#define PROBE_OUT 8
 
 enum { OP_SUB_CHAIN = 0, OP_SUB_CHAIN_FAST, OP_SUB_CHAIN_LITERAL, OP_DRAIN_NODE, OP_REPLAY_CYCLES, OP_SPEC_TERMS, OP_BATCH_DEC,
-       OP_RCP, OP_RSQRT, OP_EXP_TAB };
+       OP_RCP, OP_RSQRT, OP_EXP_TAB, OP_CHARGE_RUN, OP_MOVE_SPAN };
 
 /* tab: the exp table in shared memory (device), unused on the host */
 template <typename Tab>
@@ -66,6 +67,16 @@ PROBE_D static void probe_one(int op, const double *x, double *y, Tab tab) {
         y[1] = (double)m;
         break;
     }
+    case OP_CHARGE_RUN: {                            /* en, rate, thr, tmp, cpa2, span, tf, limit, jumps -> en, cpa2, tmp, span, tf,
+                                                        n, t_end (+inf: the limit came first) */
+        ChargeRun r = { x[0], x[4], x[3], x[5], x[6] };
+        double t_end = INFINITY;
+        const int n = charge_run(r, x[1], x[2], x[7], x[8] != 0.0, &t_end);
+        y[0] = r.en; y[1] = r.cpa2; y[2] = r.tmp; y[3] = r.span; y[4] = r.tf; y[6] = (double)n; y[7] = t_end;
+        break;
+    }
+    case OP_MOVE_SPAN:                               /* d2, en1, thr, v, pmv -> 1 if the span is taken as 1 s unseen */
+        y[0] = move_span_is_one(x[0], move_far(x[3]), x[1], x[2], x[4]) ? 1.0 : 0.0; break;
 #if defined(__CUDACC__)
     case OP_RCP: y[0] = wrsn_rcp(x[0]); break;
     case OP_RSQRT: y[0] = wrsn_rsqrt(x[0]); break;

@@ -198,7 +198,8 @@ def compare_row_with_oracle(env, v, b, o, r, prev_fit, k):
 
 
 def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=None, check_obs=False, scale2=0.05,
-                    map_size=100, scenario_index=None, controller=False, obs32=False, threads=0, rounds=0, probe=None, spread=0.0):
+                    map_size=100, scenario_index=None, controller=False, obs32=False, threads=0, rounds=0, probe=None, spread=0.0,
+                    warm_up_time=100.0, before_step=None):
     """B environments with DIFFERENT action streams (and possibly different scenarios) vs B oracle runs (ladder L6), every
     row at every request as ``compare_row_with_oracle`` states.
     ``controller``: the actions are those of the reference's RandomController — the density map s0 + s1 - 10 s2 + s3 of the
@@ -207,18 +208,20 @@ def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=No
     ``obs32``: also the float32 raster against the oracle's state at 1e-5 of the channel maximum.
     ``probe(env, rows)``: called at every request with the boolean mask of the rows compared there (e.g. to count the
     requests that reached a regime the test is about).  ``spread``: the uniform actions are drawn from [-spread, 1 + spread]
-    (before ``scale2``), so that the clipping of WRSN.step is exercised."""
+    (before ``scale2``), so that the clipping of WRSN.step is exercised.  ``warm_up_time``: the simulated time before the first
+    request, on both sides.  ``before_step(env, oracles, k, live, aid, act)``: called after the rows were compared at request k
+    and before they are stepped with the actions ``act`` (e.g. to edit the same state in the engine and in the oracles)."""
     if isinstance(scenarios, Scenario):
         scenarios = [scenarios]
     env = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, map_size=map_size,
-                      scenario_index=scenario_index, threads=threads, step_rounds=rounds)
+                      scenario_index=scenario_index, threads=threads, step_rounds=rounds, warm_up_time=warm_up_time)
     sid = _np(env.scen_id)
     B = num_envs
     rng = np.random.default_rng(seed)
     acts = rng.uniform(-spread, 1.0 + spread, size=(steps, B, 3))       # spread > 0: some components outside [0, 1] (clipped)
     acts[..., 2] *= scale2
-    oracles = [OracleWRSN(scenario_from_dict(scenarios[sid[b]].to_dict()), num_agent=num_agent, mc=mc, map_size=map_size)
-               for b in range(B)]
+    oracles = [OracleWRSN(scenario_from_dict(scenarios[sid[b]].to_dict()), num_agent=num_agent, mc=mc, map_size=map_size,
+                          warm_up_time=warm_up_time) for b in range(B)]
     for o in oracles:
         o.set_event_budget(3_000_000)
     req = env.reset()
@@ -266,6 +269,8 @@ def check_vs_oracle(scenarios, device, num_envs, steps, seed, num_agent=3, mc=No
             act_k[~live] = 0.0
         else:
             act_k = acts[k]
+        if before_step is not None:
+            before_step(env, oracles, k, live.copy(), aid, act_k)
         req = env.step(np.where(live, aid, -1).astype(np.int32), act_k, mask=mask)
         for b in range(B):
             if live[b]:
@@ -358,19 +363,24 @@ def _state_diff_but_switch(a, b):
 
 
 def check_batches_equal_event_path(scenarios, device, num_envs, steps, seed, num_agent=3, scale2=0.3, threads=0, mc=None,
-                                   probe=None):
+                                   probe=None, warm_up_time=100.0, before_step=None):
     """Whole-cycle batches (nodes_batch) leave EVERY byte of the environment record — node rows, event clock with its
     insertion counters, charger records — exactly as the event-by-event path does, over several episodes.  ``probe(env)``:
-    called with the batched simulator after every step."""
+    called with the batched simulator after every step.  ``before_step(a, b, k, act)``: called before step k with both
+    simulators and the actions (e.g. to edit the same state in both)."""
     rng = np.random.default_rng(seed)
     acts = rng.uniform(0.0, 1.0, size=(steps, num_envs, 3))
     acts[..., 2] *= scale2
-    a = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, threads=threads)
-    b = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, threads=threads)
+    a = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, threads=threads,
+                    warm_up_time=warm_up_time)
+    b = BatchedWRSN(scenarios, num_agent=num_agent, mc_type=mc, num_envs=num_envs, device=device, threads=threads,
+                    warm_up_time=warm_up_time)
     _disable_batches(b)
     a.reset(); b.reset()
     ends = 0
     for k in range(steps):
+        if before_step is not None:
+            before_step(a, b, k, acts[k])
         act = torch.as_tensor(acts[k], device=a.device)
         a.rollout_step(act); b.rollout_step(act)
         ends += int((a.req.now == a.warm_up_time).sum())           # rows that were just reset
@@ -589,11 +599,11 @@ def check_charge_kernel(scenarios, device, num_envs, steps, seed, num_agent=3, m
 
 
 def check_budget_equals_unbudgeted(scenarios, device, num_envs, calls, seed, budget, num_agent=3, scale2=0.3, threads=0, rounds=0,
-                                   mc=None, probe=None):
+                                   mc=None, probe=None, launch_probe=None):
     """A step budget (wrsn_dims.step_budget) only cuts a WRSN.step into several launches: every request an environment hands
     out — agent, time, reward, termination, clipped action — and every byte of its record at that moment are those of the
     unbudgeted run answered with the same actions.  Returns how many interrupted launches it took.  ``probe(env)``: called with
-    the unbudgeted simulator after every step."""
+    the unbudgeted simulator after every step; ``launch_probe(env)``: with the budgeted one after every launch."""
     rng = np.random.default_rng(seed)
     acts = rng.uniform(0.0, 1.0, size=(calls, num_envs, 3))
     acts[..., 2] *= scale2
@@ -626,6 +636,8 @@ def check_budget_equals_unbudgeted(scenarios, device, num_envs, calls, seed, bud
         act = torch.as_tensor(acts[cur, np.arange(num_envs)], device=b.device)
         b.rollout_step(act)
         launches += 1
+        if launch_probe is not None:
+            launch_probe(b)
         aid = _np(b.req.agent_id)
         st = rows(b)
         got = {f: _np(getattr(b.req, f)) for f in fields}

@@ -33,9 +33,9 @@ from tests.helpers import REPO
 CSRC = os.path.join(REPO, "multi_agent_rl_wrsn_b200", "csrc")
 EMU_DIR = os.path.join(REPO, "tests", "emu")
 PROBE_SRC = os.path.join(EMU_DIR, "energy_probe.cu")
-PROBE_IN, PROBE_OUT = 10, 6
+PROBE_IN, PROBE_OUT = 10, 8
 (OP_SUB_CHAIN, OP_SUB_CHAIN_FAST, OP_SUB_CHAIN_LITERAL, OP_DRAIN_NODE, OP_REPLAY_CYCLES, OP_SPEC_TERMS, OP_BATCH_DEC,
- OP_RCP, OP_RSQRT, OP_EXP_TAB) = range(10)
+ OP_RCP, OP_RSQRT, OP_EXP_TAB, OP_CHARGE_RUN, OP_MOVE_SPAN) = range(12)
 GPU = "cuda:0"
 KS = range(9, 15)                                    # binades 2^9 .. 2^14: the scenarios' threshold-to-capacity range
 SLACK = 1e-6                                         # the engine's margin above the threshold (replay_cycles, batch_dec)

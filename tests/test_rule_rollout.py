@@ -166,7 +166,7 @@ def _warm(budget):
     return prepare
 
 
-@pytest.mark.parametrize("budget,rounds", [(0, 0), (25, 0), (60, 2), (25, 2)])
+@pytest.mark.parametrize("budget,rounds", [(0, 0), (25, 0), (60, 2), (25, 2), (1, 0), (3, 0)])
 def test_mixed_batch_equals_the_restatement(host, budget, rounds):
     make = lambda: tl._mixed(B=8, step_budget=budget, step_rounds=rounds)     # noqa: E731  82 / 98 / 132 / 100 nodes
     a, b, snap = _pair(make, _warm(budget))
